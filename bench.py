@@ -8,6 +8,7 @@ tokens), fwd+bwd, bf16, per-GPU batch 12, synthetic trunk features.  BASELINE.js
 is measured in the same run and reported as the sub-record ``stage4`` (``--workload stage4`` makes it the whole line).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload fusion4|stage4|model] [--anchors 8|16]
+                  [--dump-outputs DIR]
 
 N > 1 is launched by torchrun (one rank per GPU): every rank runs its own batch-12 shard (weak scaling) and the GPT gradients
 are all-reduced over NCCL every step (DDP semantics of train2_seq.py:538 replaced by one-process-per-GPU).  Rank 0 prints
@@ -114,6 +115,24 @@ def synth_inputs(gen, batch, c, scale, pin=False):
     return ts[:3], ts[3], ts[4:]
 
 
+def dump_outputs(out_dir, named):
+    """Writes every (name, tensor) of ``named`` as ``out_dir/<name>.npy`` in float32, 64 MB in all.  Each tensor gets an equal
+    share of that; a larger tensor is stored flattened, as the elements at a fixed set of positions (drawn once per element count
+    by a generator seeded with 0), so two runs with the same arguments store the same positions and can be compared file by file."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    cap = (64 * 10 ** 6 // len(named) - 4096) // 4   # elements per file; 4 KB of the share is left for the .npy header
+    picks = {}
+    for name, t in named:
+        x = t.detach()
+        n = x.numel()
+        if n > cap:
+            if n not in picks:
+                picks[n] = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:cap].sort().values
+            x = x.reshape(-1)[picks[n].to(x.device)]
+        np.save(os.path.join(out_dir, name + ".npy"), x.float().cpu().numpy())
+
+
 def cpu_model():
     try:
         for line in open("/proc/cpuinfo"):
@@ -210,7 +229,7 @@ def cpu_sample_note(kind, cores, steps, warmup):
 def run_reference(args, rank):
     if rank != 0:
         return
-    steps, warmup = max(1, args.steps), max(0, args.warmup)
+    steps, warmup = args.steps, max(0, args.warmup)
     v, ms, kind = time_cpu(steps, warmup)
     cores = torch.get_num_threads()
     print(json.dumps({
@@ -264,6 +283,9 @@ class StageWork:
             t.grad = None
         self.gps.grad = None
         outs = self.gpt.fuse(self.feats[0], self.feats[1], self.feats[2], self.gps)
+        # kept for --dump-outputs (a replayed CUDA graph rewrites them in place); detached, so that they do not keep this step's
+        # autograd graph, and with it the parameters' gradient accumulators, alive into the next step
+        self.outs = [o.detach() for o in outs]
         # the probes are the upstream gradients (in the model they come from the ResNet layers that follow the stage); the step's
         # scalar result is the sum of the two GPS output tokens (a 12 x 2 x C reduction: the only non-dsfuse kernel of the step)
         torch.autograd.backward(outs, self.probes)
@@ -271,6 +293,13 @@ class StageWork:
             self.opt.step()
             self.ema.update()
         return outs[3].detach().sum()
+
+    def computed(self):
+        """(name, tensor) of what the last step handed back: the four outputs and the gradients of the inputs and parameters."""
+        names = ("img", "lidar", "radar", "gps")
+        named = [("C%d.out.%s" % (self.c, n), o) for n, o in zip(names, self.outs)]
+        named += [("C%d.grad.%s" % (self.c, n), t.grad) for n, t in zip(names, self.feats + [self.gps])]
+        return named + [("C%d.grad.%s" % (self.c, n), p.grad) for n, p in self.gpt.named_parameters() if p.grad is not None]
 
 
 def one_step(works):
@@ -564,8 +593,10 @@ def run_ours(args, rank, world, local_rank):
             ms = float(t.item())
         return ms, n1 - n0, clocks
 
-    steps, warmup = max(1, args.steps), max(3, args.warmup)
+    steps, warmup = args.steps, max(3, args.warmup)
     ms, launches, clocks = timed(step_resident, steps, warmup, ClockSampler(local_rank) if rank == 0 else None)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, [nt for w in works for nt in w.computed()])
     value = BATCH * world * steps / (ms * 1e-3)
     if args.quick:
         synced, sync_bad = check_grads_synced(works, world, dist)
@@ -770,11 +801,14 @@ def run_model(args, rank, world, local_rank):
             graph = None
         torch.cuda.synchronize()
 
+    last_loss = [graph_loss]   # the loss of the last resident step (--dump-outputs)
+
     def step_resident():
         if graph is not None:
             graph.replay()
             return graph_loss
-        return step_eager()
+        last_loss[0] = step_eager().detach()
+        return last_loss[0]
 
     # e2e: one pinned-host -> device batch copy (94 MB) per step into preallocated, double-buffered staging tensors on a
     # copy stream, overlapped with the previous step's compute; the step then reads the staged batch (graph mode: after a
@@ -844,12 +878,16 @@ def run_model(args, rank, world, local_rank):
             ms = float(t.item())
         return ms, (_capi.launch_count() - n0) + (graph_launches * steps if graph is not None else 0)
 
-    steps, warmup = max(1, args.steps), max(3, args.warmup)
+    steps, warmup = args.steps, max(3, args.warmup)
     sampler = ClockSampler(local_rank) if rank == 0 else None
     if sampler:
         sampler.start()
     ms, launches = timed(step_resident, steps, warmup)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:   # what a caller of train_step holds afterwards: the loss, the updated parameters, the gradients
+        params = list(model.named_parameters())
+        dump_outputs(args.dump_outputs, [("loss", last_loss[0])] + [("param." + n, p) for n, p in params] +
+                     [("grad." + n, p.grad) for n, p in params if p.grad is not None])
     ms_e2e, _ = timed(step_e2e, steps, 2, finalize=lambda: torch.cuda.current_stream().wait_event(ev_ready[e2e_k[0] & 1]))
     loss_val = float(loss_h)
     params_synced = None
@@ -910,7 +948,15 @@ def main():
                     help="embd/attn/resid dropout probability (default 0 = the parity configuration; the reference trains with 0.1)")
     ap.add_argument("--anchors", type=int, default=8, choices=[8, 16],
                     help="16 = BASELINE.json configs[4], the scaled fusion path: 512x512 inputs, 16x16 anchors -> T = 3842 tokens")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float32, 64 MB in all; a larger "
+                         "tensor is stored as a fixed, seeded sample of its elements): per stage the outputs and the gradients of the "
+                         "inputs and parameters; --workload model: the loss, the updated parameters and their gradients")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the GPU arm computed; --impl reference has no such outputs")
     global PDROP, A, SPEC
     PDROP = args.dropout
     A = args.anchors

@@ -41,6 +41,34 @@ def test_both_arms_name_the_same_workload():
     assert abs(tot / 1e9 - 92.74) < 0.05 and abs(bench.fwd_flops_per_sample(512) / 1e9 - 63.58) < 0.05
 
 
+def test_dump_outputs_keeps_64_mb_and_samples_fixed_positions(tmp_path):
+    """--dump-outputs: float32 files, 64 MB in all, small tensors whole, large ones sampled at the same positions every run."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    gen = torch.Generator().manual_seed(1)
+    named = [("big.%d" % i, torch.randn(4_000_000, generator=gen).to(torch.bfloat16)) for i in range(8)]
+    named += [("small", torch.randn(3, 5, generator=gen, dtype=torch.float64))]
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), named)
+    files = sorted(os.listdir(tmp_path / "a"))
+    assert files == sorted(n + ".npy" for n, _ in named)
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in files) <= 64 * 10 ** 6
+    for f in files:
+        a, b = np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)
+        assert a.dtype == np.float32 and np.array_equal(a, b)
+    assert np.array_equal(np.load(tmp_path / "a" / "small.npy"), named[-1][1].float().numpy())
+    big = np.load(tmp_path / "a" / "big.0.npy")
+    assert 1_000_000 < big.size < 4_000_000 and np.isin(big, named[0][1].float().numpy()).all()
+
+
+def test_steps_below_one_are_refused():
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "0"], capture_output=True,
+                         text=True, timeout=600, cwd=ROOT)
+    assert out.returncode != 0 and "--steps" in out.stderr
+
+
 def test_gpu_arm_refuses_to_run_without_a_gpu():
     """No CPU fallback on the product path: without CUDA the default arm exits with an error instead of timing the oracle."""
     import torch
