@@ -46,8 +46,8 @@ def build_tokens(img: Tensor, lidar: Tensor, radar: Tensor, gps: Tensor, pos_emb
                  seq_len: int, n_views: int) -> Tensor:
     """Token build of ``GPT.forward`` (model2_seq.py:256-272) without dropout.
 
-    img: (B*V*S, C, A, A); lidar, radar: (B*S, C, A, A); gps: (B, 2, C); pos_emb: (1, T, C).
-    Token index = ((m*S + t)*A + y)*A + x for modality slot m (V image slots, then lidar, radar);
+    img: (B*V*S, C, va, ha); lidar, radar: (B*S, C, va, ha); gps: (B, 2, C); pos_emb: (1, T, C).
+    Token index = ((m*S + t)*va + y)*ha + x for modality slot m (V image slots, then lidar, radar);
     the two GPS tokens come last.
     """
     bz = lidar.shape[0] // seq_len
@@ -155,17 +155,19 @@ def bilinear_upsample(x: Tensor, scale: int) -> Tensor:
     """``F.interpolate(x, scale_factor=scale, mode='bilinear')`` with align_corners=False
     (model2_seq.py:521-523, 539-541, 558-560), restated from the sampling formula:
     src = max((i + 0.5)/scale - 0.5, 0); i0 = floor(src); i1 = min(i0 + 1, A - 1); lam = src - i0.
+    The taps are computed in x's precision (at least float32), so a float64 call is a float64 reference.
     """
     if scale == 1:
         return x
     n, c, a_h, a_w = x.shape
+    tdt = torch.promote_types(x.dtype, torch.float32)
 
     def taps(a, s):
-        dst = torch.arange(a * s, dtype=torch.float32)
+        dst = torch.arange(a * s, dtype=tdt)
         src = torch.clamp((dst + 0.5) / s - 0.5, min=0.0)
         i0 = src.floor().to(torch.long)
         i1 = torch.clamp(i0 + 1, max=a - 1)
-        lam = (src - i0.to(torch.float32)).to(x.dtype)
+        lam = (src - i0.to(tdt)).to(x.dtype)
         return i0.to(x.device), i1.to(x.device), lam.to(x.device)
 
     y0, y1, ly = taps(a_h, scale)

@@ -35,36 +35,64 @@ def _feat(n, c, h, w, g, dev, dtype=torch.float32, nhwc=False):
     return t
 
 
-STAGE_SHAPES = [  # (B, S, A, C, H)  H = A * scale
-    (2, 5, 8, 64, 64), (2, 5, 8, 128, 32), (1, 5, 8, 256, 16), (2, 5, 8, 512, 8),
-    (1, 2, 16, 64, 32),  # scaled config: 16x16 anchors
-    (1, 3, 4, 8, 24),    # odd scale 6, tiny C
-    (1, 2, 2, 8, 8),     # 8-pixel rows: four rows per load instruction in the narrow-plane upsample backward
+# (B, S, V, A_h, A_w, C, H, W): B samples of S frames, V camera views (image frames B*V*S, slots (V+2)*S), an A_h x A_w anchor
+# grid on H x W feature maps.  The comments name the NCHW code path each row reaches.  CT is the channel tile of the NCHW
+# kernels (nchw_channel_tile: 8 if H*W >= 1024 and C % 8 == 0, else 32); "pool" is the pooling loop of tokens_fwd_nchw_kernel
+# (transpose: kh = kw = 1; lanes-W: kw in {4, 8, 16, 32}, W % 4 == 0 and nct*A_h*W/4 % 32 == 0; generic otherwise), "up-bwd"
+# the path of upsample_add_bwd_nchw_kernel (transpose: H == A_h and W == A_w; direct: W/4 in {8, 16, 32}, W/A_w % 8 == 0 and
+# H/A_h >= 2 * 32/(W/4); narrow: W in {8, 16, 32} and H/A_h % (32/W) == 0; tiny: narrow with H <= 8 * 32/W; generic otherwise).
+# A tile with nct < CT channels loads and stores channel by channel.
+STAGE_SHAPES = [
+    (2, 5, 1, 8, 8, 64, 64, 64),     # stage 1: CT 8, pool lanes-W, up-bwd direct
+    (2, 5, 1, 8, 8, 128, 32, 32),    # stage 2: CT 8, pool lanes-W, up-bwd narrow
+    (1, 5, 1, 8, 8, 256, 16, 16),    # stage 3: CT 32, pool generic (kw = 2), up-bwd narrow tiny
+    (2, 5, 1, 8, 8, 512, 8, 8),      # stage 4: CT 32, pool transpose, up-bwd transpose
+    (1, 2, 1, 16, 16, 64, 32, 32),   # scaled config, 16x16 anchors: CT 8, pool generic, up-bwd narrow
+    (1, 3, 1, 4, 4, 8, 24, 24),      # odd scale 6, tiny C: CT 32 with one 8-channel tile (nct < CT), pool generic, up-bwd generic
+    (1, 2, 1, 2, 2, 8, 8, 8),        # 8-pixel rows: CT 32, nct 8, pool lanes-W, up-bwd narrow tiny (four rows per load)
+    # several camera views: image frame b*V*S + sl of slot sl < V*S (B = 2: at B = 1 that is sl whatever the frame stride)
+    (2, 2, 2, 8, 8, 64, 64, 64),     # stage-1 plane: CT 8, pool lanes-W, up-bwd direct
+    (2, 1, 3, 2, 4, 32, 8, 16),      # V = 3, rectangular: CT 32, pool lanes-W, up-bwd narrow tiny
+    # rectangular anchor grids, the same scale on both axes
+    (1, 2, 1, 4, 8, 64, 32, 64),     # scale 8: CT 8, pool lanes-W, up-bwd direct
+    (1, 2, 1, 2, 4, 32, 8, 16),      # scale 4: CT 32, pool lanes-W, up-bwd narrow tiny
+    (1, 2, 1, 8, 16, 128, 8, 16),    # stage-4 width, scale 1: CT 32, pool transpose, up-bwd transpose
+    (2, 2, 2, 2, 4, 8, 12, 24),      # scale 6, V = 2: CT 32, nct 8, pool generic, up-bwd generic
+    # partial channel tiles
+    (1, 2, 1, 4, 8, 40, 16, 32),     # C = 40 on 512 px: CT 32, tiles 32 + 8, pool lanes-W in both, up-bwd narrow
+    (1, 2, 1, 4, 4, 36, 32, 32),     # C = 36 on 1024 px (C % 8 != 0): CT 32, tiles 32 + 4, pool lanes-W in both, up-bwd direct
+    (1, 2, 1, 2, 2, 4, 8, 8),        # C = 4: CT 32, nct 4, pool generic with 16-byte loads (nct*A_h*W/4 = 16), up-bwd narrow tiny
+    # anisotropic: row scale 6, column scale 2 (the reference never builds it, the kernels take separate per-axis scales)
+    (1, 2, 1, 4, 8, 8, 24, 16),      # CT 32, nct 8, pool generic, up-bwd narrow (H/A_h = 6 is a multiple of 32/W = 2)
 ]
+
+
+def _frames(B, S, V):
+    return (B * V * S, B * S, B * S)
 
 
 @pytest.mark.parametrize("shape", STAGE_SHAPES)
 @pytest.mark.parametrize("variant", ["nchw_f32", "nchw_bf16", "nhwc_f32", "nhwc_bf16"])
 def test_tokens_fwd_bwd(K, cuda_dev, shape, variant):
-    B, S, A, C, H = shape
+    B, S, V, Ah, Aw, C, H, W = shape
     nhwc = variant.startswith("nhwc")
     dt = torch.bfloat16 if variant.endswith("bf16") else torch.float32
     g = _gen(1)
-    T = 3 * S * A * A + 2
-    feats = [_feat(B * S, C, H, H, g, cuda_dev, dt, nhwc) for _ in range(3)]
+    T = (V + 2) * S * Ah * Aw + 2
+    feats = [_feat(n, C, H, W, g, cuda_dev, dt, nhwc) for n in _frames(B, S, V)]
     gps = torch.randn(B, 2, C, generator=g).to(cuda_dev)
     pos = torch.randn(1, T, C, generator=g).to(cuda_dev)
-    geom = K.make_geom(B, S, 1, A, A, C, H, H, K.DSF_BF16 if dt == torch.bfloat16 else K.DSF_F32, K.DSF_NHWC if nhwc else K.DSF_NCHW)
+    geom = K.make_geom(B, S, V, Ah, Aw, C, H, W, K.DSF_BF16 if dt == torch.bfloat16 else K.DSF_F32, K.DSF_NHWC if nhwc else K.DSF_NCHW)
     x = torch.empty(B * T, C, device=cuda_dev)
     K.tokens_fwd(geom, feats[0], feats[1], feats[2], gps, pos, x)
     # oracle on the same (possibly bf16-rounded) inputs, fp32 math
     fr = [f.float().contiguous().requires_grad_(True) for f in feats]
     gr, pr = gps.clone().requires_grad_(True), pos.clone().requires_grad_(True)
-    ref = R.build_tokens(*[R.anchor_pool(f, A, A) for f in fr], gr, pr, S, 1)
+    ref = R.build_tokens(*[R.anchor_pool(f, Ah, Aw) for f in fr], gr, pr, S, V)
     assert_close(x.view(B, T, C), ref, 2e-6, 1e-6, "tokens_fwd")
     # backward
     dx = torch.randn(B, T, C, generator=g).to(cuda_dev)
-    dres = [_feat(B * S, C, H, H, g, cuda_dev, dt, nhwc) for _ in range(3)]
+    dres = [_feat(n, C, H, W, g, cuda_dev, dt, nhwc) for n in _frames(B, S, V)]
     ref.backward(dx)
     douts = [torch.empty_like(f) for f in feats]
     dgps = torch.empty(B, 2, C, device=cuda_dev)
@@ -77,7 +105,8 @@ def test_tokens_fwd_bwd(K, cuda_dev, shape, variant):
     assert_close(dpos, pr.grad, 2e-6, 1e-6, "dpos_emb")
     # without the residual-branch gradient
     K.tokens_bwd(geom, dx.contiguous(), None, douts, dgps, dpos)
-    assert_close(douts[1].float(), fr[1].grad, tol, 1e-6, "tokens_bwd no-res")
+    for d, f in zip(douts, fr):
+        assert_close(d.float(), f.grad, tol, 1e-6, "tokens_bwd no-res")
 
 
 @pytest.mark.parametrize("M,C", [(962, 64), (1924, 128), (300, 256), (11544, 512), (77, 1024), (10, 8)])
@@ -147,33 +176,34 @@ def test_pack_weights_and_relu_colsum(K, cuda_dev):
 
 
 @pytest.mark.parametrize("shape", STAGE_SHAPES)
-@pytest.mark.parametrize("variant", ["nchw_f32", "nchw_bf16", "nhwc_f32"])
+@pytest.mark.parametrize("variant", ["nchw_f32", "nchw_bf16", "nhwc_f32", "nhwc_bf16"])
 def test_upsample_add_fwd_bwd(K, cuda_dev, shape, variant):
     import torch.nn.functional as F
-    B, S, A, C, H = shape
+    B, S, V, Ah, Aw, C, H, W = shape
     nhwc = variant.startswith("nhwc")
     dt = torch.bfloat16 if variant.endswith("bf16") else torch.float32
     g = _gen(3)
-    T = 3 * S * A * A + 2
-    scale = H // A
-    feats = [_feat(B * S, C, H, H, g, cuda_dev, dt, nhwc) for _ in range(3)]
+    T = (V + 2) * S * Ah * Aw + 2
+    feats = [_feat(n, C, H, W, g, cuda_dev, dt, nhwc) for n in _frames(B, S, V)]
     y = torch.randn(B, T, C, generator=g).to(cuda_dev)
-    geom = K.make_geom(B, S, 1, A, A, C, H, H, K.DSF_BF16 if dt == torch.bfloat16 else K.DSF_F32, K.DSF_NHWC if nhwc else K.DSF_NCHW)
+    geom = K.make_geom(B, S, V, Ah, Aw, C, H, W, K.DSF_BF16 if dt == torch.bfloat16 else K.DSF_F32, K.DSF_NHWC if nhwc else K.DSF_NCHW)
     outs = [torch.empty_like(f) for f in feats]
     K.upsample_add_fwd(geom, y.view(B * T, C), feats, outs)
     yr = y.clone().requires_grad_(True)
-    maps = yr[:, :T - 2].reshape(B, 3 * S, A, A, C).permute(0, 1, 4, 2, 3)
+    maps = yr[:, :T - 2].reshape(B, (V + 2) * S, Ah, Aw, C).permute(0, 1, 4, 2, 3)
     refs = []
-    for m in range(3):
-        tok = maps[:, m * S:(m + 1) * S].reshape(B * S, C, A, A)
-        up = R.bilinear_upsample(tok, scale)
-        if scale > 1:
-            assert_close(up, F.interpolate(tok, scale_factor=scale, mode="bilinear"), 1e-6, 1e-7, "oracle vs F.interpolate")
+    for m, (lo, hi) in enumerate(((0, V * S), (V * S, (V + 1) * S), ((V + 1) * S, (V + 2) * S))):
+        tok = maps[:, lo:hi].reshape(-1, C, Ah, Aw)
+        # F.interpolate with the output size samples each axis with step A / H; where both axes share one integer scale this is
+        # the oracle's restatement of the reference's F.interpolate(scale_factor=s) call
+        up = F.interpolate(tok, size=(H, W), mode="bilinear", align_corners=False)
+        if H // Ah == W // Aw:
+            assert_close(R.bilinear_upsample(tok, H // Ah), up, 1e-6, 1e-7, "oracle vs F.interpolate")
         refs.append(feats[m].float() + up)
     tol = 1e-2 if dt == torch.bfloat16 else 1e-6
     for o, r in zip(outs, refs):
         assert_close(o.float(), r, tol, 1e-6, "upsample_add_fwd")
-    douts = [_feat(B * S, C, H, H, g, cuda_dev, dt, nhwc) for _ in range(3)]
+    douts = [_feat(n, C, H, W, g, cuda_dev, dt, nhwc) for n in _frames(B, S, V)]
     dgps = torch.randn(B, 2, C, generator=g).to(cuda_dev)
     sum((r * d.float()).sum() for r, d in zip(refs, douts)).backward()
     dy = torch.empty(B * T, C, device=cuda_dev)

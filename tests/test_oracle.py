@@ -93,6 +93,60 @@ def test_token_order_and_count():
     img = torch.arange(B * S * C * A * A, dtype=torch.float32).reshape(B * S, C, A, A)
     x = R.build_tokens(img, lid, rad, gps, torch.zeros(1, 962, C), S, 1)
     assert x[1, 2 * 64 + 3 * 8 + 5, 4] == img[1 * S + 2, 4, 3, 5]
+    # several camera views and a rectangular anchor grid, token by token against the reference's stacking
+    # (model2_seq.py:256-272 and 489-493): image_tensor.view(bz, n_views * seq_len, -1, h, w), then lidar, then radar, each
+    # slot flattened in (y, x) raster order.  Every element is distinct, so a swapped axis or a wrong frame cannot match.
+    B, S, V, va, ha, C = 2, 3, 2, 2, 5, 3
+    T = (V + 2) * S * va * ha + 2
+    n = [B * V * S, B * S, B * S]
+    maps = []
+    for j, nf in enumerate(n):
+        maps.append(1000 * j + torch.arange(nf * C * va * ha, dtype=torch.float64).reshape(nf, C, va, ha))
+    gps = -1 - torch.arange(B * 2 * C, dtype=torch.float64).reshape(B, 2, C)
+    x = R.build_tokens(maps[0], maps[1], maps[2], gps, torch.zeros(1, T, C, dtype=torch.float64), S, V)
+    assert x.shape == (B, T, C)
+    for b in range(B):
+        for m in range(V + 2):
+            for t in range(S):
+                sl = m * S + t
+                if sl < V * S:
+                    frame = maps[0][b * V * S + sl]
+                elif sl < (V + 1) * S:
+                    frame = maps[1][b * S + sl - V * S]
+                else:
+                    frame = maps[2][b * S + sl - (V + 1) * S]
+                for y in range(va):
+                    for xx in range(ha):
+                        assert torch.equal(x[b, ((m * S + t) * va + y) * ha + xx], frame[:, y, xx]), (b, m, t, y, xx)
+        assert torch.equal(x[b, T - 2:], gps[b])
+
+
+@pytest.mark.parametrize("hw,va,ha", [((16, 32), 4, 8), ((8, 32), 2, 4), ((4, 8), 4, 8), ((12, 20), 3, 5),
+                                      ((13, 22), 4, 8)], ids=["s4", "s4-wide", "s1", "s4-odd-grid", "ragged"])
+def test_anchor_pool_matches_adaptive_avg_pool_on_rectangular_maps(hw, va, ha):
+    """nn.AdaptiveAvgPool2d((vert_anchors, horz_anchors)) (model2_seq.py:414), float64; "ragged": the windows of a map that is
+    no multiple of the grid overlap and differ in size."""
+    x = torch.randn(3, 5, *hw, generator=torch.Generator().manual_seed(41), dtype=torch.float64)
+    ref = torch.nn.AdaptiveAvgPool2d((va, ha))(x)
+    got = R.anchor_pool(x, va, ha)
+    assert got.shape == (3, 5, va, ha)
+    assert float((got - ref).abs().max()) < 1e-14
+
+
+@pytest.mark.parametrize("scale", [1, 2, 4, 6, 8])
+@pytest.mark.parametrize("va,ha", [(4, 8), (8, 4), (3, 5)])
+def test_bilinear_upsample_matches_interpolate_in_float64(scale, va, ha):
+    """F.interpolate(scale_factor=s, mode='bilinear', align_corners=False) (model2_seq.py:521-523) on rectangular grids, in
+    float64: the restatement is a float64 reference (taps included), so it agrees to rounding of double."""
+    import torch.nn.functional as F
+    x = torch.randn(2, 3, va, ha, generator=torch.Generator().manual_seed(43), dtype=torch.float64)
+    got = R.bilinear_upsample(x, scale)
+    ref = F.interpolate(x, scale_factor=scale, mode="bilinear", align_corners=False)
+    assert got.dtype == torch.float64 and got.shape == (2, 3, va * scale, ha * scale)
+    assert float((got - ref).abs().max()) < 1e-12
+    # the same sampling expressed with the output size, as the fused kernels see it (source step A / H per axis)
+    ref_size = F.interpolate(x, size=(va * scale, ha * scale), mode="bilinear", align_corners=False)
+    assert float((got - ref_size).abs().max()) < 1e-12
 
 
 def test_init_law_matches_reference():
