@@ -23,7 +23,7 @@ SYMBOLS = [
     "dsf_version", "dsf_last_error", "dsf_launch_count", "dsf_check_device", "dsf_set_pdl", "dsf_set_sm_margin", "dsf_dropout_inplace", "dsf_tokens_fwd", "dsf_tokens_bwd",
     "dsf_layernorm_fwd", "dsf_layernorm_bwd", "dsf_gemm_bf16_nt", "dsf_gemm_bf16_tn", "dsf_gemm_set_impl", "dsf_gemm_f32",
     "dsf_colsum", "dsf_relu_bwd", "dsf_relu_bwd_colsum", "dsf_pack_block_weights", "dsf_softmax_fwd", "dsf_softmax_bwd", "dsf_attn_fwd", "dsf_attn_bwd", "dsf_attn_bwd_parts", "dsf_attn_set_impl", "dsf_attn_drop_words",
-    "dsf_upsample_add_fwd", "dsf_upsample_add_bwd", "dsf_cast_f32_bf16", "dsf_opt_tiles", "dsf_adamw_ema_pack", "dsf_opt_upload_table", "dsf_chain_fwd", "dsf_chain_bwd",
+    "dsf_upsample_add_fwd", "dsf_upsample_add_bwd", "dsf_cast_f32_bf16", "dsf_opt_tiles", "dsf_adamw_ema_pack", "dsf_opt_upload_table", "dsf_chain_fwd",
     "dsf_stem_pack", "dsf_tail_fwd", "dsf_tail_bwd",
 ]
 
@@ -99,7 +99,6 @@ def lib():
             "dsf_upsample_add_bwd": [POINTER(Geom), P, P, P, P, P, P],
             "dsf_cast_f32_bf16": [P, P, c_int64, P],
             "dsf_chain_fwd": [P] * 25 + [c_int32, c_int32, c_float, P],
-            "dsf_chain_bwd": [P] * 32 + [c_int32, c_int32, c_int32, c_int32, P],
             "dsf_stem_pack": [P, c_int32, c_int32, c_int32, c_int32, c_int32, P, P, P, c_int32, c_int32, P],
             "dsf_tail_fwd": [P, P, P, P, P] + [c_int32] * 9 + [P],
             "dsf_tail_bwd": [P, P, P, P, P] + [c_int32] * 9 + [P],
@@ -338,19 +337,6 @@ def chain_fwd(y, x_in, wp, w1, w2, wqkv_next, bp, b1, b2, bqkv_next, ln2_g, ln2_
     _chk(lib().dsf_chain_fwd(_p(y), _p(x_in), _p(wp), _p(w1), _p(w2), _p(wqkv_next), _p(bp), _p(b1), _p(b2), _p(bqkv_next), _p(ln2_g), _p(ln2_b),
                              _p(lnn_g), _p(lnn_b), _p(x_mid), _p(x_out), _p(h2), _p(a), _p(h_next), _p(qkv_next), _p(yf), _p(mean2), _p(rstd2),
                              _p(mean_next), _p(rstd_next), M, C, eps, _stream()), "dsf_chain_fwd")
-
-
-def chain_bwd(M, C, T, nh, half_a=None, half_b=None, dx_in=None, dx_f32=None):
-    """n_embd 64 / 128: the row-local backward chain between two attention backward calls in ONE launch (see include/dsfuse.h).
-    half_a = dict(dqkv, dx_mid_in, x_in, mean1, rstd1, g1, wqkv_t, dg1, dbe1, dbqkv, db2_prev) of block i (or None);
-    half_b = dict(a, y, x_mid, mean2, rstd2, g2, w2_t, w1_t, wp_t, dxa, da, dxm, dy, dx_mid_out, delta, db1, dg2, dbe2, dbp) of block
-    i - 1 (or None).  dx_in: fp32 dx when there is no half A; dx_f32: fp32 dx destination when there is no half B."""
-    A, B = half_a or {}, half_b or {}
-    ga, gb = (lambda k: _p(A.get(k))), (lambda k: _p(B.get(k)))
-    _chk(lib().dsf_chain_bwd(ga("dqkv"), ga("dx_mid_in"), ga("x_in"), ga("mean1"), ga("rstd1"), ga("g1"), ga("wqkv_t"), ga("dg1"), ga("dbe1"),
-                             ga("dbqkv"), ga("db2_prev"), _p(dx_f32), _p(dx_in), gb("a"), gb("y"), gb("x_mid"), gb("mean2"), gb("rstd2"), gb("g2"),
-                             gb("w2_t"), gb("w1_t"), gb("wp_t"), gb("dxa"), gb("da"), gb("dxm"), gb("dy"), gb("dx_mid_out"), gb("delta"), gb("db1"),
-                             gb("dg2"), gb("dbe2"), gb("dbp"), M, C, T, nh, _stream()), "dsf_chain_bwd")
 
 
 def opt_upload_table(dst_dev, src_pinned):

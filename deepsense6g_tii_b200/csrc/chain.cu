@@ -1,4 +1,4 @@
-// Row-local chains of the transformer block for the narrow stages (n_embd 64 / 128), one launch each.
+// Row-local forward chain of the transformer block for the narrow stages (n_embd 64 / 128), one launch per block.
 //
 // At n_embd <= 128 every Linear of model2_seq.py:113-134 is a few microseconds of tensor work and each separate kernel of the
 // chain  proj -> +residual -> LayerNorm -> mlp.0 -> ReLU -> mlp.2 -> +residual -> LayerNorm(next block) -> QKV(next block)
@@ -110,8 +110,7 @@ __device__ __forceinline__ void warp_layernorm(float (&v)[NT][4], const float* _
 // block (the weights are fetched once, up front), at 128 it runs four 36 KB chunks deep, so a step never waits for L2 latency.
 constexpr int CH_WARPS = 5, CH_THREADS = CH_WARPS * 32, CH_ROWS = CH_WARPS * 16;
 template <int C> struct ChainCfg {
-  static constexpr int NS_FWD = C == 64 ? 8 : 4, NS_BWD = 4;
-  static constexpr bool STAGE_BWD = C == 64;   // backward: fp32 row tiles (dx_mid / x_in / x_mid / dx_in) and y staged in shared memory (fits at 64 only)
+  static constexpr int NS_FWD = C == 64 ? 8 : 4;
 };
 
 template <int C>
@@ -333,411 +332,6 @@ static int launch_chain_fwd(const ChainFwdArgs& a, cudaStream_t st) {
   return check_launch("chain_fwd");
 }
 
-
-// =============================================================================================== backward chain
-// Between the attention backward of block i and the attention backward of block i - 1 everything is row-local again:
-//   half A (block i):      dh1 = dqkv Wqkv            -> LayerNorm backward of ln1 (+ dx_mid of block i)  -> dx  (= d x_out of block i-1)
-//   half B (block i - 1):  da = (dx W2) o (a > 0)     -> dh2 = da W1 -> LayerNorm backward of ln2 (+ dx)   -> dx_mid
-//                          dy = dx_mid Wp             -> delta = rowsum_head(dy o y)   (what the attention backward starts from)
-// plus every column reduction that falls out of these rows: dgamma / dbeta of both LayerNorms and the bias gradients of
-// QKV (colsum dqkv), mlp.2 (colsum dx), mlp.0 (colsum da), proj (colsum dx_mid).  The weight-gradient GEMMs stay separate
-// launches (on the side stream) and read the bf16 copies this kernel writes: dxa, da, dxm (and dqkv, which it only reads).
-// Either half can be absent: the first launch of a backward has no half A (dx comes from ln_f's backward), the last one has
-// no half B (its dx goes to the token kernel in fp32).
-struct ChainBwdArgs {
-  // half A
-  const __nv_bfloat16* dqkv;      // (M, 3C) or NULL
-  const float* dx_mid_in;         // (M, C)  gradient of block i's x_mid (residual branch)
-  const float* x_in;              // (M, C)  block i's input, with mean1 / rstd1 / g1 of its ln1
-  const float *mean1, *rstd1, *g1;
-  const __nv_bfloat16* wqkv_t;    // (C, 3C)
-  float *dg1, *dbe1, *dbqkv;      // (C), (C), (3C)  accumulated
-  float* db2_prev;                // (C) bias gradient of block i-1's mlp.2 (NULL for block 0)
-  float* dx_f32;                  // (M, C) fp32 dx, written only when there is no half B
-  // half B
-  const float* dx_in;             // (M, C) fp32 dx when there is no half A
-  const __nv_bfloat16 *a, *y;     // (M, F), (M, C) saved by the forward of block i-1; a == NULL: no half B
-  const float *x_mid, *mean2, *rstd2, *g2;
-  const __nv_bfloat16 *w2_t, *w1_t, *wp_t;   // (F, C), (C, F), (C, C)
-  __nv_bfloat16 *dxa, *da, *dxm, *dy;        // bf16 operands of the weight-gradient GEMMs / the attention backward
-  float *dx_mid_out, *delta;                 // (M, C); (B, nh, T)
-  float *db1, *dg2, *dbe2, *dbp;             // (F), (C), (C), (C) accumulated
-  int M, T, nh;
-};
-
-// column sums over the 16 rows of a warp (accumulator layout) -> shared-memory accumulator red[col] (one atomic per column and warp)
-template <int NTL>
-__device__ __forceinline__ void warp_colsum(const float (&v)[NTL][4], float* red, int col0, int lane) {
-#pragma unroll
-  for (int j = 0; j < NTL; ++j) {
-    float s0 = v[j][0] + v[j][2], s1 = v[j][1] + v[j][3];
-#pragma unroll
-    for (int o = 4; o < 32; o <<= 1) { s0 += __shfl_xor_sync(0xffffffffu, s0, o); s1 += __shfl_xor_sync(0xffffffffu, s1, o); }
-    if (lane < 4) { atomicAdd(red + col0 + j * 8 + 2 * lane, s0); atomicAdd(red + col0 + j * 8 + 2 * lane + 1, s1); }
-  }
-}
-
-// LayerNorm backward of the 16 rows a warp holds: dh (gradient of the LayerNorm output, accumulator layout) is replaced by
-// dx = add + rstd * (g*dh - mean(g*dh) - xhat * mean(g*dh*xhat)); dgamma += dh * xhat and dbeta += dh go to red_g / red_b.
-template <int NT>
-__device__ __forceinline__ void warp_layernorm_bwd(float (&dh)[NT][4], const float (&add)[NT][4], const float* x_lo, const float* x_hi, const float* gamma,
-                                                   float mean_lo, float rstd_lo, float mean_hi, float rstd_hi, bool ok_lo, bool ok_hi,
-                                                   int t, int lane, float* red_g, float* red_b) {
-  constexpr int C = NT * 8;
-  constexpr float inv_c = 1.0f / (float)C;
-  float xh[NT][4];
-  float s1_lo = 0.f, s2_lo = 0.f, s1_hi = 0.f, s2_hi = 0.f;
-#pragma unroll
-  for (int j = 0; j < NT; ++j) {
-    const int n = j * 8 + 2 * t;
-    float2 x0 = make_float2(mean_lo, mean_lo), x1 = make_float2(mean_hi, mean_hi);
-    if (ok_lo) x0 = *reinterpret_cast<const float2*>(x_lo + n);
-    if (ok_hi) x1 = *reinterpret_cast<const float2*>(x_hi + n);
-    xh[j][0] = (x0.x - mean_lo) * rstd_lo; xh[j][1] = (x0.y - mean_lo) * rstd_lo;
-    xh[j][2] = (x1.x - mean_hi) * rstd_hi; xh[j][3] = (x1.y - mean_hi) * rstd_hi;
-  }
-  {  // dgamma, dbeta (before dh is overwritten)
-    float dg[NT][4];
-#pragma unroll
-    for (int j = 0; j < NT; ++j) {
-#pragma unroll
-      for (int k = 0; k < 4; ++k) dg[j][k] = dh[j][k] * xh[j][k];
-    }
-    warp_colsum<NT>(dg, red_g, 0, lane);
-    warp_colsum<NT>(dh, red_b, 0, lane);
-  }
-#pragma unroll
-  for (int j = 0; j < NT; ++j) {
-    const float2 gm = *reinterpret_cast<const float2*>(gamma + j * 8 + 2 * t);
-    dh[j][0] *= gm.x; dh[j][1] *= gm.y; dh[j][2] *= gm.x; dh[j][3] *= gm.y;
-    s1_lo += dh[j][0] + dh[j][1]; s2_lo += dh[j][0] * xh[j][0] + dh[j][1] * xh[j][1];
-    s1_hi += dh[j][2] + dh[j][3]; s2_hi += dh[j][2] * xh[j][2] + dh[j][3] * xh[j][3];
-  }
-#pragma unroll
-  for (int o = 1; o < 4; o <<= 1) {
-    s1_lo += __shfl_xor_sync(0xffffffffu, s1_lo, o); s2_lo += __shfl_xor_sync(0xffffffffu, s2_lo, o);
-    s1_hi += __shfl_xor_sync(0xffffffffu, s1_hi, o); s2_hi += __shfl_xor_sync(0xffffffffu, s2_hi, o);
-  }
-  const float m1_lo = s1_lo * inv_c, m2_lo = s2_lo * inv_c, m1_hi = s1_hi * inv_c, m2_hi = s2_hi * inv_c;
-#pragma unroll
-  for (int j = 0; j < NT; ++j) {
-    dh[j][0] = add[j][0] + rstd_lo * (dh[j][0] - m1_lo - xh[j][0] * m2_lo);
-    dh[j][1] = add[j][1] + rstd_lo * (dh[j][1] - m1_lo - xh[j][1] * m2_lo);
-    dh[j][2] = add[j][2] + rstd_hi * (dh[j][2] - m1_hi - xh[j][2] * m2_hi);
-    dh[j][3] = add[j][3] + rstd_hi * (dh[j][3] - m1_hi - xh[j][3] * m2_hi);
-  }
-}
-
-template <int C>
-__global__ void __launch_bounds__(CH_THREADS, 1) chain_bwd_kernel(ChainBwdArgs p) {
-  constexpr int NS = ChainCfg<C>::NS_BWD;
-  constexpr int F = 4 * C, NT = C / 8, KS = C / 16;
-  constexpr int LDW = C + 8, LDW2 = 64 + 8;
-  constexpr int N_QKV = 3 * C / 64, N_MLP = F / 64;
-  constexpr int ACT = CH_WARPS * 16 * LDW2;                                   // per-warp [16][64] activation sub-tiles of one step
-  constexpr int WCH = (64 * LDW + C * LDW2 > C * LDW) ? 64 * LDW + C * LDW2 : C * LDW;
-  constexpr int CHUNK = WCH + ACT;
-  extern __shared__ __align__(16) uint8_t smem_raw[];
-  __nv_bfloat16* ring = reinterpret_cast<__nv_bfloat16*>(smem_raw);   // [NS][CHUNK]
-  float* red = reinterpret_cast<float*>(ring + NS * CHUNK);            // column accumulators: [7][C] + [3C] + [F]
-  float *red_g1 = red, *red_b1 = red + C, *red_b2p = red + 2 * C, *red_g2 = red + 3 * C, *red_be2 = red + 4 * C, *red_bp = red + 5 * C;
-  float *red_bqkv = red + 6 * C, *red_db1 = red + 9 * C;
-  // n_embd 64: the row tiles the epilogues read (dx_mid_in | dx_in, x_in, x_mid: fp32; y: bf16) are staged per warp by the first
-  // cp.async group, like the forward kernel does (at 128 they do not fit next to the ring and are read from global memory)
-  constexpr bool STG = ChainCfg<C>::STAGE_BWD;
-  constexpr int LDX = C + 8;
-  float* vec = red + 9 * C + F;                                          // g1 | g2
-  float* st_add = vec + 2 * C;                                           // [CH_WARPS][16][LDX] dx_mid_in (half A) or dx_in (no half A)
-  float* st_x1 = st_add + (STG ? CH_WARPS * 16 * LDX : 0);               // x_in
-  float* st_x2 = st_x1 + (STG ? CH_WARPS * 16 * LDX : 0);                // x_mid
-  __nv_bfloat16* st_y = reinterpret_cast<__nv_bfloat16*>(st_x2 + (STG ? CH_WARPS * 16 * LDX : 0));   // [CH_WARPS][16][LDW]
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, t = lane & 3;
-  const int row0 = blockIdx.x * CH_ROWS + warp * 16;
-  const int r_lo = row0 + g, r_hi = r_lo + 8;
-  const bool ok_lo = r_lo < p.M, ok_hi = r_hi < p.M;
-  const bool half_a = p.dqkv != nullptr, half_b = p.a != nullptr;
-  const int n_a = half_a ? N_QKV : 0, n_b = half_b ? N_MLP + 1 : 0;
-  const int n_steps = n_a + n_b;
-  for (int i = tid; i < 9 * C + F; i += CH_THREADS) red[i] = 0.f;
-  pdl_trigger();
-  pdl_wait();
-
-  auto prefetch = [&](int s) {
-    __nv_bfloat16* dst = ring + (s % NS) * CHUNK;
-    if (s < n_a) {   // half A, k-chunk s of the contraction over 3C: wqkv_t[:, 64 s ..] as [C][64] + this warp's dqkv columns
-      for (int i = tid; i < C * 8; i += CH_THREADS) { const int r = i >> 3, c8 = i & 7; cp_async16(dst + r * LDW2 + c8 * 8, p.wqkv_t + (size_t)r * (3 * C) + s * 64 + c8 * 8); }
-      __nv_bfloat16* act = dst + WCH + warp * 16 * LDW2;
-      for (int i = lane; i < 16 * 8; i += 32) {
-        const int r = i >> 3, c8 = i & 7;
-        if (row0 + r < p.M) cp_async16(act + r * LDW2 + c8 * 8, p.dqkv + (size_t)(row0 + r) * (3 * C) + s * 64 + c8 * 8);
-        else *reinterpret_cast<uint4*>(act + r * LDW2 + c8 * 8) = make_uint4(0u, 0u, 0u, 0u);
-      }
-    } else if (s < n_a + N_MLP) {   // half B, hidden chunk hc: w2_t rows [64 hc, +64) x C and w1_t[:, 64 hc ..] as [C][64]
-      const int hc = s - n_a;
-      for (int i = tid; i < 64 * (C / 8); i += CH_THREADS) { const int r = i / (C / 8), c8 = i % (C / 8); cp_async16(dst + r * LDW + c8 * 8, p.w2_t + (size_t)(hc * 64 + r) * C + c8 * 8); }
-      __nv_bfloat16* d2 = dst + 64 * LDW;
-      for (int i = tid; i < C * 8; i += CH_THREADS) { const int r = i >> 3, c8 = i & 7; cp_async16(d2 + r * LDW2 + c8 * 8, p.w1_t + (size_t)r * F + hc * 64 + c8 * 8); }
-      __nv_bfloat16* act = dst + WCH + warp * 16 * LDW2;   // this warp's 64 columns of the saved mlp.0 output (ReLU decisions)
-      for (int i = lane; i < 16 * 8; i += 32) {
-        const int r = i >> 3, c8 = i & 7;
-        if (row0 + r < p.M) cp_async16(act + r * LDW2 + c8 * 8, p.a + (size_t)(row0 + r) * F + hc * 64 + c8 * 8);
-        else *reinterpret_cast<uint4*>(act + r * LDW2 + c8 * 8) = make_uint4(0u, 0u, 0u, 0u);
-      }
-    } else {   // proj data gradient: wp_t (C, C)
-      for (int i = tid; i < C * (C / 8); i += CH_THREADS) { const int r = i / (C / 8), c8 = i % (C / 8); cp_async16(dst + r * LDW + c8 * 8, p.wp_t + (size_t)r * C + c8 * 8); }
-    }
-    cp_async_commit();
-  };
-  auto acquire = [&](int s) {   // see chain_fwd_kernel
-    if (s + NS - 1 < n_steps) prefetch(s + NS - 1); else cp_async_commit();
-    cp_async_wait<NS - 1>();
-    __syncthreads();
-  };
-  auto release = [&](int s) {
-    if (s + NS < n_steps) __syncthreads();
-  };
-  // row statistics: four scalars per thread, loaded now and consumed many steps later
-  const float m1_lo = half_a && ok_lo ? p.mean1[r_lo] : 0.f, s1_lo = half_a && ok_lo ? p.rstd1[r_lo] : 0.f;
-  const float m1_hi = half_a && ok_hi ? p.mean1[r_hi] : 0.f, s1_hi = half_a && ok_hi ? p.rstd1[r_hi] : 0.f;
-  const float m2_lo = half_b && ok_lo ? p.mean2[r_lo] : 0.f, s2_lo = half_b && ok_lo ? p.rstd2[r_lo] : 0.f;
-  const float m2_hi = half_b && ok_hi ? p.mean2[r_hi] : 0.f, s2_hi = half_b && ok_hi ? p.rstd2[r_hi] : 0.f;
-  {   // first cp.async group: LayerNorm gains and (n_embd 64) the row tiles
-    if (half_a) { for (int i = tid; i < C / 4; i += CH_THREADS) cp_async16(vec + i * 4, p.g1 + i * 4); }
-    if (half_b) { for (int i = tid; i < C / 4; i += CH_THREADS) cp_async16(vec + C + i * 4, p.g2 + i * 4); }
-    if (STG) {
-      auto stage_f32 = [&](float* dstw, const float* src) {
-        for (int i = lane; i < 16 * (C / 4); i += 32) {
-          const int r = i / (C / 4), c4 = i % (C / 4);
-          if (row0 + r < p.M) cp_async16(dstw + r * LDX + c4 * 4, src + (size_t)(row0 + r) * C + c4 * 4);
-          else *reinterpret_cast<float4*>(dstw + r * LDX + c4 * 4) = make_float4(0.f, 0.f, 0.f, 0.f);
-        }
-      };
-      stage_f32(st_add + warp * 16 * LDX, half_a ? p.dx_mid_in : p.dx_in);
-      if (half_a) stage_f32(st_x1 + warp * 16 * LDX, p.x_in);
-      if (half_b) {
-        stage_f32(st_x2 + warp * 16 * LDX, p.x_mid);
-        __nv_bfloat16* yb = st_y + warp * 16 * LDW;
-        for (int i = lane; i < 16 * (C / 8); i += 32) {
-          const int r = i / (C / 8), c8 = i % (C / 8);
-          if (row0 + r < p.M) cp_async16(yb + r * LDW + c8 * 8, p.y + (size_t)(row0 + r) * C + c8 * 8);
-          else *reinterpret_cast<uint4*>(yb + r * LDW + c8 * 8) = make_uint4(0u, 0u, 0u, 0u);
-        }
-      }
-    }
-  }
-  for (int q = 0; q < NS - 1; ++q) { if (q < n_steps) prefetch(q); else cp_async_commit(); }
-  // row pointers of this thread's two rows in the staged tiles (n_embd 64) or in global memory
-  const float* add_lo = STG ? st_add + (warp * 16 + g) * LDX : (half_a ? p.dx_mid_in : p.dx_in) + (size_t)r_lo * C;
-  const float* add_hi = STG ? add_lo + 8 * LDX : (half_a ? p.dx_mid_in : p.dx_in) + (size_t)r_hi * C;
-  const bool rd_lo = STG || ok_lo, rd_hi = STG || ok_hi;   // staged tiles are zero-filled past M
-
-  float dx[NT][4];   // gradient of the residual stream between the two halves
-  int s = 0;
-  if (half_a) {
-    // ---------------------------------------------------------------- half A: dh1 = dqkv Wqkv, colsum(dqkv), ln1 backward
-#pragma unroll
-    for (int j = 0; j < NT; ++j) { dx[j][0] = dx[j][1] = dx[j][2] = dx[j][3] = 0.f; }
-    for (; s < n_a; ++s) {
-      acquire(s);
-      const __nv_bfloat16* wc = ring + (s % NS) * CHUNK;
-      const __nv_bfloat16* act = wc + WCH + warp * 16 * LDW2;
-      uint32_t afr[4][4];
-#pragma unroll
-      for (int kk = 0; kk < 4; ++kk) ldmatrix_x4(afr[kk], act + (size_t)((lane & 7) + (((lane >> 3) & 1) << 3)) * LDW2 + kk * 16 + ((lane >> 4) << 3));
-      warp_gemm<NT, 4>(dx, afr, wc, LDW2, lane);
-      {  // bias gradient of the fused QKV Linear: column sums of this warp's [16][64] dqkv sub-tile
-        float cs[8][4];
-#pragma unroll
-        for (int kk = 0; kk < 4; ++kk) {
-          // A fragment registers: [0] row g, k 2t..; [1] row g+8, k 2t..; [2] row g, k 2t+8..; [3] row g+8, k 2t+8..
-#pragma unroll
-          for (int q = 0; q < 4; ++q) {
-            const float2 f = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&afr[kk][q]));
-            cs[kk * 2 + (q >> 1)][(q & 1) * 2] = f.x;
-            cs[kk * 2 + (q >> 1)][(q & 1) * 2 + 1] = f.y;
-          }
-        }
-        warp_colsum<8>(cs, red_bqkv, s * 64, lane);
-      }
-      release(s);
-    }
-    float add[NT][4];
-#pragma unroll
-    for (int j = 0; j < NT; ++j) {
-      const int n = j * 8 + 2 * t;
-      float2 a0 = make_float2(0.f, 0.f), a1 = make_float2(0.f, 0.f);
-      if (rd_lo) a0 = *reinterpret_cast<const float2*>(add_lo + n);
-      if (rd_hi) a1 = *reinterpret_cast<const float2*>(add_hi + n);
-      add[j][0] = a0.x; add[j][1] = a0.y; add[j][2] = a1.x; add[j][3] = a1.y;
-    }
-    const float* x1_lo = STG ? st_x1 + (warp * 16 + g) * LDX : p.x_in + (size_t)r_lo * C;
-    const float* x1_hi = STG ? x1_lo + 8 * LDX : p.x_in + (size_t)r_hi * C;
-    warp_layernorm_bwd<NT>(dx, add, x1_lo, x1_hi, vec, m1_lo, s1_lo, m1_hi, s1_hi, rd_lo, rd_hi, t, lane, red_g1, red_b1);
-    if (p.db2_prev) warp_colsum<NT>(dx, red_b2p, 0, lane);
-    if (!half_b) {
-#pragma unroll
-      for (int j = 0; j < NT; ++j) {
-        const int n = j * 8 + 2 * t;
-        if (ok_lo) *reinterpret_cast<float2*>(p.dx_f32 + (size_t)r_lo * C + n) = make_float2(dx[j][0], dx[j][1]);
-        if (ok_hi) *reinterpret_cast<float2*>(p.dx_f32 + (size_t)r_hi * C + n) = make_float2(dx[j][2], dx[j][3]);
-      }
-    }
-  } else {
-    if (STG) { cp_async_wait<NS - 2>(); __syncwarp(); }   // the first group (with this warp's own staged rows) has landed
-#pragma unroll
-    for (int j = 0; j < NT; ++j) {
-      const int n = j * 8 + 2 * t;
-      float2 a0 = make_float2(0.f, 0.f), a1 = make_float2(0.f, 0.f);
-      if (rd_lo) a0 = *reinterpret_cast<const float2*>(add_lo + n);
-      if (rd_hi) a1 = *reinterpret_cast<const float2*>(add_hi + n);
-      dx[j][0] = a0.x; dx[j][1] = a0.y; dx[j][2] = a1.x; dx[j][3] = a1.y;
-    }
-  }
-
-  if (half_b) {
-    // ---------------------------------------------------------------- half B: mlp backward, ln2 backward, proj data gradient
-    uint32_t xfr[KS][4];   // bf16 A fragments of dx (also the weight-gradient operand dxa of mlp.2)
-#pragma unroll
-    for (int j = 0; j < NT; ++j) {
-      const uint32_t lo = pack2(dx[j][0], dx[j][1]), hi = pack2(dx[j][2], dx[j][3]);
-      xfr[j >> 1][(j & 1) * 2] = lo;
-      xfr[j >> 1][(j & 1) * 2 + 1] = hi;
-      const int n = j * 8 + 2 * t;
-      if (half_a) {   // (without half A the caller's ln_f backward has already written dxa)
-        if (ok_lo) *reinterpret_cast<uint32_t*>(p.dxa + (size_t)r_lo * C + n) = lo;
-        if (ok_hi) *reinterpret_cast<uint32_t*>(p.dxa + (size_t)r_hi * C + n) = hi;
-      }
-    }
-    float dh2[NT][4];
-#pragma unroll
-    for (int j = 0; j < NT; ++j) { dh2[j][0] = dh2[j][1] = dh2[j][2] = dh2[j][3] = 0.f; }
-    for (int hc = 0; hc < N_MLP; ++hc, ++s) {
-      acquire(s);
-      const __nv_bfloat16* w2c = ring + (s % NS) * CHUNK;
-      const __nv_bfloat16* w1c = w2c + 64 * LDW;
-      const __nv_bfloat16* am_lo = w2c + WCH + (warp * 16 + g) * LDW2;   // saved mlp.0 outputs of this thread's two rows, this chunk
-      const __nv_bfloat16* am_hi = am_lo + 8 * LDW2;
-      float dd[8][4];
-#pragma unroll
-      for (int j = 0; j < 8; ++j) { dd[j][0] = dd[j][1] = dd[j][2] = dd[j][3] = 0.f; }
-      warp_gemm<8, KS>(dd, xfr, w2c, LDW, lane);
-      uint32_t dfr[4][4];
-#pragma unroll
-      for (int j = 0; j < 8; ++j) {   // ReLU backward with the saved activations (model2_seq.py:123)
-        const int n = hc * 64 + j * 8 + 2 * t;
-        const uint32_t m0 = *reinterpret_cast<const uint32_t*>(am_lo + j * 8 + 2 * t);
-        const uint32_t m1 = *reinterpret_cast<const uint32_t*>(am_hi + j * 8 + 2 * t);
-        const float2 a0 = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&m0));
-        const float2 a1 = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&m1));
-        dd[j][0] = a0.x > 0.f ? dd[j][0] : 0.f; dd[j][1] = a0.y > 0.f ? dd[j][1] : 0.f;
-        dd[j][2] = a1.x > 0.f ? dd[j][2] : 0.f; dd[j][3] = a1.y > 0.f ? dd[j][3] : 0.f;
-        const uint32_t lo = pack2(dd[j][0], dd[j][1]), hi = pack2(dd[j][2], dd[j][3]);
-        dfr[j >> 1][(j & 1) * 2] = lo;
-        dfr[j >> 1][(j & 1) * 2 + 1] = hi;
-        if (ok_lo) *reinterpret_cast<uint32_t*>(p.da + (size_t)r_lo * F + n) = lo;
-        if (ok_hi) *reinterpret_cast<uint32_t*>(p.da + (size_t)r_hi * F + n) = hi;
-        // the bias gradient is the column sum of the bf16 tensor the weight-gradient GEMM reads
-        const float2 q0 = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&lo));
-        const float2 q1 = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&hi));
-        dd[j][0] = q0.x; dd[j][1] = q0.y; dd[j][2] = q1.x; dd[j][3] = q1.y;
-      }
-      warp_colsum<8>(dd, red_db1, hc * 64, lane);
-      warp_gemm<NT, 4>(dh2, dfr, w1c, LDW2, lane);
-      release(s);
-    }
-    const float* x2_lo = STG ? st_x2 + (warp * 16 + g) * LDX : p.x_mid + (size_t)r_lo * C;
-    const float* x2_hi = STG ? x2_lo + 8 * LDX : p.x_mid + (size_t)r_hi * C;
-    warp_layernorm_bwd<NT>(dh2, dx, x2_lo, x2_hi, vec + C, m2_lo, s2_lo, m2_hi, s2_hi, rd_lo, rd_hi, t, lane, red_g2, red_be2);
-    warp_colsum<NT>(dh2, red_bp, 0, lane);   // dh2 now holds dx_mid: bias gradient of proj
-#pragma unroll
-    for (int j = 0; j < NT; ++j) {
-      const uint32_t lo = pack2(dh2[j][0], dh2[j][1]), hi = pack2(dh2[j][2], dh2[j][3]);
-      xfr[j >> 1][(j & 1) * 2] = lo;
-      xfr[j >> 1][(j & 1) * 2 + 1] = hi;
-      const int n = j * 8 + 2 * t;
-      if (ok_lo) { *reinterpret_cast<float2*>(p.dx_mid_out + (size_t)r_lo * C + n) = make_float2(dh2[j][0], dh2[j][1]); *reinterpret_cast<uint32_t*>(p.dxm + (size_t)r_lo * C + n) = lo; }
-      if (ok_hi) { *reinterpret_cast<float2*>(p.dx_mid_out + (size_t)r_hi * C + n) = make_float2(dh2[j][2], dh2[j][3]); *reinterpret_cast<uint32_t*>(p.dxm + (size_t)r_hi * C + n) = hi; }
-    }
-    // proj data gradient and delta = rowsum over each head of dy o y
-    acquire(s);
-    const __nv_bfloat16* wpc = ring + (s % NS) * CHUNK;
-    float dyv[NT][4];
-#pragma unroll
-    for (int j = 0; j < NT; ++j) { dyv[j][0] = dyv[j][1] = dyv[j][2] = dyv[j][3] = 0.f; }
-    warp_gemm<NT, KS>(dyv, xfr, wpc, LDW, lane);
-    constexpr int NH = 4;               // heads (the narrow stages of model2_seq use n_head = 4); NT / NH n-tiles per head
-    float dl_lo[NH], dl_hi[NH];
-#pragma unroll
-    for (int h = 0; h < NH; ++h) { dl_lo[h] = 0.f; dl_hi[h] = 0.f; }
-#pragma unroll
-    for (int j = 0; j < NT; ++j) {
-      const int n = j * 8 + 2 * t;
-      const uint32_t lo = pack2(dyv[j][0], dyv[j][1]), hi = pack2(dyv[j][2], dyv[j][3]);
-      uint32_t y0 = 0u, y1 = 0u;
-      if (ok_lo) *reinterpret_cast<uint32_t*>(p.dy + (size_t)r_lo * C + n) = lo;
-      if (ok_hi) *reinterpret_cast<uint32_t*>(p.dy + (size_t)r_hi * C + n) = hi;
-      if (STG) {
-        y0 = *reinterpret_cast<const uint32_t*>(st_y + (warp * 16 + g) * LDW + n);
-        y1 = *reinterpret_cast<const uint32_t*>(st_y + (warp * 16 + g + 8) * LDW + n);
-      } else {
-        if (ok_lo) y0 = *reinterpret_cast<const uint32_t*>(p.y + (size_t)r_lo * C + n);
-        if (ok_hi) y1 = *reinterpret_cast<const uint32_t*>(p.y + (size_t)r_hi * C + n);
-      }
-      const float2 d0 = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&lo)), d1 = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&hi));
-      const float2 v0 = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&y0)), v1 = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&y1));
-      dl_lo[j / (NT / NH)] += d0.x * v0.x + d0.y * v0.y;
-      dl_hi[j / (NT / NH)] += d1.x * v1.x + d1.y * v1.y;
-    }
-#pragma unroll
-    for (int h = 0; h < NH; ++h) {
-      dl_lo[h] += __shfl_xor_sync(0xffffffffu, dl_lo[h], 1); dl_lo[h] += __shfl_xor_sync(0xffffffffu, dl_lo[h], 2);
-      dl_hi[h] += __shfl_xor_sync(0xffffffffu, dl_hi[h], 1); dl_hi[h] += __shfl_xor_sync(0xffffffffu, dl_hi[h], 2);
-    }
-    if (t == 0) {
-#pragma unroll
-      for (int h = 0; h < NH; ++h) {
-        if (ok_lo) p.delta[((size_t)(r_lo / p.T) * NH + h) * p.T + r_lo % p.T] = dl_lo[h];
-        if (ok_hi) p.delta[((size_t)(r_hi / p.T) * NH + h) * p.T + r_hi % p.T] = dl_hi[h];
-      }
-    }
-  }
-  // ---------------------------------------------------------------- column reductions: one atomic per column and CTA
-  __syncthreads();
-  for (int i = tid; i < 9 * C + F; i += CH_THREADS) {
-    const float v = red[i];
-    float* out = nullptr;
-    if (i < 6 * C) {
-      const int q = i / C, c = i % C;
-      float* const outs[6] = {half_a ? p.dg1 : nullptr, half_a ? p.dbe1 : nullptr, half_a ? p.db2_prev : nullptr,
-                              half_b ? p.dg2 : nullptr, half_b ? p.dbe2 : nullptr, half_b ? p.dbp : nullptr};
-      out = outs[q] ? outs[q] + c : nullptr;
-    } else if (i < 9 * C) {
-      out = half_a ? p.dbqkv + (i - 6 * C) : nullptr;
-    } else {
-      out = half_b ? p.db1 + (i - 9 * C) : nullptr;
-    }
-    if (out) atomicAdd(out, v);
-  }
-}
-
-template <int C>
-static int launch_chain_bwd(const ChainBwdArgs& a, cudaStream_t st) {
-  constexpr int F = 4 * C, LDW = C + 8, LDW2 = 72;
-  constexpr int ACT = CH_WARPS * 16 * LDW2;
-  constexpr int WCH = (64 * LDW + C * LDW2 > C * LDW) ? 64 * LDW + C * LDW2 : C * LDW;
-  constexpr int STAGE = ChainCfg<C>::STAGE_BWD ? 3 * CH_WARPS * 16 * (C + 8) * 4 + CH_WARPS * 16 * LDW * 2 : 0;
-  constexpr int SMEM = ChainCfg<C>::NS_BWD * (WCH + ACT) * 2 + (9 * C + F + 2 * C) * 4 + STAGE;
-  static_assert(SMEM <= 232448, "shared memory budget");
-  static bool configured_on[64] = {};
-  bool& configured = per_device_flag(configured_on);
-  if (!configured) {
-    if (cudaFuncSetAttribute(chain_bwd_kernel<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM) != cudaSuccess) return check_launch("chain_bwd/attr");
-    configured = true;
-  }
-  launch_pdl(chain_bwd_kernel<C>, dim3(cdiv(a.M, CH_ROWS)), dim3(CH_THREADS), (size_t)SMEM, st, a);
-  return check_launch("chain_bwd");
-}
-
 }  // namespace dsf
 
 using namespace dsf;
@@ -761,31 +355,4 @@ extern "C" int dsf_chain_fwd(const void* y, const float* x_in, const void* wp, c
                  (const __nv_bfloat16*)wqkv_next, bp, b1, b2, bqkv_next, ln2_g, ln2_b, lnn_g, lnn_b, x_mid, x_out, (__nv_bfloat16*)h2,
                  (__nv_bfloat16*)a, (__nv_bfloat16*)h_next, (__nv_bfloat16*)qkv_next, yf, mean2, rstd2, mean_next, rstd_next, M, eps};
   return C == 64 ? launch_chain_fwd<64>(p, (cudaStream_t)stream) : launch_chain_fwd<128>(p, (cudaStream_t)stream);
-}
-
-extern "C" int dsf_chain_bwd(const void* dqkv, const float* dx_mid_in, const float* x_in, const float* mean1, const float* rstd1, const float* ln1_g,
-                             const void* wqkv_t, float* dln1_g, float* dln1_b, float* dbqkv, float* db2_prev, float* dx_f32,
-                             const float* dx_in, const void* a, const void* y, const float* x_mid, const float* mean2, const float* rstd2,
-                             const float* ln2_g, const void* w2_t, const void* w1_t, const void* wp_t, void* dxa, void* da, void* dxm, void* dy,
-                             float* dx_mid_out, float* delta, float* db1, float* dln2_g, float* dln2_b, float* dbp, int32_t M, int32_t C,
-                             int32_t T, int32_t nh, void* stream) {
-  DSF_REQUIRE(C == 64 || C == 128, "chain_bwd: n_embd must be 64 or 128, got %d", C);
-  DSF_REQUIRE(nh == 4, "chain_bwd: the fused delta reduction is built for n_head = 4 (model2_seq), got %d", nh);
-  DSF_REQUIRE(M > 0 && T > 0 && M % T == 0, "chain_bwd: M=%d must be a positive multiple of T=%d", M, T);
-  const bool ha = dqkv != nullptr, hb = a != nullptr;
-  DSF_REQUIRE(ha || hb, "chain_bwd: nothing to do (neither dqkv nor a given)");
-  DSF_REQUIRE(!ha || (dx_mid_in && x_in && mean1 && rstd1 && ln1_g && wqkv_t && dln1_g && dln1_b && dbqkv), "chain_bwd: half A needs its operands");
-  DSF_REQUIRE(!hb || (y && x_mid && mean2 && rstd2 && ln2_g && w2_t && w1_t && wp_t && da && dxm && dy && dx_mid_out && delta && db1 && dln2_g &&
-                      dln2_b && dbp), "chain_bwd: half B needs its operands");
-  DSF_REQUIRE(ha ? (hb ? dxa != nullptr : dx_f32 != nullptr) : dx_in != nullptr,
-              "chain_bwd: dx must come from half A (dxa / dx_f32 destination) or from dx_in");
-  DSF_REQUIRE(aligned16(dqkv) && aligned16(dx_mid_in) && aligned16(x_in) && aligned16(wqkv_t) && aligned16(dx_f32) && aligned16(dx_in) && aligned16(a) &&
-                  aligned16(y) && aligned16(x_mid) && aligned16(w2_t) && aligned16(w1_t) && aligned16(wp_t) && aligned16(dxa) && aligned16(da) &&
-                  aligned16(dxm) && aligned16(dy) && aligned16(dx_mid_out) && aligned16(ln1_g) && aligned16(ln2_g),
-              "chain_bwd: 16-byte alignment required");
-  ChainBwdArgs p{(const __nv_bfloat16*)dqkv, dx_mid_in, x_in, mean1, rstd1, ln1_g, (const __nv_bfloat16*)wqkv_t, dln1_g, dln1_b, dbqkv, db2_prev, dx_f32,
-                 dx_in, (const __nv_bfloat16*)a, (const __nv_bfloat16*)y, x_mid, mean2, rstd2, ln2_g, (const __nv_bfloat16*)w2_t,
-                 (const __nv_bfloat16*)w1_t, (const __nv_bfloat16*)wp_t, (__nv_bfloat16*)dxa, (__nv_bfloat16*)da, (__nv_bfloat16*)dxm, (__nv_bfloat16*)dy,
-                 dx_mid_out, delta, db1, dln2_g, dln2_b, dbp, M, T, nh};
-  return C == 64 ? launch_chain_bwd<64>(p, (cudaStream_t)stream) : launch_chain_bwd<128>(p, (cudaStream_t)stream);
 }

@@ -68,13 +68,22 @@ def _side_stream(device, which=0):
     return _SIDE_STREAMS[key]
 
 
-def _chain_mode(C, env, default):
-    """Whether the row-local chain kernels (csrc/chain.cu) serve n_embd = C: env value 0 = never, 1 = n_embd 64, 2 = 64 and 128."""
+def _chain_mode(C):
+    """Whether the forward chain kernel (csrc/chain.cu) serves n_embd = C: DSF_CHAIN=0 never, 1 n_embd 64, 2 (default) 64 and 128."""
     try:
-        m = int(os.environ.get(env, default))
+        m = int(os.environ.get("DSF_CHAIN", 2))
     except ValueError:
-        m = default
+        m = 2
     return (m >= 1 and C == 64) or (m >= 2 and C == 128)
+
+
+def _use_side_stream():
+    """Whether the bf16 forward and backward put work on the side streams of ``_side_stream``.
+    Default: on while the step is being captured into a CUDA graph (the fork/join events become graph edges, free at replay:
+    -0.2 ms per step), off for eager launches (creating and recording ~40 events per step costs more host time than the
+    overlap returns).  DSF_WGRAD_STREAM=1 / 0 forces it."""
+    env = os.environ.get("DSF_WGRAD_STREAM")
+    return (env == "1") if env in ("0", "1") else torch.cuda.is_current_stream_capturing()
 
 
 def drop_site(kind, block=0):
@@ -237,10 +246,8 @@ class _Runner:
         saved.layers = []
         # Weight shadows (fp32 -> bf16, plain + transposed, one launch per block) do not depend on the activations: under
         # graph capture they are packed on the side stream while the token kernel and the first blocks run.
-        env = os.environ.get("DSF_WGRAD_STREAM")
-        use_side = (env == "1") if env in ("0", "1") else torch.cuda.is_current_stream_capturing()
         main = torch.cuda.current_stream()
-        side = _side_stream(dev) if use_side else None
+        side = _side_stream(dev) if _use_side_stream() else None
         sizes = [3 * C * C, 3 * C * C, C * C, C * C, F * C, F * C, C * F, C * F]
         packed = []
 
@@ -296,7 +303,7 @@ class _Runner:
         # per block = flash attention + dsf_chain_fwd instead of seven launches.  Measured on B200 (batch 12, graph-replayed stage
         # step, profiles/r02f_*): n_embd 64: 13.6 us per chain launch, step 1.82 -> 1.68 ms; n_embd 128: 34 us, 2.17 -> 2.09 ms.
         # DSF_CHAIN=0: never, 1: n_embd 64 only, 2 (default): n_embd 64 and 128.
-        chain = _chain_mode(C, "DSF_CHAIN", 2) and F == 4 * C and L > 0 and self.dropout is None
+        chain = _chain_mode(C) and F == 4 * C and L > 0 and self.dropout is None
         yf = torch.empty(M, C, device=dev, dtype=f32)
         saved.mean_f = torch.empty(M, device=dev, dtype=f32)
         saved.rstd_f = torch.empty(M, device=dev, dtype=f32)
@@ -404,11 +411,7 @@ class _Runner:
         # N = n_embd GEMMs and of the attention kernels, tails of the short HBM-bound kernels).  fork() orders a wgrad
         # after everything enqueued so far on the main stream; join() makes the main stream wait for the side stream
         # (before buffers the wgrads read are overwritten or released, and before the block's gradients are handed on).
-        # Default: on while the step is being captured into a CUDA graph (the fork/join events become graph edges, free
-        # at replay: -0.2 ms per step), off for eager launches (creating and recording ~40 events per step costs more host
-        # time than the overlap returns).  DSF_WGRAD_STREAM=1 / 0 forces it.
-        env = os.environ.get("DSF_WGRAD_STREAM")
-        use_side = (env == "1") if env in ("0", "1") else torch.cuda.is_current_stream_capturing()
+        use_side = _use_side_stream()
         main = torch.cuda.current_stream()
         side = _side_stream(dev) if use_side else None
         side_q = _side_stream(dev, 1) if use_side else None
@@ -526,151 +529,8 @@ class _Runner:
             self.grad_hook.finish([gbuf[L * per_block + 2 * C:]])
         return dfeats, dgps, grads
 
-    def _backward_bf16_chain(self, saved, params, douts, dgps_out, residual):
-        """Narrow stages (n_embd 64 / 128, no dropout, 4 heads): per block = attention backward (dK/dV + dQ kernels) + ONE row-local
-        chain launch (csrc/chain.cu: QKV data gradient, ln1 backward, mlp backward, ln2 backward, proj data gradient, delta, and
-        every bias / LayerNorm-parameter reduction) + the four weight-gradient GEMMs on the side stream."""
-        dev = douts[0].device
-        M, C, L, T = self.M, self.C, self.L, self.T
-        f32, bf = torch.float32, torch.bfloat16
-        F = 4 * C
-        grads = [None] * len(params)
-        dyf = torch.empty(M, C, device=dev, dtype=f32)
-        K.upsample_add_bwd(self.geom, douts, dgps_out, dyf)
-        sizes = [3 * C * C, C * C, F * C, C * F, 3 * C, C, F, C, C, C, C, C]
-        per_block = sum(sizes)
-        gbuf = torch.zeros(L * per_block + 2 * C + self.T * C, device=dev, dtype=f32)   # blocks | ln_f | pos_emb
-
-        def block_views(i):
-            out, off = [], i * per_block
-            for n in sizes:
-                out.append(gbuf[off:off + n])
-                off += n
-            return out
-
-        def bucket(i):
-            """All-reduce bucket of block i; the last block's bucket carries the ln_f gradients that follow it in the buffer (they
-            are final before any block's backward has started, so they must not wait for the tail of the backward)."""
-            return gbuf[i * per_block:(i + 1) * per_block + (2 * C if i == L - 1 else 0)]
-
-        env = os.environ.get("DSF_WGRAD_STREAM")
-        use_side = (env == "1") if env in ("0", "1") else torch.cuda.is_current_stream_capturing()
-        main = torch.cuda.current_stream()
-        side = _side_stream(dev) if use_side else None
-        side_q = _side_stream(dev, 1) if use_side else None
-
-        def fork(fn, stream=None):
-            stream = stream or side
-            if stream is None:
-                fn()
-                return
-            ev = torch.cuda.Event()
-            ev.record(main)
-            stream.wait_event(ev)
-            with torch.cuda.stream(stream):
-                fn()
-
-        def join(stream):
-            if stream is not None:
-                ev = torch.cuda.Event()
-                ev.record(stream)
-                main.wait_event(ev)
-
-        pending = None
-
-        def join_pending():
-            nonlocal pending
-            if pending is not None:
-                ev, blk, _keep = pending
-                main.wait_event(ev)
-                pending = None
-                if self.grad_hook is not None:
-                    self.grad_hook.block_ready(blk, bucket(blk))
-
-        def half_b(i, dxa):
-            """Operands / destinations of half B for block i (its MLP + proj backward)."""
-            st = saved.layers[i]
-            v = block_views(i)
-            o = _Ctx()
-            o.da = torch.empty(M, F, device=dev, dtype=bf)
-            o.dxm = torch.empty(M, C, device=dev, dtype=bf)
-            o.dy = torch.empty(M, C, device=dev, dtype=bf)
-            o.dx_mid = torch.empty(M, C, device=dev, dtype=f32)
-            o.delta = torch.empty(self.B, self.nh, T, device=dev, dtype=f32)
-            d = dict(a=st.a, y=st.y, x_mid=st.x_mid, mean2=st.mean2, rstd2=st.rstd2, g2=params[3 + 16 * i], w2_t=st.w2_t, w1_t=st.w1_t,
-                     wp_t=st.wp_t, dxa=dxa, da=o.da, dxm=o.dxm, dy=o.dy, dx_mid_out=o.dx_mid, delta=o.delta, db1=v[6], dg2=v[10], dbe2=v[11], dbp=v[5])
-            return o, d
-
-        dgf, dbf = gbuf[L * per_block:L * per_block + C], gbuf[L * per_block + C:L * per_block + 2 * C]
-        dx = torch.empty(M, C, device=dev, dtype=f32)
-        dxa_bufs = [torch.empty(M, C, device=dev, dtype=bf), torch.empty(M, C, device=dev, dtype=bf)]   # block i reads [i & 1]
-        K.layernorm_bwd(dyf, saved.x_last, params[-2], saved.mean_f, saved.rstd_f, None, dx, dgf, dbf, dx_bf16=dxa_bufs[(L - 1) & 1],
-                        dx_colsum=block_views(L - 1)[7])
-        grads[-2], grads[-1] = dgf, dbf
-        cur, d = half_b(L - 1, dxa_bufs[(L - 1) & 1])
-        K.chain_bwd(M, C, T, self.nh, half_b=d, dx_in=dx)
-        dx0 = None
-        for i in reversed(range(L)):
-            base = 1 + 16 * i
-            st = saved.layers[i]
-            dxa = dxa_bufs[i & 1]
-            dwqkv, dwp, dw1, dw2, dbqkv, dbp, db1, db2, dg1, dbt1, dg2, dbt2 = block_views(i)
-            dwqkv, dwp, dw1, dw2 = dwqkv.view(3 * C, C), dwp.view(C, C), dw1.view(F, C), dw2.view(C, F)
-
-            def mlp_proj_wgrads(cur=cur, st=st, dxa=dxa, dw2=dw2, dw1=dw1, dwp=dwp):
-                K.gemm_bf16_tn(dxa, st.a, dw2)
-                K.gemm_bf16_tn(cur.da, st.h2, dw1)
-                K.gemm_bf16_tn(cur.dxm, st.y, dwp)
-            fork(mlp_proj_wgrads)
-            dqkv = torch.empty(M, 3 * C, device=dev, dtype=bf)
-            if side is None:
-                K.attn_bwd(st.qkv, st.y, cur.dy, st.lse, cur.delta, dqkv, self.B, T, C, self.nh, None, None, parts=6)
-            else:   # dQ kernel next to the dK/dV kernel
-                fork(lambda: K.attn_bwd(st.qkv, st.y, cur.dy, st.lse, cur.delta, dqkv, self.B, T, C, self.nh, None, None, parts=4), side_q)
-                K.attn_bwd(st.qkv, st.y, cur.dy, st.lse, cur.delta, dqkv, self.B, T, C, self.nh, None, None, parts=2)
-                join(side_q)
-            fork(lambda: K.gemm_bf16_tn(dqkv, st.h1, dwqkv))
-            join_pending()   # block i+1's side-stream work is complete: its bf16 buffers may be overwritten / released now
-            if side is not None:
-                ev_blk = torch.cuda.Event()
-                ev_blk.record(side)
-                pending = (ev_blk, i, (st, cur, dqkv))
-            ha = dict(dqkv=dqkv, dx_mid_in=cur.dx_mid, x_in=st.x_in, mean1=st.mean1, rstd1=st.rstd1, g1=params[base], wqkv_t=st.wqkv_t,
-                      dg1=dg1, dbe1=dbt1, dbqkv=dbqkv, db2_prev=block_views(i - 1)[7] if i > 0 else None)
-            if i > 0:
-                nxt, d = half_b(i - 1, dxa_bufs[(i - 1) & 1])
-                K.chain_bwd(M, C, T, self.nh, half_a=ha, half_b=d)
-            else:
-                nxt = None
-                dx0 = torch.empty(M, C, device=dev, dtype=f32)
-                K.chain_bwd(M, C, T, self.nh, half_a=ha, dx_f32=dx0)
-            grads[base: base + 16] = [dg1, dbt1, dg2, dbt2,
-                                      dwqkv[C:2 * C], dbqkv[C:2 * C], dwqkv[:C], dbqkv[:C], dwqkv[2 * C:], dbqkv[2 * C:],
-                                      dwp, dbp, dw1, db1, dw2, db2]
-            saved.layers[i] = None
-            if side is None and self.grad_hook is not None:
-                self.grad_hook.block_ready(i, bucket(i))
-            cur = nxt
-        join_pending()
-        dfeats = [torch.empty_like(d_) for d_ in douts]
-        dgps = torch.empty(self.B, 2, C, device=dev, dtype=f32)
-        # pos_emb's gradient lives at the end of the flat buffer, like every other gradient of the stage: autograd adopts such views
-        # without copying them, which a deferred all-reduce relies on (a copy would be taken before the collective has run)
-        dpos = gbuf[L * per_block + 2 * C:].view(1, self.T, C)
-        K.tokens_bwd(self.geom, dx0, douts if residual else None, dfeats, dgps, dpos)
-        grads[0] = dpos
-        if self.grad_hook is not None:
-            self.grad_hook.finish([gbuf[L * per_block + 2 * C:]])
-        return dfeats, dgps, grads
-
     def backward(self, saved, params, douts, dgps_out, residual=True):
         if self.bf16:
-            # backward chain launches (csrc/chain.cu): measured on B200 34 us (n_embd 64) / 79 us (128) per launch against the ~8
-            # separate launches of 7-8 us they replace: stage step 1.683 -> 1.668 ms at 64, 2.09 -> 2.36 ms at 128 (profiles/r02g_*)
-            # -> OFF by default.  DSF_CHAIN_BWD=1: n_embd 64, 2: n_embd 64 and 128.
-            if (_chain_mode(self.C, "DSF_CHAIN_BWD", 0) and self.nh == 4 and self.L > 0 and self.dropout is None
-                    and params[13].shape[0] == 4 * self.C):
-                return self._backward_bf16_chain(saved, params, douts, dgps_out, residual)
             return self._backward_bf16(saved, params, douts, dgps_out, residual)
         dev = douts[0].device
         M, C, L = self.M, self.C, self.L

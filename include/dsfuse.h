@@ -252,22 +252,6 @@ int dsf_chain_fwd(const void* y, const float* x_in, const void* wp, const void* 
                   void* h_next, void* qkv_next, float* yf, float* mean2, float* rstd2, float* mean_next, float* rstd_next,
                   int32_t M, int32_t C, float eps, void* stream);
 
-/* Narrow stages, backward: the row-local chain between the attention backward of block i and that of block i - 1 as ONE launch.
- *   half A (block i; dqkv != NULL):     dh1 = dqkv Wqkv;  dx = dx_mid_in + LayerNorm'(dh1; x_in, ln1)          (autograd of :97-99, 118, 131)
- *                                       dln1_g / dln1_b += ..., dbqkv += colsum(dqkv), db2_prev += colsum(dx)  (bias of block i-1's mlp.2)
- *   half B (block i - 1; a != NULL):    da = (dx W2) o (a > 0);  dh2 = da W1;  dx_mid_out = dx + LayerNorm'(dh2; x_mid, ln2)   (:119-126, 132)
- *                                       dy = dx_mid_out Wp;  delta[b,h,t] = sum_d dy o y  (what dsf_attn_bwd_parts(2 | 4) starts from)
- *                                       db1 += colsum(da), dln2_g / dln2_b += ..., dbp += colsum(dx_mid_out)
- * Without half A, dx is read from dx_in (fp32); without half B, dx is written to dx_f32 (fp32).  dxa / da / dxm are the bf16
- * operands of the weight-gradient GEMMs (dsf_gemm_bf16_tn), dy feeds the attention backward.  wqkv_t (C,3C), w2_t (4C,C),
- * w1_t (C,4C), wp_t (C,C) are the transposed bf16 shadows of dsf_pack_block_weights.  All column sums are ACCUMULATED. */
-int dsf_chain_bwd(const void* dqkv, const float* dx_mid_in, const float* x_in, const float* mean1, const float* rstd1, const float* ln1_g,
-                  const void* wqkv_t, float* dln1_g, float* dln1_b, float* dbqkv, float* db2_prev, float* dx_f32,
-                  const float* dx_in, const void* a, const void* y, const float* x_mid, const float* mean2, const float* rstd2,
-                  const float* ln2_g, const void* w2_t, const void* w1_t, const void* wp_t, void* dxa, void* da, void* dxm, void* dy,
-                  float* dx_mid_out, float* delta, float* db1, float* dln2_g, float* dln2_b, float* dbp, int32_t M, int32_t C,
-                  int32_t T, int32_t nh, void* stream);
-
 /* Optimizer step as one multi-tensor launch: torch.optim.AdamW.step() (train2_seq.py:131, 539: decoupled weight decay,
  * bias-corrected moments, eps added to sqrt(v / bc2)) + EMA.update() (train2_seq.py:133-134, 315-320: shadow = decay * shadow +
  * (1 - decay) * param, taken AFTER the parameter update) + the fp32 -> bf16 repack of GPT weights (what

@@ -23,17 +23,6 @@ SHAPES = [  # (B, C, H, L, A): the four stages of the 256x256 model at B = 2, th
 ]
 
 
-@pytest.mark.parametrize("B,C,H,L,A", [(2, 64, 64, 8, 8), (2, 128, 32, 8, 8), (12, 64, 64, 8, 8)])
-def test_stage_bf16_chain_kernels_every_tensor_within_2e2(cuda_dev, monkeypatch, B, C, H, L, A):
-    """The same bar with the row-local chain kernels of csrc/chain.cu serving the forward and the backward of the narrow stages."""
-    monkeypatch.setenv("DSF_CHAIN", "2")
-    monkeypatch.setenv("DSF_CHAIN_BWD", "2")
-    pb = U.make_problem(B, C, H, L, A, cuda_dev)
-    cap = {}
-    got = U.run_dsfuse(pb, torch.bfloat16, capture=cap)
-    U.check(got, cap, pb, U.run_oracle(pb), "chain kernels")
-
-
 @pytest.mark.parametrize("B,C,H,L,A", SHAPES)
 def test_stage_bf16_every_tensor_within_2e2(cuda_dev, B, C, H, L, A):
     pb = U.make_problem(B, C, H, L, A, cuda_dev)

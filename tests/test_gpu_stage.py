@@ -406,8 +406,8 @@ def test_dropout_is_graph_safe_fresh_masks_per_replay(cuda_dev):
 
 @pytest.mark.parametrize("C,H", [(64, 64), (128, 32)])
 def test_chained_forward_matches_the_separate_kernels(cuda_dev, monkeypatch, C, H):
-    """Narrow stages can run the row-local chain of every block as one launch per direction (DSF_CHAIN / DSF_CHAIN_BWD = 2: n_embd 64
-    and 128).  Same math as the separate LayerNorm / GEMM kernels (= 0) up to the fp32 summation order inside the GEMMs."""
+    """Narrow stages can run the forward's row-local chain of every block as one launch (DSF_CHAIN = 2: n_embd 64 and 128).
+    Same math as the separate LayerNorm / GEMM kernels (= 0) up to the fp32 summation order inside the GEMMs."""
     from deepsense6g_tii_b200 import _capi as K
     from deepsense6g_tii_b200.functional import fusion_stage, param_names
     S, A, nh, L, B = 5, 8, 4, 3, 2
@@ -421,7 +421,6 @@ def test_chained_forward_matches_the_separate_kernels(cuda_dev, monkeypatch, C, 
     res, launches = [], []
     for chain in ("0", "2"):
         monkeypatch.setenv("DSF_CHAIN", chain)
-        monkeypatch.setenv("DSF_CHAIN_BWD", chain)
         pk = [p0[n].clone().requires_grad_(True) for n in names]
         n0 = K.launch_count()
         outs = fusion_stage(cfg, feats[0], feats[1], feats[2], gps, pk)
