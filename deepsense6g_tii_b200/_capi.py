@@ -332,7 +332,9 @@ def adamw_ema_pack(table_dev, tile0_dev, n_tensors, n_tiles, lr, beta1, beta2, e
 def chain_fwd(y, x_in, wp, w1, w2, wqkv_next, bp, b1, b2, bqkv_next, ln2_g, ln2_b, lnn_g, lnn_b, x_mid, x_out, h2, a, h_next, qkv_next, yf,
               mean2, rstd2, mean_next, rstd_next, eps=1e-5):
     """n_embd 64 / 128: proj + residual -> ln2 -> mlp.0 -> ReLU -> mlp.2 + residual -> (next block's ln1 -> fused QKV | ln_f) for
-    all rows in ONE launch (model2_seq.py:109, 121-126, 131-132 and :97-99 / :274 of what follows).  wqkv_next None = last block."""
+    all rows in ONE launch (model2_seq.py:109, 121-126, 131-132 and :97-99 / :274 of what follows).  wqkv_next None = last block.
+    x_mid, h2, a, mean2, rstd2, mean_next, rstd_next (and h_next with a next block) all None: the store-free inference variant,
+    which writes only x_out / qkv_next, or yf (x_out optional) after the last block (include/dsfuse.h)."""
     M, C = y.shape
     _chk(lib().dsf_chain_fwd(_p(y), _p(x_in), _p(wp), _p(w1), _p(w2), _p(wqkv_next), _p(bp), _p(b1), _p(b2), _p(bqkv_next), _p(ln2_g), _p(ln2_b),
                              _p(lnn_g), _p(lnn_b), _p(x_mid), _p(x_out), _p(h2), _p(a), _p(h_next), _p(qkv_next), _p(yf), _p(mean2), _p(rstd2),

@@ -113,7 +113,10 @@ template <int C> struct ChainCfg {
   static constexpr int NS_FWD = C == 64 ? 8 : 4;
 };
 
-template <int C>
+// SAVE = false: the inference variant (no backward follows).  It computes exactly what the SAVE = true kernel computes, by the same
+// expressions, but stores only x_out and the next block's qkv, or only yf (and x_out where given) after the last block: x_mid, h2, a,
+// h_next and the four statistics vectors are read by the backward alone.
+template <int C, bool SAVE>
 __global__ void __launch_bounds__(CH_THREADS, 1) chain_fwd_kernel(ChainFwdArgs p) {
   constexpr int NS = ChainCfg<C>::NS_FWD;
   constexpr int F = 4 * C, NT = C / 8, KS = C / 16;
@@ -211,12 +214,14 @@ __global__ void __launch_bounds__(CH_THREADS, 1) chain_fwd_kernel(ChainFwdArgs p
       xm[j][0] += b.x + x0.x; xm[j][1] += b.y + x0.y; xm[j][2] += b.x + x1.x; xm[j][3] += b.y + x1.y;
       *reinterpret_cast<float2*>(xs_lo) = make_float2(xm[j][0], xm[j][1]);   // x_mid stays on chip for the mlp.2 epilogue
       *reinterpret_cast<float2*>(xs_hi) = make_float2(xm[j][2], xm[j][3]);
-      if (ok_lo) *reinterpret_cast<float2*>(p.x_mid + (size_t)r_lo * C + n) = make_float2(xm[j][0], xm[j][1]);
-      if (ok_hi) *reinterpret_cast<float2*>(p.x_mid + (size_t)r_hi * C + n) = make_float2(xm[j][2], xm[j][3]);
+      if constexpr (SAVE) {
+        if (ok_lo) *reinterpret_cast<float2*>(p.x_mid + (size_t)r_lo * C + n) = make_float2(xm[j][0], xm[j][1]);
+        if (ok_hi) *reinterpret_cast<float2*>(p.x_mid + (size_t)r_hi * C + n) = make_float2(xm[j][2], xm[j][3]);
+      }
     }
     float m_lo, s_lo, m_hi, s_hi;
     warp_layernorm<NT>(xm, v_g2, v_be2, t, p.eps, m_lo, s_lo, m_hi, s_hi);
-    if (t == 0) {
+    if (SAVE && t == 0) {
       if (ok_lo) { p.mean2[r_lo] = m_lo; p.rstd2[r_lo] = s_lo; }
       if (ok_hi) { p.mean2[r_hi] = m_hi; p.rstd2[r_hi] = s_hi; }
     }
@@ -225,9 +230,11 @@ __global__ void __launch_bounds__(CH_THREADS, 1) chain_fwd_kernel(ChainFwdArgs p
       const uint32_t lo = pack2(xm[j][0], xm[j][1]), hi = pack2(xm[j][2], xm[j][3]);
       hfr[j >> 1][(j & 1) * 2] = lo;
       hfr[j >> 1][(j & 1) * 2 + 1] = hi;
-      const int n = j * 8 + 2 * t;
-      if (ok_lo) *reinterpret_cast<uint32_t*>(p.h2 + (size_t)r_lo * C + n) = lo;
-      if (ok_hi) *reinterpret_cast<uint32_t*>(p.h2 + (size_t)r_hi * C + n) = hi;
+      if constexpr (SAVE) {
+        const int n = j * 8 + 2 * t;
+        if (ok_lo) *reinterpret_cast<uint32_t*>(p.h2 + (size_t)r_lo * C + n) = lo;
+        if (ok_hi) *reinterpret_cast<uint32_t*>(p.h2 + (size_t)r_hi * C + n) = hi;
+      }
     }
   }
   release(0);
@@ -254,8 +261,10 @@ __global__ void __launch_bounds__(CH_THREADS, 1) chain_fwd_kernel(ChainFwdArgs p
       const uint32_t hi = pack2(fmaxf(aa[j][2] + b.x, 0.f), fmaxf(aa[j][3] + b.y, 0.f));
       afr[j >> 1][(j & 1) * 2] = lo;
       afr[j >> 1][(j & 1) * 2 + 1] = hi;
-      if (ok_lo) *reinterpret_cast<uint32_t*>(p.a + (size_t)r_lo * F + n) = lo;
-      if (ok_hi) *reinterpret_cast<uint32_t*>(p.a + (size_t)r_hi * F + n) = hi;
+      if constexpr (SAVE) {
+        if (ok_lo) *reinterpret_cast<uint32_t*>(p.a + (size_t)r_lo * F + n) = lo;
+        if (ok_hi) *reinterpret_cast<uint32_t*>(p.a + (size_t)r_hi * F + n) = hi;
+      }
     }
     warp_gemm<NT, 4>(acc2, afr, w2c, LDW2, lane);
     release(s);
@@ -270,11 +279,14 @@ __global__ void __launch_bounds__(CH_THREADS, 1) chain_fwd_kernel(ChainFwdArgs p
     const float* xs_lo = xbuf + (warp * 16 + g) * LDX + n;   // x_mid, written by this thread above
     const float2 x0 = *reinterpret_cast<const float2*>(xs_lo), x1 = *reinterpret_cast<const float2*>(xs_lo + 8 * LDX);
     acc2[j][0] += b.x + x0.x; acc2[j][1] += b.y + x0.y; acc2[j][2] += b.x + x1.x; acc2[j][3] += b.y + x1.y;
-    if (ok_lo) *reinterpret_cast<float2*>(p.x_out + (size_t)r_lo * C + n) = make_float2(acc2[j][0], acc2[j][1]);
-    if (ok_hi) *reinterpret_cast<float2*>(p.x_out + (size_t)r_hi * C + n) = make_float2(acc2[j][2], acc2[j][3]);
+    if (SAVE || p.x_out) {   // store-free last block: x_out is optional (only the ln_f backward reads it)
+      if (ok_lo) *reinterpret_cast<float2*>(p.x_out + (size_t)r_lo * C + n) = make_float2(acc2[j][0], acc2[j][1]);
+      if (ok_hi) *reinterpret_cast<float2*>(p.x_out + (size_t)r_hi * C + n) = make_float2(acc2[j][2], acc2[j][3]);
+    }
   }
   warp_layernorm<NT>(acc2, v_gn, v_ben, t, p.eps, m_lo, s_lo, m_hi, s_hi);
-  if (t == 0) {
+  // (a run-time test: the store-free variant passes NULL here; skipping these stores at compile time makes ptxas spill at n_embd 128)
+  if ((SAVE || p.meann) && t == 0) {
     if (ok_lo) { p.meann[r_lo] = m_lo; p.rstdn[r_lo] = s_lo; }
     if (ok_hi) { p.meann[r_hi] = m_hi; p.rstdn[r_hi] = s_hi; }
   }
@@ -292,9 +304,11 @@ __global__ void __launch_bounds__(CH_THREADS, 1) chain_fwd_kernel(ChainFwdArgs p
     const uint32_t lo = pack2(acc2[j][0], acc2[j][1]), hi = pack2(acc2[j][2], acc2[j][3]);
     hfr[j >> 1][(j & 1) * 2] = lo;
     hfr[j >> 1][(j & 1) * 2 + 1] = hi;
-    const int n = j * 8 + 2 * t;
-    if (ok_lo) *reinterpret_cast<uint32_t*>(p.hn + (size_t)r_lo * C + n) = lo;
-    if (ok_hi) *reinterpret_cast<uint32_t*>(p.hn + (size_t)r_hi * C + n) = hi;
+    if constexpr (SAVE) {
+      const int n = j * 8 + 2 * t;
+      if (ok_lo) *reinterpret_cast<uint32_t*>(p.hn + (size_t)r_lo * C + n) = lo;
+      if (ok_hi) *reinterpret_cast<uint32_t*>(p.hn + (size_t)r_hi * C + n) = hi;
+    }
   }
   // ---------------------------------------------------------------- next block's fused QKV, 64 output columns at a time
   for (int qc = 0; qc < N_QKV; ++qc) {
@@ -316,7 +330,7 @@ __global__ void __launch_bounds__(CH_THREADS, 1) chain_fwd_kernel(ChainFwdArgs p
   }
 }
 
-template <int C>
+template <int C, bool SAVE>
 static int launch_chain_fwd(const ChainFwdArgs& a, cudaStream_t st) {
   constexpr int LDW = C + 8, LDW2 = 72;
   constexpr int CHUNK = (C * LDW > 64 * LDW + C * LDW2) ? C * LDW : 64 * LDW + C * LDW2;
@@ -325,10 +339,10 @@ static int launch_chain_fwd(const ChainFwdArgs& a, cudaStream_t st) {
   static bool configured_on[64] = {};
   bool& configured = per_device_flag(configured_on);
   if (!configured) {
-    if (cudaFuncSetAttribute(chain_fwd_kernel<C>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM) != cudaSuccess) return check_launch("chain_fwd/attr");
+    if (cudaFuncSetAttribute(chain_fwd_kernel<C, SAVE>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM) != cudaSuccess) return check_launch("chain_fwd/attr");
     configured = true;
   }
-  launch_pdl(chain_fwd_kernel<C>, dim3(cdiv(a.M, CH_ROWS)), dim3(CH_THREADS), (size_t)SMEM, st, a);
+  launch_pdl(chain_fwd_kernel<C, SAVE>, dim3(cdiv(a.M, CH_ROWS)), dim3(CH_THREADS), (size_t)SMEM, st, a);
   return check_launch("chain_fwd");
 }
 
@@ -343,10 +357,18 @@ extern "C" int dsf_chain_fwd(const void* y, const float* x_in, const void* wp, c
                              int32_t M, int32_t C, float eps, void* stream) {
   DSF_REQUIRE(C == 64 || C == 128, "chain_fwd: n_embd must be 64 or 128 (wider stages use the tcgen05 GEMM kernels), got %d", C);
   DSF_REQUIRE(M > 0, "chain_fwd: M must be positive");
-  DSF_REQUIRE(y && x_in && wp && w1 && w2 && bp && b1 && b2 && ln2_g && ln2_b && lnn_g && lnn_b && x_mid && x_out && h2 && a && mean2 && rstd2 &&
-                  mean_next && rstd_next, "chain_fwd: NULL pointer");
-  DSF_REQUIRE(wqkv_next ? (bqkv_next && h_next && qkv_next) : (yf != nullptr),
-              "chain_fwd: the next block's QKV needs bqkv / h_next / qkv_next; the last block needs yf");
+  // The tensors only the backward reads come as one group: all given (training forward) or all NULL (store-free variant).
+  // h_next belongs to it only when there is a next block.
+  const int n_saved = (x_mid != nullptr) + (h2 != nullptr) + (a != nullptr) + (mean2 != nullptr) + (rstd2 != nullptr) +
+                      (mean_next != nullptr) + (rstd_next != nullptr) + (wqkv_next && h_next);
+  DSF_REQUIRE(n_saved == 0 || n_saved == (wqkv_next ? 8 : 7),
+              "chain_fwd: x_mid, h2, a, mean2, rstd2, mean_next, rstd_next%s must be all given or all NULL (store-free), got %d of %d",
+              wqkv_next ? ", h_next" : "", n_saved, wqkv_next ? 8 : 7);
+  const bool save = n_saved != 0;
+  DSF_REQUIRE(y && x_in && wp && w1 && w2 && bp && b1 && b2 && ln2_g && ln2_b && lnn_g && lnn_b && (x_out || (!save && !wqkv_next)),
+              "chain_fwd: NULL pointer");
+  DSF_REQUIRE(wqkv_next ? (bqkv_next && qkv_next) : (yf != nullptr),
+              "chain_fwd: the next block's QKV needs bqkv_next / qkv_next; the last block needs yf");
   DSF_REQUIRE(aligned16(y) && aligned16(x_in) && aligned16(wp) && aligned16(w1) && aligned16(w2) && aligned16(wqkv_next) && aligned16(x_mid) &&
                   aligned16(x_out) && aligned16(h2) && aligned16(a) && aligned16(h_next) && aligned16(qkv_next) && aligned16(yf) && aligned16(bp) &&
                   aligned16(b1) && aligned16(b2) && aligned16(bqkv_next) && aligned16(ln2_g) && aligned16(ln2_b) && aligned16(lnn_g) && aligned16(lnn_b),
@@ -354,5 +376,7 @@ extern "C" int dsf_chain_fwd(const void* y, const float* x_in, const void* wp, c
   ChainFwdArgs p{(const __nv_bfloat16*)y, x_in, (const __nv_bfloat16*)wp, (const __nv_bfloat16*)w1, (const __nv_bfloat16*)w2,
                  (const __nv_bfloat16*)wqkv_next, bp, b1, b2, bqkv_next, ln2_g, ln2_b, lnn_g, lnn_b, x_mid, x_out, (__nv_bfloat16*)h2,
                  (__nv_bfloat16*)a, (__nv_bfloat16*)h_next, (__nv_bfloat16*)qkv_next, yf, mean2, rstd2, mean_next, rstd_next, M, eps};
-  return C == 64 ? launch_chain_fwd<64>(p, (cudaStream_t)stream) : launch_chain_fwd<128>(p, (cudaStream_t)stream);
+  const cudaStream_t st = (cudaStream_t)stream;
+  if (save) return C == 64 ? launch_chain_fwd<64, true>(p, st) : launch_chain_fwd<128, true>(p, st);
+  return C == 64 ? launch_chain_fwd<64, false>(p, st) : launch_chain_fwd<128, false>(p, st);
 }

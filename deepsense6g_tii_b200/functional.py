@@ -24,6 +24,7 @@ reproduced bit for bit, so parity with dropout is tested by feeding the oracle t
 (``capture`` receives the attention keep-bitmaps; the elementwise masks are regenerated with
 ``dsf_dropout_inplace`` on a tensor of ones).
 """
+import contextlib
 import math
 import os
 
@@ -53,6 +54,17 @@ def _f32_linear_desc(M, N, Kd, flags, trans=None):
 
 
 class _Ctx:
+    pass
+
+
+def _release(st, *names):
+    """Forward with no backward to follow: the last reader of these tensors of block ``st`` has been enqueued, so drop them.  The
+    caching allocator hands their memory out again in stream order, i.e. only to kernels that run after the pending readers."""
+    for n in names:
+        setattr(st, n, None)
+
+
+def _keep_all(st, *names):
     pass
 
 
@@ -185,14 +197,17 @@ class _Runner:
         return dqkv
 
     # ------------------------------------------------------------------ forward
-    def forward(self, feats, gps_emb, params, residual=True):
+    def forward(self, feats, gps_emb, params, residual=True, keep=True):
         """feats: 3 tensors (N, C, H, W) [or NHWC storage]; gps_emb (B, 2, C) fp32; params: flat list.
-        residual=False returns the upsampled token maps alone (plain ``GPT.forward`` semantics)."""
+        residual=False returns the upsampled token maps alone (plain ``GPT.forward`` semantics).
+        keep=False (no backward follows): the same launches in the same order, but nothing is saved (``saved`` is None) and each
+        block's tensors are released as soon as their last reader has been enqueued."""
         if self.bf16:
-            return self._forward_bf16(feats, gps_emb, params, residual)
+            return self._forward_bf16(feats, gps_emb, params, residual, keep)
         dev = gps_emb.device
         M, C, L = self.M, self.C, self.L
         f32 = torch.float32
+        free = _keep_all if keep else _release
         saved = _Ctx()
         saved.layers = []
         x = torch.empty(M, C, device=dev, dtype=f32)
@@ -205,29 +220,37 @@ class _Runner:
             wqkv = torch.cat([qw, kw, vw], dim=0)
             bqkv = torch.cat([qb, kb, vb], dim=0)
             st.wqkv = wqkv
-            st.x_in = x
+            del wqkv
+            st.x_in, x = x, None
             st.mean1 = torch.empty(M, device=dev, dtype=f32)
             st.rstd1 = torch.empty(M, device=dev, dtype=f32)
             st.h1 = torch.empty(M, C, device=dev, dtype=f32)
-            K.layernorm_fwd(x, ln1w, ln1b, st.h1, st.mean1, st.rstd1)
-            st.qkv = self._linear_fwd(st.h1, wqkv, bqkv, f32)
+            K.layernorm_fwd(st.x_in, ln1w, ln1b, st.h1, st.mean1, st.rstd1)
+            st.qkv = self._linear_fwd(st.h1, st.wqkv, bqkv, f32)
+            free(st, "h1", "mean1", "rstd1", "wqkv")
             st.y = self._attn_fwd(st.qkv, st)
-            x_mid = self._linear_fwd(st.y, pw, pb, f32, residual=x)
-            st.x_mid = x_mid
+            free(st, "qkv", "P")
+            st.x_mid = self._linear_fwd(st.y, pw, pb, f32, residual=st.x_in)
+            free(st, "y", "x_in")
             st.mean2 = torch.empty(M, device=dev, dtype=f32)
             st.rstd2 = torch.empty(M, device=dev, dtype=f32)
             st.h2 = torch.empty(M, C, device=dev, dtype=f32)
-            K.layernorm_fwd(x_mid, ln2w, ln2b, st.h2, st.mean2, st.rstd2)
+            K.layernorm_fwd(st.x_mid, ln2w, ln2b, st.h2, st.mean2, st.rstd2)
             st.a = self._linear_fwd(st.h2, w1, b1, f32, relu=True)
+            free(st, "h2", "mean2", "rstd2")
             if self.capture is not None:
                 self.capture["relu.%d" % i] = st.a
-            x = self._linear_fwd(st.a, w2, b2, f32, residual=x_mid)
-            saved.layers.append(st)
+            x = self._linear_fwd(st.a, w2, b2, f32, residual=st.x_mid)
+            free(st, "a", "x_mid")
+            if keep:
+                saved.layers.append(st)
         saved.x_last = x
         saved.mean_f = torch.empty(M, device=dev, dtype=f32)
         saved.rstd_f = torch.empty(M, device=dev, dtype=f32)
         yf = torch.empty(M, C, device=dev, dtype=f32)
         K.layernorm_fwd(x, params[-2], params[-1], yf, saved.mean_f, saved.rstd_f)
+        if not keep:
+            saved = x = st = None
         outs = [torch.empty_like(f) for f in feats]
         K.upsample_add_fwd(self.geom, yf, feats if residual else [torch.zeros_like(f) for f in feats], outs)
         gps_out = yf.view(self.B, self.T, C)[:, self.Tm:, :].contiguous()
@@ -235,13 +258,15 @@ class _Runner:
 
     # ------------------------------------------------------------------ backward
     # ------------------------------------------------------------------ bf16 tensor-core path
-    def _forward_bf16(self, feats, gps_emb, params, residual):
+    def _forward_bf16(self, feats, gps_emb, params, residual, keep=True):
         """Per block: 1 weight-pack launch, LN, QKV GEMM, flash attention, proj GEMM(+residual), LN,
-        fc1 GEMM(+ReLU), fc2 GEMM(+residual) = 8 launches."""
+        fc1 GEMM(+ReLU), fc2 GEMM(+residual) = 8 launches.  keep=False: see ``forward``; the chain kernel runs its store-free
+        variant, so the tensors only the backward reads (x_mid, h2, a, the next h1, their statistics) are never allocated."""
         dev = gps_emb.device
         M, C, L = self.M, self.C, self.L
         f32, bf = torch.float32, torch.bfloat16
         F = params[13].shape[0] if L > 0 else 4 * C  # mlp.0.weight rows
+        free = _keep_all if keep else _release
         saved = _Ctx()
         saved.layers = []
         # Weight shadows (fp32 -> bf16, plain + transposed, one launch per block) do not depend on the activations: under
@@ -304,25 +329,34 @@ class _Runner:
         # step, profiles/r02f_*): n_embd 64: 13.6 us per chain launch, step 1.82 -> 1.68 ms; n_embd 128: 34 us, 2.17 -> 2.09 ms.
         # DSF_CHAIN=0: never, 1: n_embd 64 only, 2 (default): n_embd 64 and 128.
         chain = _chain_mode(C) and F == 4 * C and L > 0 and self.dropout is None
+        # the separate kernels take x_mid, h2, a and every LayerNorm's statistics as operands; the chain kernel writes them only
+        # for the backward
+        saving = keep or not chain
         yf = torch.empty(M, C, device=dev, dtype=f32)
-        saved.mean_f = torch.empty(M, device=dev, dtype=f32)
-        saved.rstd_f = torch.empty(M, device=dev, dtype=f32)
+        saved.mean_f = torch.empty(M, device=dev, dtype=f32) if saving else None
+        saved.rstd_f = torch.empty(M, device=dev, dtype=f32) if saving else None
         nxt = None  # chain mode: (st, h1, qkv, mean1, rstd1) of block i, produced by block i-1's chain launch
         for i in range(L):
             (ln1w, ln1b, ln2w, ln2b, kw, kb, qw, qb, vw, vb, pw, pb, w1, b1, w2, b2) = params[1 + 16 * i: 17 + 16 * i]
             st = take(i) if nxt is None else nxt
             nxt = None
             bqkv = st.bqkv
-            st.x_in = x
-            if not hasattr(st, "h1"):
+            st.x_in, x = x, None
+            if not hasattr(st, "qkv"):
                 stats = torch.empty(2, M, device=dev, dtype=f32)
                 st.mean1, st.rstd1 = stats[0], stats[1]
+                del stats
                 st.h1 = torch.empty(M, C, device=dev, dtype=bf)
-                K.layernorm_fwd(x, ln1w, ln1b, st.h1, st.mean1, st.rstd1)
+                K.layernorm_fwd(st.x_in, ln1w, ln1b, st.h1, st.mean1, st.rstd1)
                 st.qkv = torch.empty(M, 3 * C, device=dev, dtype=bf)
                 K.gemm_bf16_nt(st.h1, st.wqkv, st.qkv, bias=bqkv)
-            stats2 = torch.empty(2, M, device=dev, dtype=f32)
-            st.mean2, st.rstd2 = stats2[0], stats2[1]
+            free(st, "h1", "mean1", "rstd1")
+            if saving:
+                stats2 = torch.empty(2, M, device=dev, dtype=f32)
+                st.mean2, st.rstd2 = stats2[0], stats2[1]
+                del stats2
+            else:
+                st.mean2 = st.rstd2 = None
             st.y = torch.empty(M, C, device=dev, dtype=bf)
             st.lse = torch.empty(self.B, self.nh, self.T, device=dev, dtype=f32)
             st.drop_bits = None
@@ -331,35 +365,49 @@ class _Runner:
                 if "capture" in self.dropout:
                     self.dropout["capture"]["attn_bits.%d" % i] = st.drop_bits
             K.attn_fwd(st.qkv, st.y, st.lse, self.B, self.T, C, self.nh, self._drop("attn", i), st.drop_bits)
-            st.x_mid = torch.empty(M, C, device=dev, dtype=f32)
-            st.h2 = torch.empty(M, C, device=dev, dtype=bf)
-            st.a = torch.empty(M, F, device=dev, dtype=bf)
-            x_new = torch.empty(M, C, device=dev, dtype=f32)
+            free(st, "qkv", "lse", "drop_bits")   # (a dropout["capture"] dict keeps its own reference to drop_bits)
+            if saving:
+                st.x_mid = torch.empty(M, C, device=dev, dtype=f32)
+                st.h2 = torch.empty(M, C, device=dev, dtype=bf)
+                st.a = torch.empty(M, F, device=dev, dtype=bf)
+            else:
+                st.x_mid = st.h2 = st.a = None
+            # the store-free chain needs no x_out after the last block: only the ln_f backward reads it
+            x_new = torch.empty(M, C, device=dev, dtype=f32) if saving or i + 1 < L else None
             if chain:
                 if i + 1 < L:
                     sn = take(i + 1)
-                    statn = torch.empty(2, M, device=dev, dtype=f32)
-                    sn.mean1, sn.rstd1 = statn[0], statn[1]
-                    sn.h1 = torch.empty(M, C, device=dev, dtype=bf)
+                    if saving:
+                        statn = torch.empty(2, M, device=dev, dtype=f32)
+                        sn.mean1, sn.rstd1 = statn[0], statn[1]
+                        del statn
+                        sn.h1 = torch.empty(M, C, device=dev, dtype=bf)
+                    else:
+                        sn.mean1 = sn.rstd1 = sn.h1 = None
                     sn.qkv = torch.empty(M, 3 * C, device=dev, dtype=bf)
-                    K.chain_fwd(st.y, x, st.wp, st.w1, st.w2, sn.wqkv, pb, b1, b2, sn.bqkv, ln2w, ln2b, params[1 + 16 * (i + 1)],
+                    K.chain_fwd(st.y, st.x_in, st.wp, st.w1, st.w2, sn.wqkv, pb, b1, b2, sn.bqkv, ln2w, ln2b, params[1 + 16 * (i + 1)],
                                 params[2 + 16 * (i + 1)], st.x_mid, x_new, st.h2, st.a, sn.h1, sn.qkv, None, st.mean2, st.rstd2, sn.mean1, sn.rstd1)
                     nxt = sn
+                    del sn
                 else:   # last block: the chain ends with ln_f
-                    K.chain_fwd(st.y, x, st.wp, st.w1, st.w2, None, pb, b1, b2, None, ln2w, ln2b, params[-2], params[-1], st.x_mid, x_new,
+                    K.chain_fwd(st.y, st.x_in, st.wp, st.w1, st.w2, None, pb, b1, b2, None, ln2w, ln2b, params[-2], params[-1], st.x_mid, x_new,
                                 st.h2, st.a, None, None, yf, st.mean2, st.rstd2, saved.mean_f, saved.rstd_f)
             else:
-                K.gemm_bf16_nt(st.y, st.wp, st.x_mid, bias=pb, residual=x, drop=self._drop("proj", i))
+                K.gemm_bf16_nt(st.y, st.wp, st.x_mid, bias=pb, residual=st.x_in, drop=self._drop("proj", i))
                 K.layernorm_fwd(st.x_mid, ln2w, ln2b, st.h2, st.mean2, st.rstd2)
                 K.gemm_bf16_nt(st.h2, st.w1, st.a, bias=b1, relu=True)
                 K.gemm_bf16_nt(st.a, st.w2, x_new, bias=b2, residual=st.x_mid, drop=self._drop("mlp", i))
             if self.capture is not None:
                 self.capture["relu.%d" % i] = st.a
-            x = x_new
-            saved.layers.append(st)
+            free(st, "x_in", "y", "x_mid", "h2", "mean2", "rstd2", "a")
+            x, x_new = x_new, None
+            if keep:
+                saved.layers.append(st)
         saved.x_last = x
         if not chain:
             K.layernorm_fwd(x, params[-2], params[-1], yf, saved.mean_f, saved.rstd_f)
+        if not keep:
+            saved = x = st = nxt = None
         outs = [torch.empty_like(f) for f in feats]
         K.upsample_add_fwd(self.geom, yf, feats if residual else [torch.zeros_like(f) for f in feats], outs)
         gps_out = yf.view(self.B, self.T, C)[:, self.Tm:, :].contiguous()
@@ -623,25 +671,20 @@ def _layout_of(t):
     raise RuntimeError("feature maps must be contiguous or channels_last")
 
 
-class FusionStageFn(torch.autograd.Function):
-    """(image, lidar, radar feature maps, gps_emb, *GPT params) -> (image', lidar', radar', gps_out)."""
-
-    @staticmethod
-    def forward(ctx, cfg, img, lidar, radar, gps_emb, *params):
-        for t, n in ((img, "image features"), (lidar, "lidar features"), (radar, "radar features")):
-            if not t.is_cuda:
-                raise RuntimeError("%s must be CUDA tensors (the fusion stage has no CPU path)" % n)
-        # Every launch goes to the CURRENT device's stream with raw pointers: all operands must live on one device, and that
-        # device is made current for the whole call (tensors on cuda:1 while cuda:0 is current — nn.DataParallel replicas,
-        # TransFuser(cfg, 'cuda:1') without set_device — would otherwise fault instead of raising).
-        for t in (lidar, radar, gps_emb) + tuple(params):
-            if t.device != img.device:
-                raise RuntimeError("fusion stage: all inputs and parameters must be on %s, found a tensor on %s" % (img.device, t.device))
-        with torch.cuda.device(img.device):
-            return FusionStageFn._forward(ctx, cfg, img, lidar, radar, gps_emb, *params)
-
-    @staticmethod
-    def _forward(ctx, cfg, img, lidar, radar, gps_emb, *params):
+@contextlib.contextmanager
+def _stage_call(cfg, img, lidar, radar, gps_emb, params):
+    """Input checks and set-up of one ``fusion_stage`` call, shared by the training and the inference forward.  Yields
+    (runner, [img, lidar, radar], gps_emb, flat fp32 params, residual, memory format of the maps) with the inputs' device current."""
+    for t, n in ((img, "image features"), (lidar, "lidar features"), (radar, "radar features")):
+        if not t.is_cuda:
+            raise RuntimeError("%s must be CUDA tensors (the fusion stage has no CPU path)" % n)
+    # Every launch goes to the CURRENT device's stream with raw pointers: all operands must live on one device, and that
+    # device is made current for the whole call (tensors on cuda:1 while cuda:0 is current — nn.DataParallel replicas,
+    # TransFuser(cfg, 'cuda:1') without set_device — would otherwise fault instead of raising).
+    for t in (lidar, radar, gps_emb) + tuple(params):
+        if t.device != img.device:
+            raise RuntimeError("fusion stage: all inputs and parameters must be on %s, found a tensor on %s" % (img.device, t.device))
+    with torch.cuda.device(img.device):
         K.check_device()
         layout = _layout_of(img)
         if _layout_of(lidar) != layout or _layout_of(radar) != layout:
@@ -672,13 +715,23 @@ class FusionStageFn(torch.autograd.Function):
                                           "p = 0 parity path)")
         else:
             r.dropout = None
-        outs, gps_out, saved = r.forward([img.detach(), lidar.detach(), radar.detach()], gps_emb.detach(), plist, residual)
+        yield (r, [img.detach(), lidar.detach(), radar.detach()], gps_emb.detach(), plist, residual,
+               torch.channels_last if layout == K.DSF_NHWC else torch.contiguous_format)
+
+
+class FusionStageFn(torch.autograd.Function):
+    """(image, lidar, radar feature maps, gps_emb, *GPT params) -> (image', lidar', radar', gps_out)."""
+
+    @staticmethod
+    def forward(ctx, cfg, img, lidar, radar, gps_emb, *params):
+        with _stage_call(cfg, img, lidar, radar, gps_emb, params) as (r, feats, gps, plist, residual, mf):
+            outs, gps_out, saved = r.forward(feats, gps, plist, residual)
         ctx.runner, ctx.saved_state, ctx.plist, ctx.residual = r, saved, plist, residual
         ctx.device = img.device
         ctx.param_versions = [p._version for p in params]
         ctx.params_ref = params
-        ctx.feat_mf = torch.channels_last if layout == K.DSF_NHWC else torch.contiguous_format
-        ctx.gps_dtype = gps_emb.dtype
+        ctx.feat_mf = mf
+        ctx.gps_dtype = gps.dtype
         return outs[0], outs[1], outs[2], gps_out
 
     @staticmethod
@@ -712,8 +765,18 @@ class FusionStageFn(torch.autograd.Function):
 def fusion_stage(cfg, img, lidar, radar, gps_emb, params):
     """cfg: dict(seq_len, n_views, vert_anchors, horz_anchors, n_head, n_layer, compute_dtype[, residual][, dropout][, grad_hook]
     [, capture]).  ``capture`` (a dict, diagnostics / tests) receives ``relu.{i}``: the (B*T, 4C) mlp.0 output of block i, whose
-    sign pattern is the set of ReLU decisions this evaluation took (see tests/tools/bf16_error_model.py)."""
-    return FusionStageFn.apply(cfg, img, lidar, radar, gps_emb, *params)
+    sign pattern is the set of ReLU decisions this evaluation took (see tests/tools/bf16_error_model.py).
+
+    When autograd would record no node for the call — grad mode off (``torch.no_grad``, ``torch.inference_mode``), or neither a
+    map, ``gps_emb`` nor a parameter requiring grad — the stage runs the same kernels in the same order without keeping anything
+    for a backward: each block's tensors are released once their last reader is enqueued, and the narrow stages' chain kernel
+    writes only what the next block reads.  The four outputs are bit-identical to the training forward's and do not require grad."""
+    needs_graph = torch.is_grad_enabled() and any(t.requires_grad for t in (img, lidar, radar, gps_emb, *params))
+    if needs_graph or cfg.get("capture") is not None:
+        return FusionStageFn.apply(cfg, img, lidar, radar, gps_emb, *params)
+    with _stage_call(cfg, img, lidar, radar, gps_emb, params) as (r, feats, gps, plist, residual, _mf):
+        outs, gps_out, _ = r.forward(feats, gps, plist, residual, keep=False)
+    return outs[0], outs[1], outs[2], gps_out
 
 
 # ------------------------------------------------------------------------------------------------ stem / tail of Encoder.forward

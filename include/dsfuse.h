@@ -245,7 +245,11 @@ int dsf_tail_bwd(const float* dfused, void* dimg, void* dlidar, void* dradar, fl
  *   or     (last block)              yf = LayerNorm(x_out; ln_f) in fp32                                                (:274)
  * y (M,C) bf16; x_in, x_mid, x_out, yf (M,C) fp32; wp (C,C), w1 (4C,C), w2 (C,4C), wqkv_next (3C,C) bf16 weight shadows as packed
  * by dsf_pack_block_weights; h2, h_next (M,C), a (M,4C), qkv_next (M,3C) bf16 and the four statistics vectors (M) are the
- * tensors the backward reads.  No dropout on this path (the caller keeps the separate kernels when p > 0). */
+ * tensors the backward reads.  No dropout on this path (the caller keeps the separate kernels when p > 0).
+ * Store-free variant (inference, no backward follows): x_mid, h2, a, mean2, rstd2, mean_next, rstd_next and, when wqkv_next is
+ * given, h_next are one group: all non-NULL runs the kernel above, all NULL a kernel that computes the same values by the same
+ * expressions (x_out, qkv_next and yf come out bit-identical) but writes only x_out and qkv_next, or only yf after the last block,
+ * where x_out may then be NULL too.  Any other mix is an error. */
 int dsf_chain_fwd(const void* y, const float* x_in, const void* wp, const void* w1, const void* w2, const void* wqkv_next,
                   const float* bp, const float* b1, const float* b2, const float* bqkv_next, const float* ln2_g,
                   const float* ln2_b, const float* lnn_g, const float* lnn_b, float* x_mid, float* x_out, void* h2, void* a,
