@@ -24,7 +24,7 @@ SYMBOLS = [
     "dsf_layernorm_fwd", "dsf_layernorm_bwd", "dsf_gemm_bf16_nt", "dsf_gemm_bf16_tn", "dsf_gemm_set_impl", "dsf_gemm_f32",
     "dsf_colsum", "dsf_relu_bwd", "dsf_relu_bwd_colsum", "dsf_pack_block_weights", "dsf_softmax_fwd", "dsf_softmax_bwd", "dsf_attn_fwd", "dsf_attn_bwd", "dsf_attn_bwd_parts", "dsf_attn_set_impl", "dsf_attn_drop_words",
     "dsf_upsample_add_fwd", "dsf_upsample_add_bwd", "dsf_cast_f32_bf16", "dsf_opt_tiles", "dsf_adamw_ema_pack", "dsf_opt_upload_table", "dsf_chain_fwd",
-    "dsf_stem_pack", "dsf_tail_fwd", "dsf_tail_bwd",
+    "dsf_stem_pack", "dsf_tail_fwd", "dsf_tail_bwd", "dsf_stage_workspace_size", "dsf_stage_fwd",
 ]
 
 
@@ -55,6 +55,31 @@ class OptTensor(ctypes.Structure):
     """``dsf_opt_tensor`` (include/dsfuse.h): one parameter tensor of the fused AdamW + EMA + bf16-repack step."""
     _fields_ = ([(n, c_void_p) for n in ("p", "g", "m", "v", "ema", "shadow", "shadow_t", "copy_f32")] +
                 [(n, c_int32) for n in ("rows", "cols", "row_off", "ld_t")] + [("weight_decay", c_float), ("reserved", c_int32)])
+
+
+SHADOW_KEYS = ("wqkv", "wqkv_t", "wp", "wp_t", "w1", "w1_t", "w2", "w2_t", "bqkv")
+
+
+class DropoutCfg(ctypes.Structure):
+    """``dsf_dropout_cfg`` (include/dsfuse.h): the dropout probabilities of one GPT in train() mode."""
+    _fields_ = [("embd", c_float), ("attn", c_float), ("resid", c_float), ("seed", ctypes.c_uint64), ("step", ctypes.c_uint32),
+                ("seed_dev", c_void_p)]
+
+
+class StageDesc(ctypes.Structure):
+    """``dsf_stage_desc`` (include/dsfuse.h): one fusion stage for ``dsf_stage_fwd``."""
+    _fields_ = ([("geom", Geom)] + [(n, c_int32) for n in ("n_head", "n_layer", "F", "residual", "chain", "prepacked")] +
+                [("dropout", POINTER(DropoutCfg))])
+
+
+class BlockShadows(ctypes.Structure):
+    """``dsf_block_shadows`` (include/dsfuse.h): the bf16 weight shadows of one block."""
+    _fields_ = [(n, c_void_p) for n in SHADOW_KEYS]
+
+
+class StageParams(ctypes.Structure):
+    """``dsf_stage_params`` (include/dsfuse.h)."""
+    _fields_ = [("params", POINTER(c_void_p)), ("shadows", POINTER(BlockShadows)), ("ready", POINTER(c_void_p)), ("repack", c_int32)]
 
 
 _lib = None
@@ -110,6 +135,10 @@ def lib():
             fn = getattr(L, name)
             fn.argtypes = argtypes
             fn.restype = c_int32
+        L.dsf_stage_workspace_size.argtypes = [POINTER(StageDesc), POINTER(ctypes.c_size_t)]
+        L.dsf_stage_workspace_size.restype = c_int32
+        L.dsf_stage_fwd.argtypes = [POINTER(StageDesc), POINTER(StageParams)] + [P] * 9 + [ctypes.c_size_t, P]
+        L.dsf_stage_fwd.restype = c_int32
         L.dsf_attn_drop_words.argtypes = [c_int32, c_int32, c_int32]
         L.dsf_attn_drop_words.restype = c_int64
         _lib = L
@@ -347,3 +376,37 @@ def opt_upload_table(dst_dev, src_pinned):
         raise RuntimeError("opt_upload_table: the host table must be pinned memory")
     _chk(lib().dsf_opt_upload_table(_p(dst_dev), c_void_p(src_pinned.data_ptr()), src_pinned.numel() * src_pinned.element_size(), _stream()),
          "dsf_opt_upload_table")
+
+
+def make_stage_desc(geom, n_head, n_layer, F, residual=True, chain=-1, prepacked=False, dropout=None):
+    """``dsf_stage_desc``; ``dropout`` a ``DropoutCfg`` or None (the descriptor keeps it alive)."""
+    d = StageDesc(geom, n_head, n_layer, F, 1 if residual else 0, chain, 1 if prepacked else 0)
+    if dropout is not None:
+        d.dropout = ctypes.pointer(dropout)
+    return d
+
+
+def stage_workspace_size(desc):
+    """Bytes of device workspace ``stage_fwd`` needs for ``desc`` (the formula is in include/dsfuse.h)."""
+    n = ctypes.c_size_t(0)
+    _chk(lib().dsf_stage_workspace_size(ctypes.byref(desc), ctypes.byref(n)), "dsf_stage_workspace_size")
+    return n.value
+
+
+def stage_fwd(desc, params, feats, gps_emb, outs, gps_out, workspace, workspace_bytes=None, shadows=None, repack=False, ready=None):
+    """One whole inference forward of a fusion stage (``dsf_stage_fwd``).  params: the flat fp32 parameter tensors in
+    ``functional.param_names`` order; shadows: None or one dict of bf16 shadow views (``SHADOW_KEYS``) per block; ready: None or one
+    ``torch.cuda.Event`` per block that block's shadows are waited for; workspace: a uint8 CUDA tensor, or a raw device address with
+    ``workspace_bytes``."""
+    ptrs = (c_void_p * len(params))(*[p.data_ptr() for p in params])
+    sh = None
+    if shadows is not None:
+        sh = (BlockShadows * len(shadows))(*[BlockShadows(*[v[k].data_ptr() for k in SHADOW_KEYS]) for v in shadows])
+    ev = None if ready is None else (c_void_p * len(ready))(*[e.cuda_event for e in ready])
+    prm = StageParams(ptrs, sh, ev, 1 if repack else 0)
+    if isinstance(workspace, torch.Tensor):
+        ws, nbytes = workspace.data_ptr(), workspace.numel() if workspace_bytes is None else workspace_bytes
+    else:
+        ws, nbytes = workspace, workspace_bytes
+    _chk(lib().dsf_stage_fwd(ctypes.byref(desc), ctypes.byref(prm), _p(feats[0]), _p(feats[1]), _p(feats[2]), _p(gps_emb), _p(outs[0]),
+                             _p(outs[1]), _p(outs[2]), _p(gps_out), c_void_p(ws), nbytes, _stream()), "dsf_stage_fwd")

@@ -80,13 +80,33 @@ def _side_stream(device, which=0):
     return _SIDE_STREAMS[key]
 
 
-def _chain_mode(C):
-    """Whether the forward chain kernel (csrc/chain.cu) serves n_embd = C: DSF_CHAIN=0 never, 1 n_embd 64, 2 (default) 64 and 128."""
+def _chain_mode():
+    """The ``chain`` field of ``dsf_stage_desc`` that DSF_CHAIN selects: unset -> -1 (the library's default rule, the same as 2),
+    0 never, 1 the forward chain kernel (csrc/chain.cu) at n_embd 64, 2 at n_embd 64 and 128."""
+    env = os.environ.get("DSF_CHAIN")
     try:
-        m = int(os.environ.get("DSF_CHAIN", 2))
+        return -1 if env is None else min(max(int(env), 0), 2)
     except ValueError:
-        m = 2
-    return (m >= 1 and C == 64) or (m >= 2 and C == 128)
+        return -1
+
+
+def _new_shadows(C, F, device):
+    """Buffers for one block's bf16 weight shadows (plain + transposed, one flat allocation) and its fused fp32 QKV bias, as a dict
+    of the views ``dsf_pack_block_weights`` writes (keys ``_capi.SHADOW_KEYS``)."""
+    shapes = [(3 * C, C), (C, 3 * C), (C, C), (C, C), (F, C), (C, F), (C, F), (F, C)]
+    flat = torch.empty(sum(a * b for a, b in shapes), device=device, dtype=torch.bfloat16)
+    views, off = {}, 0
+    for k, (a, b) in zip(K.SHADOW_KEYS, shapes):
+        views[k] = flat[off:off + a * b].view(a, b)
+        off += a * b
+    views["bqkv"] = torch.empty(3 * C, device=device, dtype=torch.float32)
+    return views
+
+
+def _pack(params, i, v):
+    """dsf_pack_block_weights of block i's fp32 parameters into the shadow views ``v``."""
+    (ln1w, ln1b, ln2w, ln2b, kw, kb, qw, qb, vw, vb, pw, pb, w1, b1, w2, b2) = params[1 + 16 * i: 17 + 16 * i]
+    K.pack_block_weights(qw, kw, vw, pw, w1, w2, qb, kb, vb, tuple(v[k] for k in K.SHADOW_KEYS))
 
 
 def _use_side_stream():
@@ -200,10 +220,11 @@ class _Runner:
     def forward(self, feats, gps_emb, params, residual=True, keep=True):
         """feats: 3 tensors (N, C, H, W) [or NHWC storage]; gps_emb (B, 2, C) fp32; params: flat list.
         residual=False returns the upsampled token maps alone (plain ``GPT.forward`` semantics).
-        keep=False (no backward follows): the same launches in the same order, but nothing is saved (``saved`` is None) and each
-        block's tensors are released as soon as their last reader has been enqueued."""
+        keep=False (no backward follows): the same launches in the same order, but nothing is saved (``saved`` is None); in bf16 mode
+        that is one ``dsf_stage_fwd`` call, in fp32 mode each block's tensors are released as soon as their last reader has been
+        enqueued."""
         if self.bf16:
-            return self._forward_bf16(feats, gps_emb, params, residual, keep)
+            return self._forward_bf16(feats, gps_emb, params, residual) if keep else self._infer_bf16(feats, gps_emb, params, residual)
         dev = gps_emb.device
         M, C, L = self.M, self.C, self.L
         f32 = torch.float32
@@ -258,48 +279,65 @@ class _Runner:
 
     # ------------------------------------------------------------------ backward
     # ------------------------------------------------------------------ bf16 tensor-core path
-    def _forward_bf16(self, feats, gps_emb, params, residual, keep=True):
-        """Per block: 1 weight-pack launch, LN, QKV GEMM, flash attention, proj GEMM(+residual), LN,
-        fc1 GEMM(+ReLU), fc2 GEMM(+residual) = 8 launches.  keep=False: see ``forward``; the chain kernel runs its store-free
-        variant, so the tensors only the backward reads (x_mid, h2, a, the next h1, their statistics) are never allocated."""
+    def _infer_bf16(self, feats, gps_emb, params, residual):
+        """No backward follows: the whole stage is one ``dsf_stage_fwd`` call (csrc/stage.cu), which enqueues the launches of
+        ``_forward_bf16`` in the same order, with the chain kernel's store-free variant, on one workspace allocation."""
+        C, L = self.C, self.L
+        F = params[13].shape[0] if L > 0 else 4 * C  # mlp.0.weight rows
+        drop = None
+        if self.dropout is not None:
+            d, sd = self.dropout, self.dropout.get("seed_dev")
+            drop = K.DropoutCfg(float(d.get("embd", 0.0)), float(d.get("attn", 0.0)), float(d.get("resid", 0.0)), int(d["seed"]),
+                                int(d.get("step", 0)), None if sd is None else sd.data_ptr())
+        dev, sh = gps_emb.device, self.shadows
+        stale = sh is not None and not sh["fresh"]
+        shadows, ready, repack = (None if sh is None else sh["views"]), None, stale
+        if _use_side_stream() and L > 0:
+            # As in _forward_bf16: the weight packs run on the side stream and block i waits for its own pack only, so they overlap
+            # the token kernel and the blocks before i.  The buffers are allocated on the current stream, which reads them.
+            shadows = sh["views"] if sh is not None else [_new_shadows(C, F, dev) for _ in range(L)]
+            side, ready, repack = _side_stream(dev), [], False
+            ev = torch.cuda.Event()
+            ev.record(torch.cuda.current_stream())
+            side.wait_event(ev)
+            with torch.cuda.stream(side):
+                for i in range(L):
+                    if sh is None or stale:
+                        _pack(params, i, shadows[i])
+                    ready.append(torch.cuda.Event())
+                    ready[-1].record(side)
+        desc = K.make_stage_desc(self.geom, self.nh, L, F, residual, _chain_mode(), shadows is not None, drop)
+        ws = torch.empty(K.stage_workspace_size(desc), device=dev, dtype=torch.uint8)
+        outs = [torch.empty_like(f) for f in feats]
+        gps_out = torch.empty(self.B, 2, C, device=dev, dtype=torch.float32)
+        K.stage_fwd(desc, params, feats, gps_emb, outs, gps_out, ws, shadows=shadows, repack=repack, ready=ready)
+        if stale:
+            sh["owner"].mark_shadows_fresh()
+        return outs, gps_out, None
+
+    def _forward_bf16(self, feats, gps_emb, params, residual):
+        """Training forward.  Per block: 1 weight-pack launch, LN, QKV GEMM, flash attention, proj GEMM(+residual), LN,
+        fc1 GEMM(+ReLU), fc2 GEMM(+residual) = 8 launches."""
         dev = gps_emb.device
         M, C, L = self.M, self.C, self.L
         f32, bf = torch.float32, torch.bfloat16
         F = params[13].shape[0] if L > 0 else 4 * C  # mlp.0.weight rows
-        free = _keep_all if keep else _release
         saved = _Ctx()
         saved.layers = []
         # Weight shadows (fp32 -> bf16, plain + transposed, one launch per block) do not depend on the activations: under
         # graph capture they are packed on the side stream while the token kernel and the first blocks run.
         main = torch.cuda.current_stream()
         side = _side_stream(dev) if _use_side_stream() else None
-        sizes = [3 * C * C, 3 * C * C, C * C, C * C, F * C, F * C, C * F, C * F]
         packed = []
 
         def pack(i):
-            (ln1w, ln1b, ln2w, ln2b, kw, kb, qw, qb, vw, vb, pw, pb, w1, b1, w2, b2) = params[1 + 16 * i: 17 + 16 * i]
             st = _Ctx()
-            if self.shadows is not None:   # persistent shadows: up to date (written by the fused optimizer step), or re-packed in place
-                v = self.shadows["views"][i]
-                st.wqkv, st.wqkv_t, st.wp, st.wp_t, st.w1, st.w1_t, st.w2, st.w2_t, st.bqkv = (
-                    v["wqkv"], v["wqkv_t"], v["wp"], v["wp_t"], v["w1"], v["w1_t"], v["w2"], v["w2_t"], v["bqkv"])
-                if not self.shadows["fresh"]:
-                    K.pack_block_weights(qw, kw, vw, pw, w1, w2, qb, kb, vb,
-                                         (st.wqkv, st.wqkv_t, st.wp, st.wp_t, st.w1, st.w1_t, st.w2, st.w2_t, st.bqkv))
-                return st
-            # one flat bf16 buffer holds the 8 weight shadows of this block (plain + transposed)
-            flat = torch.empty(sum(sizes), device=dev, dtype=bf)
-            views, off = [], 0
-            for n in sizes:
-                views.append(flat[off:off + n])
-                off += n
-            st.wqkv, st.wqkv_t = views[0].view(3 * C, C), views[1].view(C, 3 * C)
-            st.wp, st.wp_t = views[2].view(C, C), views[3].view(C, C)
-            st.w1, st.w1_t = views[4].view(F, C), views[5].view(C, F)
-            st.w2, st.w2_t = views[6].view(C, F), views[7].view(F, C)
-            st.bqkv = torch.empty(3 * C, device=dev, dtype=f32)
-            K.pack_block_weights(qw, kw, vw, pw, w1, w2, qb, kb, vb,
-                                 (st.wqkv, st.wqkv_t, st.wp, st.wp_t, st.w1, st.w1_t, st.w2, st.w2_t, st.bqkv))
+            # persistent shadows: up to date (written by the fused optimizer step), or re-packed in place
+            v = self.shadows["views"][i] if self.shadows is not None else _new_shadows(C, F, dev)
+            if self.shadows is None or not self.shadows["fresh"]:
+                _pack(params, i, v)
+            for k in K.SHADOW_KEYS:
+                setattr(st, k, v[k])
             return st
 
         if side is not None:
@@ -327,14 +365,13 @@ class _Runner:
         # Narrow stages (no dropout): everything between two attention calls is row-local and runs as ONE launch (csrc/chain.cu):
         # per block = flash attention + dsf_chain_fwd instead of seven launches.  Measured on B200 (batch 12, graph-replayed stage
         # step, profiles/r02f_*): n_embd 64: 13.6 us per chain launch, step 1.82 -> 1.68 ms; n_embd 128: 34 us, 2.17 -> 2.09 ms.
-        # DSF_CHAIN=0: never, 1: n_embd 64 only, 2 (default): n_embd 64 and 128.
-        chain = _chain_mode(C) and F == 4 * C and L > 0 and self.dropout is None
-        # the separate kernels take x_mid, h2, a and every LayerNorm's statistics as operands; the chain kernel writes them only
-        # for the backward
-        saving = keep or not chain
+        # DSF_CHAIN=0: never, 1: n_embd 64 only, 2 (default): n_embd 64 and 128.  The same rule as dsf_stage_fwd's (csrc/stage.cu), so
+        # the inference forward launches the same kernels.
+        m = _chain_mode()
+        chain = ((m != 0 and C == 64) or (m in (-1, 2) and C == 128)) and F == 4 * C and L > 0 and self.dropout is None
         yf = torch.empty(M, C, device=dev, dtype=f32)
-        saved.mean_f = torch.empty(M, device=dev, dtype=f32) if saving else None
-        saved.rstd_f = torch.empty(M, device=dev, dtype=f32) if saving else None
+        saved.mean_f = torch.empty(M, device=dev, dtype=f32)
+        saved.rstd_f = torch.empty(M, device=dev, dtype=f32)
         nxt = None  # chain mode: (st, h1, qkv, mean1, rstd1) of block i, produced by block i-1's chain launch
         for i in range(L):
             (ln1w, ln1b, ln2w, ln2b, kw, kb, qw, qb, vw, vb, pw, pb, w1, b1, w2, b2) = params[1 + 16 * i: 17 + 16 * i]
@@ -350,13 +387,9 @@ class _Runner:
                 K.layernorm_fwd(st.x_in, ln1w, ln1b, st.h1, st.mean1, st.rstd1)
                 st.qkv = torch.empty(M, 3 * C, device=dev, dtype=bf)
                 K.gemm_bf16_nt(st.h1, st.wqkv, st.qkv, bias=bqkv)
-            free(st, "h1", "mean1", "rstd1")
-            if saving:
-                stats2 = torch.empty(2, M, device=dev, dtype=f32)
-                st.mean2, st.rstd2 = stats2[0], stats2[1]
-                del stats2
-            else:
-                st.mean2 = st.rstd2 = None
+            stats2 = torch.empty(2, M, device=dev, dtype=f32)
+            st.mean2, st.rstd2 = stats2[0], stats2[1]
+            del stats2
             st.y = torch.empty(M, C, device=dev, dtype=bf)
             st.lse = torch.empty(self.B, self.nh, self.T, device=dev, dtype=f32)
             st.drop_bits = None
@@ -365,25 +398,17 @@ class _Runner:
                 if "capture" in self.dropout:
                     self.dropout["capture"]["attn_bits.%d" % i] = st.drop_bits
             K.attn_fwd(st.qkv, st.y, st.lse, self.B, self.T, C, self.nh, self._drop("attn", i), st.drop_bits)
-            free(st, "qkv", "lse", "drop_bits")   # (a dropout["capture"] dict keeps its own reference to drop_bits)
-            if saving:
-                st.x_mid = torch.empty(M, C, device=dev, dtype=f32)
-                st.h2 = torch.empty(M, C, device=dev, dtype=bf)
-                st.a = torch.empty(M, F, device=dev, dtype=bf)
-            else:
-                st.x_mid = st.h2 = st.a = None
-            # the store-free chain needs no x_out after the last block: only the ln_f backward reads it
-            x_new = torch.empty(M, C, device=dev, dtype=f32) if saving or i + 1 < L else None
+            st.x_mid = torch.empty(M, C, device=dev, dtype=f32)
+            st.h2 = torch.empty(M, C, device=dev, dtype=bf)
+            st.a = torch.empty(M, F, device=dev, dtype=bf)
+            x_new = torch.empty(M, C, device=dev, dtype=f32)
             if chain:
                 if i + 1 < L:
                     sn = take(i + 1)
-                    if saving:
-                        statn = torch.empty(2, M, device=dev, dtype=f32)
-                        sn.mean1, sn.rstd1 = statn[0], statn[1]
-                        del statn
-                        sn.h1 = torch.empty(M, C, device=dev, dtype=bf)
-                    else:
-                        sn.mean1 = sn.rstd1 = sn.h1 = None
+                    statn = torch.empty(2, M, device=dev, dtype=f32)
+                    sn.mean1, sn.rstd1 = statn[0], statn[1]
+                    del statn
+                    sn.h1 = torch.empty(M, C, device=dev, dtype=bf)
                     sn.qkv = torch.empty(M, 3 * C, device=dev, dtype=bf)
                     K.chain_fwd(st.y, st.x_in, st.wp, st.w1, st.w2, sn.wqkv, pb, b1, b2, sn.bqkv, ln2w, ln2b, params[1 + 16 * (i + 1)],
                                 params[2 + 16 * (i + 1)], st.x_mid, x_new, st.h2, st.a, sn.h1, sn.qkv, None, st.mean2, st.rstd2, sn.mean1, sn.rstd1)
@@ -399,15 +424,11 @@ class _Runner:
                 K.gemm_bf16_nt(st.a, st.w2, x_new, bias=b2, residual=st.x_mid, drop=self._drop("mlp", i))
             if self.capture is not None:
                 self.capture["relu.%d" % i] = st.a
-            free(st, "x_in", "y", "x_mid", "h2", "mean2", "rstd2", "a")
-            x, x_new = x_new, None
-            if keep:
-                saved.layers.append(st)
+            x = x_new
+            saved.layers.append(st)
         saved.x_last = x
         if not chain:
             K.layernorm_fwd(x, params[-2], params[-1], yf, saved.mean_f, saved.rstd_f)
-        if not keep:
-            saved = x = st = nxt = None
         outs = [torch.empty_like(f) for f in feats]
         K.upsample_add_fwd(self.geom, yf, feats if residual else [torch.zeros_like(f) for f in feats], outs)
         gps_out = yf.view(self.B, self.T, C)[:, self.Tm:, :].contiguous()
@@ -770,9 +791,11 @@ def fusion_stage(cfg, img, lidar, radar, gps_emb, params):
     When autograd would record no node for the call — grad mode off (``torch.no_grad``, ``torch.inference_mode``), or neither a
     map, ``gps_emb`` nor a parameter requiring grad — the stage runs the same kernels in the same order without keeping anything
     for a backward: each block's tensors are released once their last reader is enqueued, and the narrow stages' chain kernel
-    writes only what the next block reads.  The four outputs are bit-identical to the training forward's and do not require grad."""
+    writes only what the next block reads; in bf16 mode the whole stage is one ``dsf_stage_fwd`` call of the C ABI.  The four outputs
+    are bit-identical to the training forward's and do not require grad.  ``capture`` diagnostics (``cfg["capture"]``, or
+    ``cfg["dropout"]["capture"]``) take the training path."""
     needs_graph = torch.is_grad_enabled() and any(t.requires_grad for t in (img, lidar, radar, gps_emb, *params))
-    if needs_graph or cfg.get("capture") is not None:
+    if needs_graph or cfg.get("capture") is not None or "capture" in (cfg.get("dropout") or {}):
         return FusionStageFn.apply(cfg, img, lidar, radar, gps_emb, *params)
     with _stage_call(cfg, img, lidar, radar, gps_emb, params) as (r, feats, gps, plist, residual, _mf):
         outs, gps_out, _ = r.forward(feats, gps, plist, residual, keep=False)

@@ -22,6 +22,7 @@
 #ifndef DSFUSE_H_
 #define DSFUSE_H_
 
+#include <stddef.h>
 #include <stdint.h>
 
 #ifdef __cplusplus
@@ -295,6 +296,78 @@ int dsf_adamw_ema_pack(const dsf_opt_tensor* tensors_dev, const int32_t* tile0_d
 
 /* fp32 -> bf16 conversion (weight shadow refresh), n elements. */
 int dsf_cast_f32_bf16(const float* src, void* dst, int64_t n, void* stream);
+
+/* ---------------------------------------------------------------- whole fusion stage, inference forward (bf16 mode)
+ * One GPT fusion stage without a backward to follow (model2_seq.py:515-526: pool -> GPT -> upsample + residual), in one call:
+ * the token kernel, the embedding dropout, per block LayerNorm / fused QKV GEMM / flash attention and either the chain kernel
+ * (store-free variant) or proj / ln2 / fc1 / fc2, then ln_f unless the chain ended with it, the upsample-add and the copy of the
+ * two GPS token rows.  Each of those is one of the entry points above, launched on `stream` in that order; the call launches
+ * nothing else (dsf_launch_count advances by exactly their launches), allocates nothing and never synchronises, so it can be
+ * captured into a CUDA graph.  Compute mode is bf16 (tensor-core GEMMs and attention, fp32 residual stream). */
+
+/* nn.Dropout probabilities of one GPT in train() mode (model2_seq.py:104, 109/125, 272).  Site ids: 0 = embedding, and per block
+ * i 1 + 3i = attention, 2 + 3i = proj output, 3 + 3i = mlp output; see dsf_dropout for seed / step / seed_dev. */
+typedef struct {
+  float embd, attn, resid;    /* drop probabilities in [0, 1); 0 disables a site */
+  uint64_t seed;
+  uint32_t step;
+  const uint64_t* seed_dev;   /* nullable DEVICE pointer */
+} dsf_dropout_cfg;
+
+typedef struct {
+  dsf_geom geom;      /* maps and tokens; geom.C = n_embd */
+  int32_t n_head;     /* head size C / n_head in {16, 32, 64, 128}; C % 64 == 0 */
+  int32_t n_layer;    /* >= 0 */
+  int32_t F;          /* MLP width (block_exp * C), a multiple of 64 */
+  int32_t residual;   /* 1: out = feat + up(tokens) (Encoder); 0: out = up(tokens) (GPT.forward) */
+  int32_t chain;      /* -1: default rule (chain kernel at C = 64 and 128); 0 never, 1 C = 64, 2 C = 64 and 128 (as DSF_CHAIN).
+                       * It runs only when also F == 4C, n_layer > 0 and dropout is off. */
+  int32_t prepacked;  /* 1: dsf_stage_params.shadows will be given (the workspace then has no room for shadows), 0: it is NULL */
+  const dsf_dropout_cfg* dropout;  /* HOST pointer, nullable: NULL (or every p == 0) = no dropout */
+} dsf_stage_desc;
+
+/* bf16 weight shadows of one block, as dsf_pack_block_weights writes them (DEVICE pointers, 16-byte aligned). */
+typedef struct {
+  void *wqkv, *wqkv_t, *wp, *wp_t, *w1, *w1_t, *w2, *w2_t;
+  float* bqkv;
+} dsf_block_shadows;
+
+typedef struct {
+  /* HOST array of 1 + 16 * n_layer + 2 DEVICE pointers to the fp32 parameters in the reference's state-dict order: pos_emb (T, C),
+   * per block ln1.weight, ln1.bias, ln2.weight, ln2.bias, attn.{key, query, value}.{weight, bias}, attn.proj.{weight, bias},
+   * mlp.0.{weight, bias}, mlp.2.{weight, bias}, then ln_f.weight, ln_f.bias. */
+  const float* const* params;
+  /* HOST array of n_layer pre-packed shadows, or NULL: each block is then packed into the workspace from params (one
+   * dsf_pack_block_weights launch per block).  Given: repack = 1 re-packs each block into them first (one launch per block),
+   * repack = 0 uses them as they are. */
+  const dsf_block_shadows* shadows;
+  /* HOST array of n_layer cudaEvent_t (passed as void*), or NULL; entries may be NULL.  With pre-packed shadows, the call makes
+   * `stream` wait for ready[i] just before the first launch that reads block i's shadows, so shadows still being packed on
+   * another stream overlap the blocks before i (under CUDA-graph capture, events recorded in the same capture). */
+  void* const* ready;
+  int32_t repack;
+} dsf_stage_params;
+
+/* Workspace bytes dsf_stage_fwd needs for `d`.  With A(n) = n rounded up to a multiple of 256, M = B * T, T = (V + 2) * S * A_h * A_w + 2:
+ *     2 A(4MC)                          x (fp32 residual stream, ping-pong)
+ *   + A(2MC) + A(6MC) + A(2MC)          h1, qkv, y (bf16)
+ *   + A(4 B n_head T) + A(8M)           attention log-sum-exp, LayerNorm mean / rstd (fp32)
+ *   + A(4MC)                            yf (ln_f output, fp32)
+ *   + [no chain, n_layer > 0]  A(4MC) + A(2MC) + A(2MF)                x_mid (fp32), h2, a (bf16)
+ *   + [attention dropout]  A(4 dsf_attn_drop_words(B, T, n_head))     keep bits
+ *   + [prepacked == 0]  s (2 A(6C^2) + 2 A(2C^2) + 4 A(2FC) + A(12C))   bf16 shadows + fused QKV bias
+ *                       with s = 2 shadow slots if the chain runs and n_layer > 1, else min(n_layer, 1)
+ * Returns DSF_EINVAL (and *bytes = 0) for a descriptor dsf_stage_fwd would reject. */
+int dsf_stage_workspace_size(const dsf_stage_desc* d, size_t* bytes);
+
+/* img (B*V*S, C, H, W), lidar / radar (B*S, C, H, W) [geom.feat_dtype, geom.layout]; gps_emb (B, 2, C) fp32
+ *   -> img_out / lidar_out / radar_out, same shapes, dtype and layout as the maps, gps_out (B, 2, C) fp32.
+ * workspace: DEVICE memory of at least dsf_stage_workspace_size(d) bytes, 256-byte aligned, owned by the caller; it may be reused
+ * by the next call on the same stream.  Every pointer is checked (NULL, 16-byte alignment, workspace size and alignment) before
+ * anything is enqueued.  The outputs must not alias the inputs or the workspace. */
+int dsf_stage_fwd(const dsf_stage_desc* d, const dsf_stage_params* p, const void* img, const void* lidar, const void* radar,
+                  const float* gps_emb, void* img_out, void* lidar_out, void* radar_out, float* gps_out, void* workspace,
+                  size_t workspace_bytes, void* stream);
 
 #ifdef __cplusplus
 }
