@@ -22,7 +22,7 @@ EPI_BIAS, EPI_RELU, EPI_RESIDUAL, EPI_ACCUM = 1, 2, 4, 8
 SYMBOLS = [
     "dsf_version", "dsf_last_error", "dsf_launch_count", "dsf_check_device", "dsf_set_pdl", "dsf_set_sm_margin", "dsf_dropout_inplace", "dsf_tokens_fwd", "dsf_tokens_bwd",
     "dsf_layernorm_fwd", "dsf_layernorm_bwd", "dsf_gemm_bf16_nt", "dsf_gemm_bf16_tn", "dsf_gemm_set_impl", "dsf_gemm_f32",
-    "dsf_colsum", "dsf_relu_bwd", "dsf_relu_bwd_colsum", "dsf_pack_block_weights", "dsf_softmax_fwd", "dsf_softmax_bwd", "dsf_attn_fwd", "dsf_attn_bwd", "dsf_attn_bwd_parts", "dsf_attn_set_impl", "dsf_attn_drop_words",
+    "dsf_colsum", "dsf_relu_bwd", "dsf_relu_bwd_colsum", "dsf_pack_block_weights", "dsf_softmax_fwd", "dsf_softmax_bwd", "dsf_attn_fwd", "dsf_attn_bwd", "dsf_attn_bwd_parts", "dsf_attn_drop_words",
     "dsf_upsample_add_fwd", "dsf_upsample_add_bwd", "dsf_cast_f32_bf16", "dsf_opt_tiles", "dsf_adamw_ema_pack", "dsf_opt_upload_table", "dsf_chain_fwd",
     "dsf_stem_pack", "dsf_tail_fwd", "dsf_tail_bwd", "dsf_stage_workspace_size", "dsf_stage_fwd",
 ]
@@ -116,7 +116,6 @@ def lib():
             "dsf_attn_fwd": [P, P, P, c_int32, c_int32, c_int32, c_int32, POINTER(Dropout), P, P],
             "dsf_attn_bwd": [P, P, P, P, P, P, c_int32, c_int32, c_int32, c_int32, POINTER(Dropout), P, P],
             "dsf_attn_bwd_parts": [P, P, P, P, P, P, c_int32, c_int32, c_int32, c_int32, POINTER(Dropout), P, c_int32, P],
-            "dsf_attn_set_impl": [c_int32],
             "dsf_set_pdl": [c_int32],
             "dsf_set_sm_margin": [c_int32],
             "dsf_gemm_set_impl": [c_int32],
@@ -294,11 +293,6 @@ def set_pdl(on):
 def set_sm_margin(sms):
     """Size persistent grids for (SM count - sms): leaves room for concurrently running NCCL kernels (even, 0..64)."""
     _chk(lib().dsf_set_sm_margin(int(sms)), "dsf_set_sm_margin")
-
-
-def attn_set_impl(impl):
-    """Forward CTA shape: 0 = default (128-row CTAs, two per SM), 1 = force 128-row CTAs, 2 = force 256-row CTAs; process-wide."""
-    _chk(lib().dsf_attn_set_impl(impl), "dsf_attn_set_impl")
 
 
 def upsample_add_fwd(g, y, feats, outs):

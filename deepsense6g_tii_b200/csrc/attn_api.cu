@@ -3,7 +3,6 @@
 // (B, nh, T, T) score tensor is never materialised.  The kernels live in attn_tc2.cu; this file holds the C ABI, argument
 // checks and the small rowsum(dO * O) kernel of the backward.
 #include <algorithm>
-#include <atomic>
 
 #include "tc_common.cuh"
 
@@ -43,8 +42,7 @@ attn_delta_kernel(const __nv_bfloat16* __restrict__ y, const __nv_bfloat16* __re
 }
 
 // warp-specialised, TMA-fed kernels (attn_tc2.cu)
-int attn_fwd_run(const void* qkv, void* y, float* lse, int B, int T, int C, int nh, const dsf_dropout* drop, uint32_t* bits, int force_nwg,
-                 cudaStream_t st);
+int attn_fwd_run(const void* qkv, void* y, float* lse, int B, int T, int C, int nh, const dsf_dropout* drop, uint32_t* bits, cudaStream_t st);
 int attn_bwd_run(const void* qkv, const void* y, const void* dy, const float* lse, float* delta, void* dqkv, int B, int T, int C, int nh,
                  const dsf_dropout* drop, uint32_t* bits, int parts, cudaStream_t st);
 
@@ -54,19 +52,9 @@ int run_attn_delta(const void* y, const void* dy, float* delta, int B, int T, in
   return check_launch("attn_bwd/delta");
 }
 
-// forward CTA shape: 0 = default (128-row CTAs, two per SM), 1 = force 128-row CTAs, 2 = force 256-row CTAs (one per SM, two
-// softmax warpgroups sharing each K/V tile).  Read with relaxed atomics: calls are re-entrant, the selector is a tuning knob.
-static std::atomic<int> g_attn_impl{0};
-
 }  // namespace dsf
 
 using namespace dsf;
-
-extern "C" int dsf_attn_set_impl(int32_t impl) {
-  DSF_REQUIRE(impl >= 0 && impl <= 2, "attn_set_impl: impl must be 0 (default), 1 (128-row forward CTAs) or 2 (256-row forward CTAs)");
-  g_attn_impl.store(impl, std::memory_order_relaxed);
-  return DSF_OK;
-}
 
 static int check_attn_drop(const char* who, const dsf_dropout* drop, const uint32_t* bits, bool& on) {
   on = drop && drop->p > 0.f;
@@ -96,7 +84,7 @@ extern "C" int dsf_attn_fwd(const void* qkv, void* y, float* lse, int32_t B, int
   DSF_REQUIRE(aligned16(qkv) && aligned16(y), "attn_fwd: 16-byte alignment required");
   DSF_REQUIRE(B <= 65535 && nh <= 65535, "attn_fwd: grid too large");
   if (int e = check_head_size("attn_fwd", C / nh)) return e;
-  return attn_fwd_run(qkv, y, lse, B, T, C, nh, drop_on ? drop : nullptr, drop_bits, g_attn_impl.load(std::memory_order_relaxed), (cudaStream_t)stream);
+  return attn_fwd_run(qkv, y, lse, B, T, C, nh, drop_on ? drop : nullptr, drop_bits, (cudaStream_t)stream);
 }
 
 static int attn_bwd_impl(const void* qkv, const void* y, const void* dy, const float* lse, float* delta, void* dqkv, int32_t B, int32_t T,

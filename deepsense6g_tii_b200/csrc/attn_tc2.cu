@@ -5,13 +5,13 @@
 //     token rows zero-filled) into swizzled shared memory through an mbarrier ring,
 //   * one elected thread issues every tcgen05.mma, running ahead of the math warps (S(j+1) is issued before
 //     softmax(j) finishes; the P.V / dV / dK / dQ MMAs are issued as soon as the bf16 tile lands in smem),
-//   * forward: two softmax warpgroups (2 x 128 query rows) share each K/V tile (ping-pong on the tensor pipe),
+//   * forward: one softmax warpgroup per 128 query rows, two CTAs per SM; S and P are double-buffered in TMEM,
 //   * backward: accumulators (dK, dV / dQ) stay in TMEM across the whole loop, S/dP are double-buffered.
 // Shared-memory operand images: TMA tiles are [half][row][ROWB bytes] with the hardware swizzle that matches
 // ROWB (128/64/32 B for head sizes >=64/32/16); the same image is read as a K-major operand (rows = M/N)
-// or an MN-major operand (rows = K).  P / dS tiles written by threads use the no-swizzle core-matrix layout.
+// or an MN-major operand (rows = K).  P / dS are written by the math warps back into tensor memory (bf16, two
+// per column) and feed the next MMA as TS-mode A operands.
 #include <algorithm>
-#include <cstdlib>
 
 #include "tc_common.cuh"
 
@@ -25,8 +25,9 @@ __device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap* m, 
       "l"(reinterpret_cast<uint64_t>(m)), "r"(bar), "r"(c0), "r"(c1), "r"(c2)
       : "memory");
 }
-// ---- optional in-kernel timeline (make trace -> libdsfuse_trace.so, scripts/attn_trace.py): CTA (0,0,0) of the forward
-// kernel stamps clock64() at the hand-over points of its MMA warp and of one softmax warp per warpgroup.
+// ---- optional in-kernel timeline (make trace -> libdsfuse_trace.so, scripts/attn_trace.py): CTA (0,0,0) of the forward and
+// dK/dV kernels stamps clock64() at the hand-over points of one warp per math warpgroup (rows 0, 1; the forward has one) and
+// of its MMA warp (row 2).
 #ifdef DSF_ATTN_TRACE
 __device__ long long g_attn_trace[3][64][6];
 #define TRACE(who, it, slot)                                                                               \
@@ -69,19 +70,11 @@ __device__ __forceinline__ void ex2_poly2(uint64_t x, float& p0, float& p1) {
   p1 = __int_as_float(__float_as_int(q1) + (__float_as_int(t1) << 23));
 }
 
-// 2^x of a packed pair: pair number j of a tile goes to the polynomial when POLY > 0 and j % POLY == POLY - 1, else to MUFU.EX2
-template <int POLY>
-__device__ __forceinline__ uint64_t ex2_pair(uint64_t x, int j) {
-  float p0, p1;
-  if (POLY > 0 && (j % (POLY > 0 ? POLY : 1)) == POLY - 1) {
-    ex2_poly2(x, p0, p1);
-  } else {
-    float x0, x1;
-    unpack2(x, x0, x1);
-    p0 = ex2_approx(x0);
-    p1 = ex2_approx(x1);
-  }
-  return pack2(p0, p1);
+// 2^x of a packed pair on MUFU.EX2
+__device__ __forceinline__ uint64_t ex2_pair(uint64_t x) {
+  float x0, x1;
+  unpack2(x, x0, x1);
+  return pack2(ex2_approx(x0), ex2_approx(x1));
 }
 // (Packing on the ALU pipe instead of cvt.rn.bf16x2 — bit pattern + 0x8000, then one byte permute per pair — measured slower in all
 // three kernels: forward 24.4 -> 25.7 us, dK/dV 28.7 -> 30.7 us at head size 16; profiles/r02al_attn_pack_alu.txt.)
@@ -121,9 +114,6 @@ __device__ __forceinline__ uint32_t attn_keep_word(const AttnDrop& a, uint64_t r
 __device__ __forceinline__ void named_bar_sync(int id, int nthreads) {
   asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
 }
-__device__ __forceinline__ void named_bar_arrive(int id, int nthreads) {
-  asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
-}
 
 template <int HS>
 struct HeadCfg {
@@ -147,12 +137,6 @@ __device__ __forceinline__ uint64_t mnmaj_desc(uint32_t tile, int R, int kk) {
   using H = HeadCfg<HS>;
   return make_smem_desc(tile + (uint32_t)kk * 16 * H::ROWB, (uint32_t)R * H::ROWB, 8 * H::ROWB, H::SWZ);
 }
-// K-major operand over a thread-written no-swizzle [128 x KC] bf16 tile (core matrices: 128 B along K, KC*16 B along M)
-template <int KC>
-__device__ __forceinline__ uint64_t pdesc(uint32_t tile, int kk) {
-  return make_smem_desc(tile + (uint32_t)kk * 256, 128, KC * 16, SWZ_NONE);
-}
-
 // The MMA-issuing helpers below are WARP-COLLECTIVE: all 32 lanes of the issuer warp call them with uniform
 // arguments.  Base descriptors are computed in warp-uniform control flow (so they live in uniform registers) and
 // per-k-step offsets are compile-time immediates; only the tcgen05.mma / tcgen05.commit themselves run under
@@ -177,25 +161,10 @@ __device__ __forceinline__ void mma_over_head(uint32_t tmem_d, uint32_t a_tile, 
   }
   __syncwarp();
 }
-// D[128 x HS] (+)= P(no-swizzle [128 x KC]) . B(tile with KC rows, MN-major)
-template <int HS, int KC>
-__device__ __forceinline__ void mma_over_rows(uint32_t tmem_d, uint32_t p_tile, uint32_t b_tile, uint32_t idesc, bool accumulate) {
-  using H = HeadCfg<HS>;
-  const uint64_t dp = make_smem_desc(p_tile, 128, KC * 16, SWZ_NONE);
-  const uint64_t db = make_smem_desc(b_tile, (uint32_t)KC * H::ROWB, 8 * H::ROWB, H::SWZ);
-  const uint32_t acc = accumulate ? 1u : 0u;
-  if (elect_one()) {
-#pragma unroll
-    for (int kk = 0; kk < KC / 16; ++kk)
-      tc_mma_bf16(tmem_d, dp + (uint32_t)((kk * 256) >> 4), db + (uint32_t)((kk * 16 * H::ROWB) >> 4), idesc, kk == 0 ? acc : 1u);
-  }
-  __syncwarp();
-}
-
 // D[128 x HS] (+)= P(tensor memory, [128 x KC] bf16 packed two per column at p_tmem) . B(tile with KC rows, MN-major)
-// CW = 0: the packed columns are contiguous (8 per K = 16 step).  CW = 32 / 16 (backward kernels): every math warpgroup owns CW
-// fp32 columns of the tile and overwrites the first CW / 2 of them with its packed values, so K-step kk (16 values = 8 packed
-// columns) sits at column (16 kk / CW) * CW + (16 kk % CW) / 2: 0, 8, 32, 40 for CW = 32 and 0, 16, 32, 48 for CW = 16.
+// CW = 0 (forward): the packed columns are contiguous (8 per K = 16 step).  CW = 32 (backward kernels): every math warpgroup owns
+// 32 fp32 columns of the tile and overwrites the first 16 of them with its packed values, so K-step kk (16 values = 8 packed
+// columns) sits at column (16 kk / CW) * CW + (16 kk % CW) / 2: 0, 8, 32, 40.
 template <int HS, int KC, int CW = 0>
 __device__ __forceinline__ void mma_over_rows_ts(uint32_t tmem_d, uint32_t p_tmem, uint32_t b_tile, uint32_t idesc, bool accumulate) {
   using H = HeadCfg<HS>;
@@ -233,16 +202,6 @@ __device__ __forceinline__ void tma_tile(uint32_t dst, const CUtensorMap* m, uin
   for (int hf = 0; hf < H::NHALF; ++hf) tma_load_3d(dst + hf * R * H::ROWB, m, bar, col0 + hf * H::BOXC, row0, b);
 }
 
-// write 32 bf16 values (16 packed words) of row `row`, columns c..c+31 of a no-swizzle [128 x KC] tile
-template <int KC>
-__device__ __forceinline__ void store_p32(uint8_t* tile, int row, int c, const uint32_t (&pk)[16]) {
-#pragma unroll
-  for (int cc = 0; cc < 4; ++cc) {
-    uint8_t* dst = tile + ((size_t)(row >> 3) * (KC / 8) + (c >> 3) + cc) * 128 + (row & 7) * 16;
-    *reinterpret_cast<uint4*>(dst) = make_uint4(pk[4 * cc], pk[4 * cc + 1], pk[4 * cc + 2], pk[4 * cc + 3]);
-  }
-}
-
 __device__ __forceinline__ void store_row16_bf16(__nv_bfloat16* dst, const uint32_t (&a)[16], float scale) {
 #pragma unroll
   for (int e = 0; e < 16; e += 8)
@@ -260,32 +219,29 @@ __device__ __forceinline__ void store_row16_bf16(__nv_bfloat16* dst, const uint3
 // P^T / dS^T are written back (bf16, two per column) over the S^T / dP^T tiles in tensor memory and feed the dV / dK MMAs as
 // TS-mode A operands; per-query statistics (lse, delta) are staged per WARP in shared memory (each lane fetches one pair a
 // tile ahead, a __syncwarp publishes them), so the math warps never meet at a CTA-wide barrier inside the loop.
-//
-// NP = math warpgroup PAIRS: 2 NP warpgroups of 128 threads split a tile's 64 query columns in 64 / (2 NP) = 32 or 16 columns
-// each (all of them work on EVERY tile).  The in-kernel timeline shows the math warps as the critical path at head sizes <= 64:
-// the same warps take tile after tile, so a tile costs their whole latency chain (tcgen05.ld -> MUFU -> tcgen05.st -> wait::st ->
-// mbarrier) — halving the columns per warp shortens that chain; the MMA / TMA schedule is unchanged (ds_full collects 256 NP arrivals).
-template <int HS, int BQ, int ST, int NP>
+// Two math warpgroups of 128 threads split a tile's 64 query columns, 32 each (both work on EVERY tile); the note above
+// launch_bwd_kv has the measurements of the four-warpgroup variant that was removed.
+template <int HS, int BQ, int ST>
 struct BwdKV2 {
   static constexpr int KV_BYTES = 128 * HS * 2, Q_BYTES = BQ * HS * 2;
   static constexpr int K_OFF = 0, V_OFF = KV_BYTES, Q_OFF = 2 * KV_BYTES, DO_OFF = Q_OFF + ST * Q_BYTES;
   static constexpr int BAR_OFF = DO_OFF + ST * Q_BYTES;
   static constexpr int NBAR = 2 + 2 * ST + 4;
   static constexpr int STAT_OFF = BAR_OFF + NBAR * 8 + 16;  // lse (log2 units) | delta of ALL queries of this (batch, head), padded to tiles
-  static constexpr int THREADS = 256 * NP + 64;
+  static constexpr int THREADS = 256 + 64;
   static_assert(4 * BQ + 2 * HS <= 512, "TMEM budget");
   static_assert(STAT_OFF % 16 == 0, "float4 reads of the statistics");
   static int dyn_bytes(int T) { return STAT_OFF + 2 * cdiv(T, BQ) * BQ * 4 + 1024; }
 };
 
-// POLY: every POLY-th pair of exponentials on the FMA pipe (ex2_poly2); the dropout-free math runs on packed fp32 pairs.
-template <int HS, int BQ, int ST, int NP, bool DROP, int POLY>
-__global__ void __launch_bounds__(256 * NP + 64, 1)
+// The dropout-free math runs on packed fp32 pairs.
+template <int HS, int BQ, int ST, bool DROP>
+__global__ void __launch_bounds__(256 + 64, 1)
 attn_bwd_kv2_kernel(const __grid_constant__ CUtensorMap tmKV, const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmDO,
                     const float* __restrict__ lse, const float* __restrict__ delta, __nv_bfloat16* __restrict__ dqkv, int T, int C, int nh,
                     float scale, AttnDrop ad) {
-  using L = BwdKV2<HS, BQ, ST, NP>;
-  constexpr int MMAW = 8 * NP, TMAW = 8 * NP + 1;  // warp roles: 0 .. 8*NP-1 math, then MMA issuer, TMA producer
+  using L = BwdKV2<HS, BQ, ST>;
+  constexpr int MMAW = 8, TMAW = 9;  // warp roles: 0 .. 7 math, then MMA issuer, TMA producer
   extern __shared__ uint8_t smem_raw[];
   const uint32_t sbase = (smem_u32(smem_raw) + 1023u) & ~1023u;
   uint8_t* smem = smem_raw + (sbase - smem_u32(smem_raw));
@@ -301,7 +257,7 @@ attn_bwd_kv2_kernel(const __grid_constant__ CUtensorMap tmKV, const __grid_const
     mbar_init(kv_full, 1);
     mbar_init(acc_done, 1);
     for (int s = 0; s < ST; ++s) { mbar_init(q_full + 8 * s, 1); mbar_init(q_empty + 8 * s, 1); }
-    for (int w = 0; w < 2; ++w) { mbar_init(s_full + 8 * w, 1); mbar_init(ds_full + 8 * w, 256 * NP); }
+    for (int w = 0; w < 2; ++w) { mbar_init(s_full + 8 * w, 1); mbar_init(ds_full + 8 * w, 256); }
     fence_barrier_init();
   }
   if (warp == MMAW) { tmem_alloc(tmem_slot, 512); tmem_relinquish(); }
@@ -354,23 +310,23 @@ attn_bwd_kv2_kernel(const __grid_constant__ CUtensorMap tmKV, const __grid_const
         mbar_wait(ds_full + 8 * bf, (i >> 1) & 1);
         TRACE(2, i, 3);
         tc_fence_after();
-        mma_over_rows_ts<HS, BQ, 32 / NP>(tm_dv, tmem_base + bf * 2 * BQ, sbase + L::DO_OFF + st * L::Q_BYTES, idesc_g, i > 0);
-        mma_over_rows_ts<HS, BQ, 32 / NP>(tm_dk, tmem_base + bf * 2 * BQ + BQ, sbase + L::Q_OFF + st * L::Q_BYTES, idesc_g, i > 0);
+        mma_over_rows_ts<HS, BQ, 32>(tm_dv, tmem_base + bf * 2 * BQ, sbase + L::DO_OFF + st * L::Q_BYTES, idesc_g, i > 0);
+        mma_over_rows_ts<HS, BQ, 32>(tm_dk, tmem_base + bf * 2 * BQ + BQ, sbase + L::Q_OFF + st * L::Q_BYTES, idesc_g, i > 0);
         tc_commit_elect(q_empty + 8 * st);
         TRACE(2, i, 4);
       }
       tc_commit_elect(acc_done);
     }
   } else {
-    constexpr int CW = BQ / (2 * NP);  // query columns of a tile per warpgroup
-    const int wgi = warp >> 2;         // warpgroup 0 .. 2 NP - 1: columns wgi * CW ..
+    constexpr int CW = BQ / 2;  // query columns of a tile per warpgroup
+    const int wgi = warp >> 2;  // warpgroup 0 / 1: columns wgi * CW ..
     const int row = (warp & 3) * 32 + lane;
     const uint32_t lane_off = (uint32_t)((warp & 3) * 32) << 16;
     const bool key_ok = (kv0 + row) < T;
     const float scale_log2 = scale * 1.4426950408889634f;
     const float* lse_g = lse + ((size_t)b * nh + h) * T;
     const float* delta_g = delta + ((size_t)b * nh + h) * T;
-    static_assert(BQ == 64 && (CW == 32 || CW == 16), "a 64-query tile in 32- or 16-column shares");
+    static_assert(BQ == 64, "a 64-query tile in two 32-column shares");
     const size_t bh = (size_t)b * nh + h;
     const int kw = kv0 / 32 + (warp & 3);  // bitmap word holding this warp's 32 keys
     // lse (log2 units) and delta of every query of this (batch, head) are copied to shared memory ONCE by the math warps
@@ -378,7 +334,7 @@ attn_bwd_kv2_kernel(const __grid_constant__ CUtensorMap tmKV, const __grid_const
     // tile and warp cost ~250 of the ~1200 cycles a math warp spends on a tile.)  Padding queries get lse = +inf -> P = 0.  Both are stored negated.
     float* s_lse = reinterpret_cast<float*>(smem + L::STAT_OFF);
     float* s_delta = s_lse + n_q * BQ;
-    for (int idx = threadIdx.x; idx < n_q * BQ; idx += 256 * NP) {
+    for (int idx = threadIdx.x; idx < n_q * BQ; idx += 256) {
       s_lse[idx] = idx < T ? __ldg(lse_g + idx) * -1.4426950408889634f : -INFINITY;  // NEGATED: x = s * c + (-lse), d = p * (dp + (-delta))
       s_delta[idx] = idx < T ? -__ldg(delta_g + idx) : 0.f;
     }
@@ -389,26 +345,26 @@ attn_bwd_kv2_kernel(const __grid_constant__ CUtensorMap tmKV, const __grid_const
       wv = qq < T ? ad.bits[(bh * T + qq) * ad.Tw + kw] : 0u;
     };
     if (DROP) fetch_w(0);
-    named_bar_sync(1, 256 * NP);  // statistics visible to all math warps
+    named_bar_sync(1, 256);  // statistics visible to all math warps
     for (int i = 0; i < n_q; ++i) {
       const int bf = i & 1;
       const float* wst = s_lse + i * BQ + wgi * CW;
       const float* wsd = s_delta + i * BQ + wgi * CW;
       const uint32_t myw = wv;
-      if ((warp & 3) == 0 && wgi < 2) TRACE(wgi, i, 0);
+      if ((warp & 3) == 0) TRACE(wgi, i, 0);
       if (DROP && i + 1 < n_q) fetch_w(i + 1);
-      if ((warp & 3) == 0 && wgi < 2) TRACE(wgi, i, 1);
+      if ((warp & 3) == 0) TRACE(wgi, i, 1);
       // s_full(i) also says that buffer bf is free: S^T / dP^T (i) were issued after dV / dK (i-2), the MMAs of one thread
       // complete in order, and the commit covers every MMA issued before it
       mbar_wait(s_full + 8 * bf, (i >> 1) & 1);
-      if ((warp & 3) == 0 && wgi < 2) TRACE(wgi, i, 2);
+      if ((warp & 3) == 0) TRACE(wgi, i, 2);
       tc_fence_after();
       const uint32_t tm_s = tmem_base + bf * 2 * BQ + lane_off + wgi * CW, tm_dp = tm_s + BQ;
       uint32_t rs[CW], rp[CW];
-      if constexpr (CW == 32) { tmem_ld32(tm_s, rs); tmem_ld32(tm_dp, rp); }
-      else { tmem_ld16(tm_s, rs); tmem_ld16(tm_dp, rp); }
+      tmem_ld32(tm_s, rs);
+      tmem_ld32(tm_dp, rp);
       tmem_wait_ld();
-      if ((warp & 3) == 0 && wgi < 2) TRACE(wgi, i, 3);
+      if ((warp & 3) == 0) TRACE(wgi, i, 3);
       const uint64_t sc2 = pack2(scale_log2, scale_log2);
 #pragma unroll
       for (int c = 0; c < CW; c += 16) {
@@ -423,7 +379,7 @@ attn_bwd_kv2_kernel(const __grid_constant__ CUtensorMap tmKV, const __grid_const
 #pragma unroll
             for (int u = 0; u < 4; u += 2) {
               const uint64_t x = fma2(pack2(__uint_as_float(rs[c + e + u]), __uint_as_float(rs[c + e + u + 1])), sc2, u ? nl.y : nl.x);
-              const uint64_t p2 = ex2_pair<POLY>(x, (c + e + u) / 2);
+              const uint64_t p2 = ex2_pair(x);
               const uint64_t t2 = add2(pack2(__uint_as_float(rp[c + e + u]), __uint_as_float(rp[c + e + u + 1])), u ? nd.y : nd.x);
               pk[(e + u) / 2] = pack_bf16x2_pair(p2);
               dk[(e + u) / 2] = pack_bf16x2_pair(mul2(p2, t2));
@@ -454,24 +410,23 @@ attn_bwd_kv2_kernel(const __grid_constant__ CUtensorMap tmKV, const __grid_const
         tmem_st8(tm_s + c / 2, pk);
         tmem_st8(tm_dp + c / 2, dk);
       }
-      if ((warp & 3) == 0 && wgi < 2) TRACE(wgi, i, 4);
+      if ((warp & 3) == 0) TRACE(wgi, i, 4);
       tmem_wait_st();
       tc_fence_before();
       mbar_arrive(ds_full + 8 * bf);
-      if ((warp & 3) == 0 && wgi < 2) TRACE(wgi, i, 5);
+      if ((warp & 3) == 0) TRACE(wgi, i, 5);
     }
     mbar_wait(acc_done, 0);
     tc_fence_after();
     const int ld = 3 * C;
     __nv_bfloat16* dk_row = dqkv + ((size_t)b * T + kv0 + row) * ld + C + h * HS;
     __nv_bfloat16* dv_row = dk_row + C;
-    // even warpgroups drain dK, odd ones dV; with two pairs each takes half of the head's columns (hs = 16: the first pair only)
-    constexpr int NSPLIT = (NP == 2 && HS >= 32) ? 2 : 1;
-    constexpr int CH = HS / NSPLIT;
+    // warpgroup 0 drains dK, warpgroup 1 dV.  (wgi is 0 or 1, but the compiler cannot tell: `which` and `part` keep the
+    // instructions this kernel was measured with.)
     const int which = wgi & 1, part = wgi >> 1;
-    if (part < NSPLIT) {
+    if (part < 1) {
 #pragma unroll 1
-      for (int c = part * CH; c < (part + 1) * CH; c += 16) {
+      for (int c = part * HS; c < (part + 1) * HS; c += 16) {
         uint32_t a[16];
         tmem_ld16((which == 0 ? tm_dk : tm_dv) + lane_off + c, a);
         tmem_wait_ld();
@@ -488,30 +443,32 @@ attn_bwd_kv2_kernel(const __grid_constant__ CUtensorMap tmKV, const __grid_const
 // CTA = 128 queries (Q, dO resident); loop over 64-key tiles.  Threads own query rows:
 //   S = Q K^T, dP = dO V^T -> dS = exp2(S*c - lse) (dP - delta) * scale -> dQ += dS K
 // dS (bf16) is written back over the dP tile in tensor memory and feeds dQ += dS K as a TS-mode A operand.
+// The two stationary operands, the Q and dO rows of the CTA's 128 queries, live in tensor memory (written once by the math
+// warps straight from global memory) and feed the S = Q K^T and dP = dO V^T MMAs as TS-mode A operands.  A tcgen05.mma whose A
+// operand comes from shared memory spends ~128 cycles fetching its 128 x 16 slice whatever N is, so the 64-wide S / dP MMAs ran
+// at a quarter of the tensor pipe's rate; from tensor memory they are N-bound (measured +-0 at T = 962, +6 % at T = 3842; the
+// shared-memory variant was removed).
 template <int HS, int ST>
 struct BwdQ2 {
   static constexpr int BKV = 64;
   static constexpr int Q_BYTES = 128 * HS * 2, KV_BYTES = BKV * HS * 2;
-  static constexpr int Q_OFF = 0, DO_OFF = Q_BYTES, K_OFF = 2 * Q_BYTES, V_OFF = K_OFF + ST * KV_BYTES;
+  // the K / V rings start after 2 * Q_BYTES that nothing reads (where the shared-memory Q / dO tiles were): the layout as measured
+  static constexpr int K_OFF = 2 * Q_BYTES, V_OFF = K_OFF + ST * KV_BYTES;
   static constexpr int BAR_OFF = V_OFF + ST * KV_BYTES;
   static constexpr int NBAR = 2 + 2 * ST + 4;
   static constexpr int DYN = BAR_OFF + NBAR * 8 + 16 + 1024;
   static_assert(4 * BKV + HS <= 512, "TMEM budget");
 };
 
-// AT = true: the two stationary operands of this kernel, the Q and dO rows of the CTA's 128 queries, live in tensor memory
-// (written once by the math warps straight from global memory) and feed the S = Q K^T and dP = dO V^T MMAs as TS-mode A
-// operands.  A tcgen05.mma whose A operand comes from shared memory spends ~128 cycles fetching its 128 x 16 slice whatever
-// N is, so the 64-wide S / dP MMAs ran at a quarter of the tensor pipe's rate; from tensor memory they are N-bound.
-// NP = math warpgroup pairs, as in the dK/dV kernel: 2 NP warpgroups share every key tile (64 / (2 NP) columns each).
-template <int HS, int ST, bool AT, int NP, bool DROP, int POLY>
-__global__ void __launch_bounds__(256 * NP + 64, 1)
+// Two math warpgroups share every key tile (32 columns each), as in the dK/dV kernel.
+template <int HS, int ST, bool DROP>
+__global__ void __launch_bounds__(256 + 64, 1)
 attn_bwd_q2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmDO, const __grid_constant__ CUtensorMap tmKV,
                    const float* __restrict__ lse, const float* __restrict__ delta, __nv_bfloat16* __restrict__ dqkv, int T, int C, int nh,
                    float scale, AttnDrop ad, const __nv_bfloat16* __restrict__ qkv, const __nv_bfloat16* __restrict__ dy) {
   using L = BwdQ2<HS, ST>;
   constexpr int BKV = L::BKV;
-  constexpr int MMAW = 8 * NP, TMAW = 8 * NP + 1;
+  constexpr int MMAW = 8, TMAW = 9;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t sbase = (smem_u32(smem_raw) + 1023u) & ~1023u;
   const uint32_t bar0 = sbase + L::BAR_OFF;
@@ -520,15 +477,15 @@ attn_bwd_q2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
   const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0), lane = threadIdx.x & 31;  // warp-uniform for the compiler
   const int q0 = blockIdx.x * 128, h = blockIdx.y, b = blockIdx.z;
   const int n_kv = (T + BKV - 1) / BKV;
-  constexpr uint32_t TMEM_COLS = (4 * BKV + HS + (AT ? (HS >= 32 ? HS : 32) : 0)) <= 256 ? 256 : 512;
+  constexpr uint32_t TMEM_COLS = (4 * BKV + HS + (HS >= 32 ? HS : 32)) <= 256 ? 256 : 512;
   static_assert(4 * BKV + 2 * HS <= 512, "TMEM budget (S/dP double-buffered, dQ, Q and dO rows)");
 
   pdl_trigger();
   if (threadIdx.x == 0) {
-    mbar_init(q_full, AT ? 256 : 1);
+    mbar_init(q_full, 256);
     mbar_init(acc_done, 1);
     for (int s = 0; s < ST; ++s) { mbar_init(kv_full + 8 * s, 1); mbar_init(kv_empty + 8 * s, 1); }
-    for (int w = 0; w < 2; ++w) { mbar_init(s_full + 8 * w, 1); mbar_init(ds_full + 8 * w, 256 * NP); }
+    for (int w = 0; w < 2; ++w) { mbar_init(s_full + 8 * w, 1); mbar_init(ds_full + 8 * w, 256); }
     fence_barrier_init();
   }
   if (warp == MMAW) { tmem_alloc(tmem_slot, TMEM_COLS); tmem_relinquish(); }
@@ -540,15 +497,10 @@ attn_bwd_q2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
   asm volatile("ld.shared.b32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot));
   pdl_wait();  // set-up above overlaps the previous kernel's tail
   const uint32_t tm_dq = tmem_base + 4 * BKV;
-  const uint32_t tm_q = tm_dq + HS, tm_do = tm_q + (HS >= 32 ? HS / 2 : 16);  // AT: packed Q / dO rows (HS/2 columns each, >= 16 apart)
+  const uint32_t tm_q = tm_dq + HS, tm_do = tm_q + (HS >= 32 ? HS / 2 : 16);  // packed Q / dO rows (HS/2 columns each, >= 16 apart)
 
   if (warp == TMAW) {
     if (lane == 0) {
-      if (!AT) {
-        mbar_expect_tx(q_full, 2 * L::Q_BYTES);
-        tma_tile<HS>(sbase + L::Q_OFF, &tmQ, q_full, h * HS, q0, b, 128);
-        tma_tile<HS>(sbase + L::DO_OFF, &tmDO, q_full, h * HS, q0, b, 128);
-      }
       for (int j = 0; j < n_kv; ++j) {
         const int st = j % ST;
         if (j >= ST) mbar_wait(kv_empty + 8 * st, ((j / ST) - 1) & 1);
@@ -564,13 +516,8 @@ attn_bwd_q2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
       mbar_wait(q_full, 0);
       mbar_wait(kv_full, 0);
       tc_fence_after();
-      if (AT) {
-        mma_over_head_ts<HS>(tmem_base, tm_q, sbase + L::K_OFF, BKV, idesc_s);
-        mma_over_head_ts<HS>(tmem_base + BKV, tm_do, sbase + L::V_OFF, BKV, idesc_s);
-      } else {
-        mma_over_head<HS>(tmem_base, sbase + L::Q_OFF, 128, sbase + L::K_OFF, BKV, idesc_s);
-        mma_over_head<HS>(tmem_base + BKV, sbase + L::DO_OFF, 128, sbase + L::V_OFF, BKV, idesc_s);
-      }
+      mma_over_head_ts<HS>(tmem_base, tm_q, sbase + L::K_OFF, BKV, idesc_s);
+      mma_over_head_ts<HS>(tmem_base + BKV, tm_do, sbase + L::V_OFF, BKV, idesc_s);
       tc_commit_elect(s_full);
       for (int j = 0; j < n_kv; ++j) {
         const int bf = j & 1, st = j % ST;
@@ -578,26 +525,21 @@ attn_bwd_q2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
           const int sn = (j + 1) % ST, bn = (j + 1) & 1;
           mbar_wait(kv_full + 8 * sn, ((j + 1) / ST) & 1);
           tc_fence_after();
-          if (AT) {
-            mma_over_head_ts<HS>(tmem_base + bn * 2 * BKV, tm_q, sbase + L::K_OFF + sn * L::KV_BYTES, BKV, idesc_s);
-            mma_over_head_ts<HS>(tmem_base + bn * 2 * BKV + BKV, tm_do, sbase + L::V_OFF + sn * L::KV_BYTES, BKV, idesc_s);
-          } else {
-            mma_over_head<HS>(tmem_base + bn * 2 * BKV, sbase + L::Q_OFF, 128, sbase + L::K_OFF + sn * L::KV_BYTES, BKV, idesc_s);
-            mma_over_head<HS>(tmem_base + bn * 2 * BKV + BKV, sbase + L::DO_OFF, 128, sbase + L::V_OFF + sn * L::KV_BYTES, BKV, idesc_s);
-          }
+          mma_over_head_ts<HS>(tmem_base + bn * 2 * BKV, tm_q, sbase + L::K_OFF + sn * L::KV_BYTES, BKV, idesc_s);
+          mma_over_head_ts<HS>(tmem_base + bn * 2 * BKV + BKV, tm_do, sbase + L::V_OFF + sn * L::KV_BYTES, BKV, idesc_s);
           tc_commit_elect(s_full + 8 * bn);
         }
         mbar_wait(ds_full + 8 * bf, (j >> 1) & 1);
         tc_fence_after();
-        mma_over_rows_ts<HS, BKV, 32 / NP>(tm_dq, tmem_base + bf * 2 * BKV + BKV, sbase + L::K_OFF + st * L::KV_BYTES, idesc_q, j > 0);
+        mma_over_rows_ts<HS, BKV, 32>(tm_dq, tmem_base + bf * 2 * BKV + BKV, sbase + L::K_OFF + st * L::KV_BYTES, idesc_q, j > 0);
         tc_commit_elect(kv_empty + 8 * st);
       }
       tc_commit_elect(acc_done);
     }
   } else {
-    constexpr int CW = BKV / (2 * NP);  // key columns of a tile per warpgroup
-    static_assert(BKV == 64 && (CW == 32 || CW == 16), "a 64-key tile in 32- or 16-column shares");
-    const int wgi = warp >> 2;          // warpgroup 0 .. 2 NP - 1: columns wgi * CW ..
+    constexpr int CW = BKV / 2;  // key columns of a tile per warpgroup
+    static_assert(BKV == 64, "a 64-key tile in two 32-column shares");
+    const int wgi = warp >> 2;   // warpgroup 0 / 1: columns wgi * CW ..
     const int row = (warp & 3) * 32 + lane;
     const uint32_t lane_off = (uint32_t)((warp & 3) * 32) << 16;
     const int q = q0 + row;
@@ -605,7 +547,7 @@ attn_bwd_q2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
     const float scale_log2 = scale * 1.4426950408889634f;
     const float my_lse = q_ok ? lse[((size_t)b * nh + h) * T + q] * 1.4426950408889634f : INFINITY;
     const float my_delta = q_ok ? delta[((size_t)b * nh + h) * T + q] : 0.f;
-    if (AT && wgi < 2) {  // warpgroup 0 parks the Q row of its query in tensor memory, warpgroup 1 the dO row (two bf16 per column)
+    if (wgi < 2) {  // warpgroup 0 parks the Q row of its query in tensor memory, warpgroup 1 the dO row (two bf16 per column)
       const __nv_bfloat16* src = wgi == 0 ? qkv + ((size_t)b * T + q) * (3 * C) + h * HS : dy + ((size_t)b * T + q) * C + h * HS;
       const uint32_t dst = (wgi == 0 ? tm_q : tm_do) + lane_off;
 #pragma unroll 1
@@ -636,8 +578,8 @@ attn_bwd_q2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
       const uint32_t tm_s = tmem_base + bf * 2 * BKV + lane_off + wgi * CW, tm_dp = tm_s + BKV;
       const bool full = kv0 + BKV <= T;  // only the last key tile needs the column mask
       uint32_t rs[CW], rp[CW];
-      if constexpr (CW == 32) { tmem_ld32(tm_s, rs); tmem_ld32(tm_dp, rp); }
-      else { tmem_ld16(tm_s, rs); tmem_ld16(tm_dp, rp); }
+      tmem_ld32(tm_s, rs);
+      tmem_ld32(tm_dp, rp);
       tmem_wait_ld();
 #pragma unroll
       for (int c = 0; c < CW; c += 16) {
@@ -648,7 +590,7 @@ attn_bwd_q2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
 #pragma unroll
           for (int e = 0; e < 16; e += 2) {
             const uint64_t x = fma2(pack2(__uint_as_float(rs[c + e]), __uint_as_float(rs[c + e + 1])), sc2, nl2);
-            const uint64_t p2 = ex2_pair<POLY>(x, (c + e) / 2);
+            const uint64_t p2 = ex2_pair(x);
             const uint64_t t2 = add2(pack2(__uint_as_float(rp[c + e]), __uint_as_float(rp[c + e + 1])), nd2);
             dk[e / 2] = pack_bf16x2_pair(mul2(p2, t2));
           }
@@ -675,8 +617,8 @@ attn_bwd_q2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
     mbar_wait(acc_done, 0);
     tc_fence_after();
     __nv_bfloat16* dq_row = dqkv + ((size_t)b * T + q) * (3 * C) + h * HS;
-    // the head's columns are drained in 16-column groups by as many warpgroups as there are groups (at most 2 * NP)
-    constexpr int NG = (HS / 16) < 2 * NP ? (HS / 16) : 2 * NP;
+    // the head's columns are drained in 16-column groups by as many warpgroups as there are groups (at most 2)
+    constexpr int NG = (HS / 16) < 2 ? (HS / 16) : 2;
     constexpr int CH = HS / NG;
     const int g = wgi;
     if (g < NG) {
@@ -695,51 +637,44 @@ attn_bwd_q2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constan
 }
 
 // =============================================================================================== forward (v3 schedule)
-// Same roles as attn_fwd2_kernel, but S and P are double-buffered PER warpgroup so the softmax warps never
-// wait for the tensor pipe: S_w(j+2) is issued as soon as softmax_w(j) has drained its S buffer, and
-// softmax_w(j+1) may write its P tile while P.V_w(j) is still reading the other one.  K and V ride in
-// separate TMA rings because K(j+2) is consumed two iterations ahead of V(j).  BKV = 64.
-// NWG = softmax warpgroups (128 query rows each) per CTA.  NWG = 2: one CTA per SM, the two warpgroups share every K/V
-// tile.  NWG = 1: a CTA is half as big in every resource (192 threads, 256 TMEM columns, <= 113 KB of shared memory), TWO
-// of them share an SM: the same MUFU / tensor-pipe mix per SM, but the grid is scheduled in 128-row units, which matters
-// when the 256-row grid does not fill the 148 SMs evenly (T = 962, 48 heads: 192 CTAs = 2 rounds at 65 %; 384 half-size
-// CTAs on 296 slots = 1.3 rounds).
-template <int HS, int KST, int VST, int NWG = 2, bool PT = false>
+// One softmax warpgroup owns the CTA's 128 query rows.  S and P are double-buffered so the softmax warps never wait for the
+// tensor pipe: S(j+2) is issued as soon as softmax(j) has drained its S buffer, and softmax(j+1) may write its P tile while
+// P.V(j) is still reading the other one.  K and V ride in separate TMA rings because K(j+2) is consumed two iterations ahead
+// of V(j).  BKV = 64.  A CTA needs 192 threads, 256 TMEM columns and <= 113 KB of shared memory, so TWO of them share an SM
+// (see attn_fwd_run for the measured alternative).
+// The bf16 probabilities never touch shared memory: the softmax warps write them back (packed two per column) over the S tile
+// they came from and P.V runs with its A operand in tensor memory (tcgen05.mma [d], [a], b-desc).
+// POLY: every POLY-th pair of probabilities of a full, dropout-free tile is exponentiated by ex2_poly2 instead of MUFU.EX2
+// (see attn_fwd_run for the measurements).
+template <int HS, int KST, int VST>
 struct Fwd3 {
   static constexpr int BKV = 64;
-  static constexpr int Q_BYTES = 128 * HS * 2, KV_BYTES = BKV * HS * 2, P_BYTES = 128 * BKV * 2;
-  static constexpr int Q_OFF = 0, K_OFF = NWG * Q_BYTES, V_OFF = K_OFF + KST * KV_BYTES, P_OFF = V_OFF + VST * KV_BYTES;
-  static constexpr int BAR_OFF = P_OFF + (PT ? 0 : 2 * NWG * P_BYTES);  // P tiles live in tensor memory when PT
+  static constexpr int POLY = HS >= 128 ? 4 : 3;
+  static constexpr int Q_BYTES = 128 * HS * 2, KV_BYTES = BKV * HS * 2;
+  static constexpr int Q_OFF = 0, K_OFF = Q_BYTES, V_OFF = K_OFF + KST * KV_BYTES, BAR_OFF = V_OFF + VST * KV_BYTES;
   static constexpr int NBAR = 1 + 2 * KST + 2 * VST + 12;
   static constexpr int DYN = BAR_OFF + NBAR * 8 + 16 + 1024;
-  static constexpr int THREADS = 128 * NWG + 64;
-  static constexpr int MIN_CTAS = NWG == 1 ? 2 : 1;
-  static constexpr uint32_t TMEM_COLS = NWG == 1 ? 256 : 512;
-  static_assert(2 * NWG * BKV + NWG * HS <= (int)TMEM_COLS, "TMEM budget");
-  static_assert(DYN <= 232448 / MIN_CTAS - 1024 * (MIN_CTAS - 1), "shared memory budget");
+  static constexpr int THREADS = 128 + 64;
+  static constexpr uint32_t TMEM_COLS = 256;
+  static_assert(2 * BKV + HS <= (int)TMEM_COLS, "TMEM budget");
+  static_assert(DYN <= 232448 / 2 - 1024, "shared memory budget of two CTAs per SM");
 };
 
-// PT = true: the bf16 probabilities never touch shared memory — the softmax warps write them back (packed two per column)
-// over the S tile they came from and P.V runs with its A operand in tensor memory (tcgen05.mma [d], [a], b-desc).
-// PP = true (experiment, DSF_ATTN_PINGPONG=1): the two softmax warpgroups take turns in the exponential phase (named
-// barriers 3 / 4) so that one warpgroup's MUFU.EX2 work runs under the other's max / rescale bookkeeping.
-// POLY > 0: every POLY-th pair of probabilities of a full, dropout-free tile is exponentiated by ex2_poly2 instead of MUFU.EX2.
-template <int HS, int KST, int VST, bool PT, bool PP, int NWG = 2, int POLY = 0>
-__global__ void __launch_bounds__(128 * NWG + 64, NWG == 1 ? 2 : 1)
+template <int HS, int KST, int VST>
+__global__ void __launch_bounds__(128 + 64, 2)
 attn_fwd3_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmKV, __nv_bfloat16* __restrict__ y,
                  float* __restrict__ lse, int T, int C, int nh, float scale_log2, AttnDrop ad) {
-  using L = Fwd3<HS, KST, VST, NWG, PT>;
-  constexpr int BKV = L::BKV;
-  constexpr int MMAW = 4 * NWG, TMAW = 4 * NWG + 1;  // warp roles: 0 .. 4*NWG-1 softmax, then MMA issuer, TMA producer
-  static_assert(!PP || NWG == 2, "ping-pong needs two warpgroups");
+  using L = Fwd3<HS, KST, VST>;
+  constexpr int BKV = L::BKV, POLY = L::POLY;
+  constexpr int MMAW = 4, TMAW = 5;  // warp roles: 0 .. 3 softmax, then MMA issuer, TMA producer
   extern __shared__ uint8_t smem_raw[];
   const uint32_t sbase = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  uint8_t* smem = smem_raw + (sbase - smem_u32(smem_raw));
   const uint32_t bar0 = sbase + L::BAR_OFF;
+  // s_full / p_full / p_empty: two barriers (one per buffer) in 32-byte slots
   const uint32_t q_full = bar0, k_full = bar0 + 8, k_empty = k_full + 8 * KST, v_full = k_empty + 8 * KST, v_empty = v_full + 8 * VST,
                  s_full = v_empty + 8 * VST, p_full = s_full + 32, p_empty = p_full + 32, tmem_slot = p_empty + 32;
   const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0), lane = threadIdx.x & 31;  // warp-uniform for the compiler
-  const int q0 = blockIdx.x * (128 * NWG), h = blockIdx.y, b = blockIdx.z;
+  const int q0 = blockIdx.x * 128, h = blockIdx.y, b = blockIdx.z;
   const int n_kv = (T + BKV - 1) / BKV;
 
   pdl_trigger();
@@ -747,7 +682,7 @@ attn_fwd3_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
     mbar_init(q_full, 1);
     for (int s = 0; s < KST; ++s) { mbar_init(k_full + 8 * s, 1); mbar_init(k_empty + 8 * s, 1); }
     for (int s = 0; s < VST; ++s) { mbar_init(v_full + 8 * s, 1); mbar_init(v_empty + 8 * s, 1); }
-    for (int i = 0; i < 2 * NWG; ++i) { mbar_init(s_full + 8 * i, 1); mbar_init(p_full + 8 * i, 128); mbar_init(p_empty + 8 * i, 1); }
+    for (int i = 0; i < 2; ++i) { mbar_init(s_full + 8 * i, 1); mbar_init(p_full + 8 * i, 128); mbar_init(p_empty + 8 * i, 1); }
     fence_barrier_init();
   }
   if (warp == MMAW) { tmem_alloc(tmem_slot, L::TMEM_COLS); tmem_relinquish(); }
@@ -766,8 +701,8 @@ attn_fwd3_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
 
   if (warp == TMAW) {
     if (lane == 0) {
-      mbar_expect_tx(q_full, NWG * L::Q_BYTES);
-      for (int w = 0; w < NWG; ++w) tma_tile<HS>(sbase + L::Q_OFF + w * L::Q_BYTES, &tmQ, q_full, h * HS, q0 + 128 * w, b, 128);
+      mbar_expect_tx(q_full, L::Q_BYTES);
+      tma_tile<HS>(sbase + L::Q_OFF, &tmQ, q_full, h * HS, q0, b, 128);
       for (int j = 0; j < n_kv; ++j) {
         const int ks = j % KST, vs = j % VST;
         if (j >= KST) mbar_wait(k_empty + 8 * ks, ((j / KST) - 1) & 1);
@@ -786,51 +721,42 @@ attn_fwd3_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
       for (int jj = 0; jj < 2 && jj < n_kv; ++jj) {
         mbar_wait(k_full + 8 * (jj % KST), (jj / KST) & 1);
         tc_fence_after();
-        for (int w = 0; w < NWG; ++w) {
-          mma_over_head<HS>(tmem_base + (w * 2 + jj) * BKV, sbase + L::Q_OFF + w * L::Q_BYTES, 128, sbase + L::K_OFF + (jj % KST) * L::KV_BYTES,
-                            BKV, idesc_s);
-          tc_commit_elect(s_full + 8 * (w * 2 + jj));
-        }
+        mma_over_head<HS>(tmem_base + jj * BKV, sbase + L::Q_OFF, 128, sbase + L::K_OFF + (jj % KST) * L::KV_BYTES, BKV, idesc_s);
+        tc_commit_elect(s_full + 8 * jj);
         tc_commit_elect(k_empty + 8 * (jj % KST));
       }
       for (int j = 0; j < n_kv; ++j) {
         const int buf = j & 1, vs = j % VST;
         TRACE(2, j, 0);
         mbar_wait(v_full + 8 * vs, (j / VST) & 1);
-        for (int w = 0; w < NWG; ++w) {
-          const int sb = w * 2 + buf;
-          TRACE(2, j, 1 + 2 * w);
-          mbar_wait(p_full + 8 * sb, (j >> 1) & 1);
-          TRACE(2, j, 2 + 2 * w);
+        TRACE(2, j, 1);
+        mbar_wait(p_full + 8 * buf, (j >> 1) & 1);
+        TRACE(2, j, 2);
+        tc_fence_after();
+        mma_over_rows_ts<HS, BKV>(tmem_base + 2 * BKV, tmem_base + buf * BKV, sbase + L::V_OFF + vs * L::KV_BYTES, idesc_o, j > 0);
+        tc_commit_elect(p_empty + 8 * buf);
+        tc_commit_elect(v_empty + 8 * vs);
+        if (j + 2 < n_kv) {
+          const int ks = (j + 2) % KST;
+          mbar_wait(k_full + 8 * ks, ((j + 2) / KST) & 1);
           tc_fence_after();
-          if (PT)
-            mma_over_rows_ts<HS, BKV>(tmem_base + 2 * NWG * BKV + w * HS, tmem_base + sb * BKV, sbase + L::V_OFF + vs * L::KV_BYTES, idesc_o, j > 0);
-          else
-            mma_over_rows<HS, BKV>(tmem_base + 2 * NWG * BKV + w * HS, sbase + L::P_OFF + sb * L::P_BYTES, sbase + L::V_OFF + vs * L::KV_BYTES, idesc_o,
-                                   j > 0);
-          tc_commit_elect(p_empty + 8 * sb);
-          if (w == NWG - 1) tc_commit_elect(v_empty + 8 * vs);
-          if (j + 2 < n_kv) {
-            const int ks = (j + 2) % KST;
-            if (w == 0) { mbar_wait(k_full + 8 * ks, ((j + 2) / KST) & 1); tc_fence_after(); }
-            mma_over_head<HS>(tmem_base + sb * BKV, sbase + L::Q_OFF + w * L::Q_BYTES, 128, sbase + L::K_OFF + ks * L::KV_BYTES, BKV, idesc_s);
-            tc_commit_elect(s_full + 8 * sb);
-            if (w == NWG - 1) tc_commit_elect(k_empty + 8 * ks);
-          }
+          mma_over_head<HS>(tmem_base + buf * BKV, sbase + L::Q_OFF, 128, sbase + L::K_OFF + ks * L::KV_BYTES, BKV, idesc_s);
+          tc_commit_elect(s_full + 8 * buf);
+          tc_commit_elect(k_empty + 8 * ks);
         }
       }
     }
   } else {
+    // w = warp >> 2 is 0 for every softmax warp, but the compiler cannot tell: the terms in w keep the instructions this kernel
+    // was measured with
     const int w = warp >> 2;
     const int row = (warp & 3) * 32 + lane;
     const uint32_t lane_off = (uint32_t)((warp & 3) * 32) << 16;
-    const uint32_t tm_o = tmem_base + 2 * NWG * BKV + w * HS + lane_off;
+    const uint32_t tm_o = tmem_base + 2 * BKV + w * HS + lane_off;
     float m_run = -INFINITY, l_run = 0.f;
-    if (PP && w == 1) named_bar_arrive(3, 256);  // warpgroup 0 goes first
     for (int j = 0; j < n_kv; ++j) {
       const int kv0 = j * BKV, buf = j & 1, sb = w * 2 + buf;
       const uint32_t tm_s = tmem_base + sb * BKV + lane_off;
-      uint8_t* p_tile = smem + L::P_OFF + sb * L::P_BYTES;
       if ((warp & 3) == 0) TRACE(w, j, 0);
       mbar_wait(s_full + 8 * sb, (j >> 1) & 1);
       if ((warp & 3) == 0) TRACE(w, j, 1);
@@ -880,16 +806,13 @@ attn_fwd3_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
         m_run = m_new;
       }
       if ((warp & 3) == 0) TRACE(w, j, 3);
-      // P in shared memory: wait until P.V(j-2) has retired its buffer.  P in tensor memory (PT): the buffer is the S tile itself,
-      // and s_full(j) already implies it — S(j) was issued after P.V(j-2) by the same thread, whose MMAs complete in order.
-      if (!PT && j >= 2) mbar_wait(p_empty + 8 * sb, ((j >> 1) - 1) & 1);
-      if (PP) named_bar_sync(3 + w, 256);  // my turn on the exponential unit
-      if ((warp & 3) == 0) TRACE(w, j, 4);
+      // the P buffer is the S tile itself, and s_full(j) already says it is free: S(j) was issued after P.V(j-2) by the same
+      // thread, whose MMAs complete in order
       float l_add = 0.f;
       const bool full = kv0 + BKV <= T;
       const int qrow = q0 + 128 * w + row;
       const uint64_t rowid = ((uint64_t)b * nh + h) * T + qrow;
-      if (POLY > 0 && PT && full && !ad.thresh8) {
+      if (full && !ad.thresh8) {
         // packed fast path: x = s * scale - m as FFMA2, the row sum as FADD2, every POLY-th pair off the MUFU pipe
         const uint64_t sc2 = pack2(scale_log2, scale_log2), nm2 = pack2(-m_run, -m_run);
         uint64_t lsum = pack2(0.f, 0.f);
@@ -901,7 +824,7 @@ attn_fwd3_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
             const uint32_t a0 = half ? r1[i] : r0[i], a1 = half ? r1[i + 1] : r0[i + 1];
             const uint64_t x = fma2(pack2(__uint_as_float(a0), __uint_as_float(a1)), sc2, nm2);
             float p0, p1;
-            if (((i / 2) % (POLY > 0 ? POLY : 1)) == POLY - 1) {
+            if ((i / 2) % POLY == POLY - 1) {
               ex2_poly2(x, p0, p1);
             } else {
               float x0, x1;
@@ -942,13 +865,10 @@ attn_fwd3_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
           }
           pk[i / 2] = pack_bf16x2(p0, p1);
         }
-        if (PT) tmem_st16(tm_s + half * 16, pk);  // keys 32*half .. +31 -> packed columns 16*half .. +15 of the S tile
-        else store_p32<BKV>(p_tile, row, half * 32, pk);
+        tmem_st16(tm_s + half * 16, pk);  // keys 32*half .. +31 -> packed columns 16*half .. +15 of the S tile
       }
-      if (PP) named_bar_arrive(4 - w, 256);  // hand the exponential unit to the other warpgroup
       l_run += l_add;
-      if (PT) tmem_wait_st();
-      else fence_proxy_async();
+      tmem_wait_st();
       tc_fence_before();
       mbar_arrive(p_full + 8 * sb);
       if ((warp & 3) == 0) TRACE(w, j, 5);
@@ -1002,20 +922,14 @@ static int make_tmap3(CUtensorMap* m, const void* base, int ncols, int T, int B,
   return DSF_OK;
 }
 
-// Exponentials of the forward kernel moved from MUFU.EX2 to the FMA pipe (ex2_poly2): every 3rd pair at head sizes <= 64, every 4th
-// at 128.  Measured on B200 (scripts/bench_attn_parts.py, batch 12, T = 962; profiles/r02ah_attn_exp_poly.txt), none / every 4th / 3rd /
-// 2nd pair: hs 16: 28.1 / 25.2 / 24.4 / 25.3 us, hs 32: 28.6 / 25.5 / 24.8 / 25.5, hs 64: 30.3 / 27.0 / 27.1 / 27.8, hs 128: 35.4 / 34.8 /
-// 35.7 / 35.1 us; T = 3842, hs 128: 64.9 / 55.0 / 56.0 / 57.4 us (932 -> 1099 TF/s).  DSF_ATTN_EXP_POLY=0 keeps every exponential on MUFU.
-static const bool g_attn_exp_poly = getenv("DSF_ATTN_EXP_POLY") ? atoi(getenv("DSF_ATTN_EXP_POLY")) != 0 : true;
-
-template <int HS, int KST, int VST, int NWG, int POLY>
-static int launch_fwd3p(const void* qkv, void* y, float* lse, int B, int T, int C, int nh, const AttnDrop& ad, cudaStream_t st) {
-  using L = Fwd3<HS, KST, VST, NWG, true>;
+template <int HS, int KST, int VST>
+static int launch_fwd3(const void* qkv, void* y, float* lse, int B, int T, int C, int nh, const AttnDrop& ad, cudaStream_t st) {
+  using L = Fwd3<HS, KST, VST>;
   using H = HeadCfg<HS>;
   static bool configured_on[64] = {};
   bool& configured = per_device_flag(configured_on);
   if (!configured) {
-    if (cudaFuncSetAttribute(attn_fwd3_kernel<HS, KST, VST, true, false, NWG, POLY>, cudaFuncAttributeMaxDynamicSharedMemorySize, L::DYN) != cudaSuccess)
+    if (cudaFuncSetAttribute(attn_fwd3_kernel<HS, KST, VST>, cudaFuncAttributeMaxDynamicSharedMemorySize, L::DYN) != cudaSuccess)
       return check_launch("attn_fwd3/attr");
     configured = true;
   }
@@ -1023,68 +937,56 @@ static int launch_fwd3p(const void* qkv, void* y, float* lse, int B, int T, int 
   if (int e = make_tmap3(&tmQ, qkv, 3 * C, T, B, H::BOXC, 128)) return e;
   if (int e = make_tmap3(&tmKV, qkv, 3 * C, T, B, H::BOXC, L::BKV)) return e;
   const float scale_log2 = (1.0f / sqrtf((float)HS)) * 1.4426950408889634f;
-  dim3 grid(cdiv(T, 128 * NWG), nh, B);
-  launch_pdl(attn_fwd3_kernel<HS, KST, VST, true, false, NWG, POLY>, grid, dim3(L::THREADS), L::DYN, st, tmQ, tmKV, (__nv_bfloat16*)y, lse, T, C, nh,
-             scale_log2, ad);
+  dim3 grid(cdiv(T, 128), nh, B);
+  launch_pdl(attn_fwd3_kernel<HS, KST, VST>, grid, dim3(L::THREADS), L::DYN, st, tmQ, tmKV, (__nv_bfloat16*)y, lse, T, C, nh, scale_log2, ad);
   return check_launch("attn_fwd3");
-}
-
-template <int HS, int KST, int VST, int NWG>
-static int launch_fwd3(const void* qkv, void* y, float* lse, int B, int T, int C, int nh, const AttnDrop& ad, cudaStream_t st) {
-  if constexpr (NWG == 1) {  // the default 128-row CTAs
-    if (g_attn_exp_poly) return launch_fwd3p<HS, KST, VST, NWG, (HS >= 128 ? 4 : 3)>(qkv, y, lse, B, T, C, nh, ad, st);
-  }
-  return launch_fwd3p<HS, KST, VST, NWG, 0>(qkv, y, lse, B, T, C, nh, ad, st);
 }
 
 int run_attn_delta(const void* y, const void* dy, float* delta, int B, int T, int C, int nh, cudaStream_t st);  // attn_api.cu
 
-// Q / dO rows of the dQ kernel parked in tensor memory as TS-mode A operands (default on: +-0 at T = 962, +6 % at T = 3842)
-static const bool g_attn_a_in_tmem = getenv("DSF_ATTN_A_TMEM") ? atoi(getenv("DSF_ATTN_A_TMEM")) != 0 : true;
-// Math warpgroup pairs of the two backward kernels (template parameter NP, see attn_bwd_kv2_kernel).  Only NP = 1 is built.  Measured on
-// B200 (scripts/bench_attn_parts.py, batch 12, T = 962, head size 16 / 32 / 64 / 128; profiles/r02aj_attn_pairs.txt): four warpgroups
-// sharing every tile (NP = 2) run the dK/dV kernel in 29.1 / 31.9 / 42.0 / 59.7 us against 28.7 / 31.7 / 41.2 / 59.3 us and the dQ kernel
-// in 25.3 / 27.8 / 33.0 / 44.8 against 25.9 / 27.7 / 32.1 / 44.6 us.  The in-kernel timeline (profiles/r02aj_attn_trace.txt) says why:
-// halving a warp's columns shortens its tile from ~740 to ~670 cycles only — the tile is a fixed latency chain (tcgen05.ld, wait::ld,
-// tcgen05.st, wait::st, fence, mbarrier), not arithmetic.  An earlier variant whose two pairs took alternate tiles (git history) lost
-// to NP = 1 as well: with two S^T/dP^T buffers the next tile of a pair cannot be issued before its previous one is consumed.
-constexpr int kBwdPairs = 1;
-// The backward kernels keep every exponential on MUFU.EX2 (template parameter POLY = 0): they run 32 exponentials per thread and tile
-// against the forward's 64 and are bound by the per-tile latency chain, not by the MUFU pipe — with every 3rd pair on the FMA pipe the
-// dK/dV kernel measured 30.2 / 32.7 / 41.9 / 62.9 us against 28.4 / 31.6 / 41.4 / 60.3 us (head size 16 / 32 / 64 / 128, batch 12,
-// T = 962; profiles/r02ai_attn_bwd_poly.txt).  The packed-pair arithmetic (FFMA2 / FADD2 / FMUL2) stays: -1.3 / -1.8 us at 16 / 32.
-
-template <int HS, int BQ, int STA, int NP, bool DROP, int POLY>
+// Backward kernels: measured variants that were removed (scripts/bench_attn_parts.py, B200, batch 12, T = 962, head size
+// 16 / 32 / 64 / 128):
+// * Four math warpgroups sharing every tile instead of two (profiles/r02aj_attn_pairs.txt): dK/dV 29.1 / 31.9 / 42.0 / 59.7 us
+//   against 28.7 / 31.7 / 41.2 / 59.3 us, dQ 25.3 / 27.8 / 33.0 / 44.8 against 25.9 / 27.7 / 32.1 / 44.6 us.  The in-kernel timeline
+//   (profiles/r02aj_attn_trace.txt) says why: halving a warp's columns shortens its tile from ~740 to ~670 cycles only — the tile
+//   is a fixed latency chain (tcgen05.ld, wait::ld, tcgen05.st, wait::st, fence, mbarrier), not arithmetic.  An earlier variant
+//   whose two pairs of warpgroups took alternate tiles (git history) lost as well: with two S^T/dP^T buffers the next tile of a
+//   pair cannot be issued before its previous one is consumed.
+// * Every 3rd pair of exponentials on the FMA pipe, as in the forward (profiles/r02ai_attn_bwd_poly.txt): dK/dV 30.2 / 32.7 / 41.9 /
+//   62.9 us against 28.4 / 31.6 / 41.4 / 60.3 us.  They run 32 exponentials per thread and tile against the forward's 64 and are
+//   bound by the per-tile latency chain, not by the MUFU pipe, so every exponential stays on MUFU.EX2.  The packed-pair arithmetic
+//   (FFMA2 / FADD2 / FMUL2) stays: -1.3 / -1.8 us at head size 16 / 32.
+template <int HS, int BQ, int STA, bool DROP>
 static int launch_bwd_kv(const CUtensorMap& tmKV128, const CUtensorMap& tmQs, const CUtensorMap& tmDOs, const float* lse, const float* delta, void* dqkv,
                          dim3 grid, int T, int C, int nh, float scale, const AttnDrop& ad, cudaStream_t st) {
-  using LA = BwdKV2<HS, BQ, STA, NP>;
+  using LA = BwdKV2<HS, BQ, STA>;
   const int dyn = LA::dyn_bytes(T);
   if (dyn > 232448) { set_error("attn_bwd: T = %d needs %d bytes of shared memory for the per-query statistics (limit 232448)", T, dyn); return DSF_EUNSUPPORTED; }
   static bool configured_on[64] = {};
   bool& configured = per_device_flag(configured_on);
   if (!configured) {
-    if (cudaFuncSetAttribute(attn_bwd_kv2_kernel<HS, BQ, STA, NP, DROP, POLY>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448) != cudaSuccess)
+    if (cudaFuncSetAttribute(attn_bwd_kv2_kernel<HS, BQ, STA, DROP>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448) != cudaSuccess)
       return check_launch("attn_bwd2/kv/attr");
     configured = true;
   }
-  launch_pdl(attn_bwd_kv2_kernel<HS, BQ, STA, NP, DROP, POLY>, grid, dim3(LA::THREADS), dyn, st, tmKV128, tmQs, tmDOs, lse, delta, (__nv_bfloat16*)dqkv, T, C,
-             nh, scale, ad);
+  launch_pdl(attn_bwd_kv2_kernel<HS, BQ, STA, DROP>, grid, dim3(LA::THREADS), dyn, st, tmKV128, tmQs, tmDOs, lse, delta, (__nv_bfloat16*)dqkv, T, C, nh,
+             scale, ad);
   return check_launch("attn_bwd2/kv");
 }
 
-template <int HS, int STB, bool AT, int NP, bool DROP, int POLY>
+template <int HS, int STB, bool DROP>
 static int launch_bwd_q(const CUtensorMap& tmQ128, const CUtensorMap& tmDO128, const CUtensorMap& tmKV64, const float* lse, const float* delta, void* dqkv,
                         dim3 grid, int T, int C, int nh, float scale, const AttnDrop& ad, const void* qkv, const void* dy, cudaStream_t st) {
   using LB = BwdQ2<HS, STB>;
   static bool configured_on[64] = {};
   bool& configured = per_device_flag(configured_on);
   if (!configured) {
-    if (cudaFuncSetAttribute(attn_bwd_q2_kernel<HS, STB, AT, NP, DROP, POLY>, cudaFuncAttributeMaxDynamicSharedMemorySize, LB::DYN) != cudaSuccess)
+    if (cudaFuncSetAttribute(attn_bwd_q2_kernel<HS, STB, DROP>, cudaFuncAttributeMaxDynamicSharedMemorySize, LB::DYN) != cudaSuccess)
       return check_launch("attn_bwd2/q/attr");
     configured = true;
   }
-  launch_pdl(attn_bwd_q2_kernel<HS, STB, AT, NP, DROP, POLY>, grid, dim3(256 * NP + 64), LB::DYN, st, tmQ128, tmDO128, tmKV64, lse, delta, (__nv_bfloat16*)dqkv, T,
-             C, nh, scale, ad, (const __nv_bfloat16*)qkv, (const __nv_bfloat16*)dy);
+  launch_pdl(attn_bwd_q2_kernel<HS, STB, DROP>, grid, dim3(256 + 64), LB::DYN, st, tmQ128, tmDO128, tmKV64, lse, delta, (__nv_bfloat16*)dqkv, T, C, nh,
+             scale, ad, (const __nv_bfloat16*)qkv, (const __nv_bfloat16*)dy);
   return check_launch("attn_bwd2/q");
 }
 
@@ -1103,20 +1005,17 @@ static int launch_bwd2(const void* qkv, const void* y, const void* dy, const flo
     if (int e = make_tmap3(&tmKV128, qkv, 3 * C, T, B, H::BOXC, 128)) return e;
     if (int e = make_tmap3(&tmQs, qkv, 3 * C, T, B, H::BOXC, BQ)) return e;
     if (int e = make_tmap3(&tmDOs, dy, C, T, B, H::BOXC, BQ)) return e;
-#define DSF_KV(DROP) launch_bwd_kv<HS, BQ, STA, kBwdPairs, DROP, 0>(tmKV128, tmQs, tmDOs, lse, (const float*)delta, dqkv, grid, T, C, nh, scale, ad, st)
-    if (int e = drop ? DSF_KV(true) : DSF_KV(false)) return e;
-#undef DSF_KV
+    const int e = drop ? launch_bwd_kv<HS, BQ, STA, true>(tmKV128, tmQs, tmDOs, lse, delta, dqkv, grid, T, C, nh, scale, ad, st)
+                       : launch_bwd_kv<HS, BQ, STA, false>(tmKV128, tmQs, tmDOs, lse, delta, dqkv, grid, T, C, nh, scale, ad, st);
+    if (e) return e;
   }
   if (parts & 4) {
     CUtensorMap tmQ128, tmDO128, tmKV64;
     if (int e = make_tmap3(&tmQ128, qkv, 3 * C, T, B, H::BOXC, 128)) return e;
     if (int e = make_tmap3(&tmDO128, dy, C, T, B, H::BOXC, 128)) return e;
     if (int e = make_tmap3(&tmKV64, qkv, 3 * C, T, B, H::BOXC, 64)) return e;
-#define DSF_Q(AT, DROP) launch_bwd_q<HS, STB, AT, kBwdPairs, DROP, 0>(tmQ128, tmDO128, tmKV64, lse, (const float*)delta, dqkv, grid, T, C, nh, scale, ad, qkv, dy, st)
-    int e;
-    if (g_attn_a_in_tmem) e = drop ? DSF_Q(true, true) : DSF_Q(true, false);
-    else e = drop ? DSF_Q(false, true) : DSF_Q(false, false);
-#undef DSF_Q
+    const int e = drop ? launch_bwd_q<HS, STB, true>(tmQ128, tmDO128, tmKV64, lse, delta, dqkv, grid, T, C, nh, scale, ad, qkv, dy, st)
+                       : launch_bwd_q<HS, STB, false>(tmQ128, tmDO128, tmKV64, lse, delta, dqkv, grid, T, C, nh, scale, ad, qkv, dy, st);
     if (e) return e;
   }
   return DSF_OK;
@@ -1124,7 +1023,7 @@ static int launch_bwd2(const void* qkv, const void* y, const void* dy, const flo
 
 #ifdef DSF_ATTN_TRACE
 }  // namespace dsf
-extern "C" int dsf_debug_attn_trace(long long* host_out) {  // 3 x 64 x 6 clock64 stamps of the last forward launch
+extern "C" int dsf_debug_attn_trace(long long* host_out) {  // 3 x 64 x 6 clock64 stamps of the last traced launch
   return cudaMemcpyFromSymbol(host_out, dsf::g_attn_trace, sizeof(dsf::g_attn_trace)) == cudaSuccess ? 0 : 2;
 }
 namespace dsf {
@@ -1146,27 +1045,23 @@ static AttnDrop make_attn_drop(const dsf_dropout* d, uint32_t* bits, int T) {
   return a;
 }
 
-// Forward CTA shape (see Fwd3): force_nwg 0 / 1 = 128-row CTAs, two per SM (default); 2 = 256-row CTAs, one per SM.  Measured on
-// B200 (scripts/bench_kernels.py attnq, batch 12, T = 962): 42 vs 48 us at hs = 128, 36 vs 43 (hs = 64), 34 vs 41 (hs = 32), 33 vs
-// 40 us (hs = 16); T = 3842, batch 2, hs = 128: 68 vs 80 us (891 vs 760 TF/s) — the half-size CTAs win even where the 256-row
-// grid fills the SMs in one round: two independent MMA / TMA / softmax pipelines per SM overlap better than one pipeline with
-// two softmax warpgroups, and the grid is scheduled in finer units.
-int attn_fwd_run(const void* qkv, void* y, float* lse, int B, int T, int C, int nh, const dsf_dropout* drop, uint32_t* bits, int force_nwg,
-                 cudaStream_t st) {
+// Forward, measured variants that were removed:
+// * CTA shape: 128-row CTAs, two per SM, against 256-row CTAs (two softmax warpgroups sharing every K/V tile), one per SM.  On
+//   B200 (scripts/bench_kernels.py attnq, batch 12, T = 962): 42 vs 48 us at hs = 128, 36 vs 43 (hs = 64), 34 vs 41 (hs = 32), 33
+//   vs 40 us (hs = 16); T = 3842, batch 2, hs = 128: 68 vs 80 us (891 vs 760 TF/s) — the half-size CTAs win even where the 256-row
+//   grid fills the SMs in one round: two independent MMA / TMA / softmax pipelines per SM overlap better than one pipeline with
+//   two softmax warpgroups, and the grid is scheduled in finer units.
+// * Exponentials (Fwd3::POLY): moving every 3rd pair from MUFU.EX2 to the FMA pipe (ex2_poly2) at head sizes <= 64 and every 4th at
+//   128 is kept.  On B200 (scripts/bench_attn_parts.py, batch 12, T = 962; profiles/r02ah_attn_exp_poly.txt), none / every 4th /
+//   3rd / 2nd pair: hs 16: 28.1 / 25.2 / 24.4 / 25.3 us, hs 32: 28.6 / 25.5 / 24.8 / 25.5, hs 64: 30.3 / 27.0 / 27.1 / 27.8, hs 128:
+//   35.4 / 34.8 / 35.7 / 35.1 us; T = 3842, hs 128: 64.9 / 55.0 / 56.0 / 57.4 us (932 -> 1099 TF/s).
+int attn_fwd_run(const void* qkv, void* y, float* lse, int B, int T, int C, int nh, const dsf_dropout* drop, uint32_t* bits, cudaStream_t st) {
   const AttnDrop ad = make_attn_drop(drop, bits, T);
-  if (force_nwg != 2) {
-    switch (C / nh) {
-      case 16: return launch_fwd3<16, 3, 2, 1>(qkv, y, lse, B, T, C, nh, ad, st);
-      case 32: return launch_fwd3<32, 3, 2, 1>(qkv, y, lse, B, T, C, nh, ad, st);
-      case 64: return launch_fwd3<64, 3, 2, 1>(qkv, y, lse, B, T, C, nh, ad, st);
-      case 128: return launch_fwd3<128, 2, 2, 1>(qkv, y, lse, B, T, C, nh, ad, st);
-    }
-  }
   switch (C / nh) {
-    case 16: return launch_fwd3<16, 3, 2, 2>(qkv, y, lse, B, T, C, nh, ad, st);
-    case 32: return launch_fwd3<32, 3, 2, 2>(qkv, y, lse, B, T, C, nh, ad, st);
-    case 64: return launch_fwd3<64, 3, 2, 2>(qkv, y, lse, B, T, C, nh, ad, st);
-    case 128: return launch_fwd3<128, 3, 2, 2>(qkv, y, lse, B, T, C, nh, ad, st);
+    case 16: return launch_fwd3<16, 3, 2>(qkv, y, lse, B, T, C, nh, ad, st);
+    case 32: return launch_fwd3<32, 3, 2>(qkv, y, lse, B, T, C, nh, ad, st);
+    case 64: return launch_fwd3<64, 3, 2>(qkv, y, lse, B, T, C, nh, ad, st);
+    case 128: return launch_fwd3<128, 2, 2>(qkv, y, lse, B, T, C, nh, ad, st);
   }
   set_error("attn_fwd: head size %d not supported (16, 32, 64, 128)", C / nh);
   return DSF_EUNSUPPORTED;

@@ -7,7 +7,6 @@
 // Warp roles (320 threads): warp 0 = TMA producer, warp 1 = TMEM allocator + MMA issuer, warps 2..9 = epilogue
 // (TMEM lane quarter = warp % 4, column half = (warp - 2) / 4).
 #include <algorithm>
-#include <cstdlib>
 
 #include "tc_common.cuh"
 
@@ -29,46 +28,8 @@ struct EpiArgs2 {
   int flags;
   int N;          // row length for the dropout element index m*N + n
   const __nv_bfloat16* relu_src;  // nullable: v = relu_src[m,n] > 0 ? v : 0 (ReLU backward fused into the dgrad GEMM)
-  int ablate;     // diagnostics (DSF_GEMM_ABLATE): 1 = skip the epilogue body, 2 = skip the TMA loads (results are garbage)
   DropArgs drop;  // resid_drop (model2_seq.py:109,125): after bias/ReLU, before the residual add
 };
-
-__device__ __forceinline__ void epi_store32(const EpiArgs2& e, int row, int n, const uint32_t (&r)[32]) {
-  float v[32];
-#pragma unroll
-  for (int j = 0; j < 32; ++j) v[j] = __uint_as_float(r[j]);
-  if (e.flags & DSF_EPI_BIAS) {
-#pragma unroll
-    for (int j = 0; j < 32; j += 4) {
-      const float4 b = __ldg(reinterpret_cast<const float4*>(e.bias + n + j));
-      v[j] += b.x; v[j + 1] += b.y; v[j + 2] += b.z; v[j + 3] += b.w;
-    }
-  }
-  if (e.flags & DSF_EPI_RELU) {
-#pragma unroll
-    for (int j = 0; j < 32; ++j) v[j] = fmaxf(v[j], 0.f);
-  }
-  const size_t off = (size_t)row * e.ldc + n;
-  if (e.flags & DSF_EPI_RESIDUAL) {
-    const float4* rp = reinterpret_cast<const float4*>(e.residual + off);
-#pragma unroll
-    for (int j = 0; j < 8; ++j) {
-      const float4 t = rp[j];
-      v[4 * j] += t.x; v[4 * j + 1] += t.y; v[4 * j + 2] += t.z; v[4 * j + 3] += t.w;
-    }
-  }
-  if (e.c_dtype == DSF_F32) {
-    float4* cp = reinterpret_cast<float4*>(reinterpret_cast<float*>(e.C) + off);
-#pragma unroll
-    for (int j = 0; j < 8; ++j) cp[j] = make_float4(v[4 * j], v[4 * j + 1], v[4 * j + 2], v[4 * j + 3]);
-  } else {
-    uint4* cp = reinterpret_cast<uint4*>(reinterpret_cast<__nv_bfloat16*>(e.C) + off);
-#pragma unroll
-    for (int j = 0; j < 4; ++j)
-      cp[j] = make_uint4(pack_bf16x2(v[8 * j], v[8 * j + 1]), pack_bf16x2(v[8 * j + 2], v[8 * j + 3]),
-                         pack_bf16x2(v[8 * j + 4], v[8 * j + 5]), pack_bf16x2(v[8 * j + 6], v[8 * j + 7]));
-  }
-}
 
 // epilogue math on 32 accumulator columns of one row: (+bias)(relu)(+residual); row_ok guards the residual read
 __device__ __forceinline__ void epi_math32(const EpiArgs2& e, int row, int n, const uint32_t (&r)[32], float (&v)[32], bool row_ok) {
@@ -169,7 +130,6 @@ gemm_nt2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
         for (int kb = 0; kb < num_k; ++kb, ++it) {
           const int s = it % STAGES;
           mbar_wait(bar_empty + s * 8, ((it / STAGES) & 1) ^ 1);
-          if (epi.ablate & 2) { mbar_arrive(bar_full + s * 8); continue; }
           mbar_expect_tx(bar_full + s * 8, L::STAGE_BYTES);
           const uint32_t sa = base + s * L::STAGE_BYTES, sb = sa + L::A_BYTES;
           tma_load_2d(sa, &tmA, bar_full + s * 8, kb * G2_BK, m0);
@@ -217,7 +177,7 @@ gemm_nt2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
       const int m0 = (tile % m_tiles) * G2_BM, n0 = (tile / m_tiles) * BN;
       mbar_wait(acc_full + ab * 8, (i >> 1) & 1);
       tc_fence_after();
-      if (ch >= NSPLIT || m0 + q * 32 >= M || (epi.ablate & 1)) {  // nothing to store for this warp
+      if (ch >= NSPLIT || m0 + q * 32 >= M) {  // nothing to store for this warp
         tc_fence_before();
         __syncwarp();
         if (lane == 0) mbar_arrive(acc_empty + ab * 8);
@@ -255,7 +215,6 @@ gemm_nt2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
             for (int j = 0; j < 16; ++j) w[hh * 16 + j] = pack_bf16x2(v[2 * j], v[2 * j + 1]);
           }
         }
-        if (!(epi.ablate & 8)) {
 #pragma unroll
         for (int j = 0; j < 8; ++j) {
           const uint32_t dst = sbuf + lane * 128 + ((j ^ (lane & 7)) << 4);
@@ -263,14 +222,8 @@ gemm_nt2_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
                        : "memory");
         }
         fence_proxy_async();
-        } else {
-          uint32_t acc = 0;
-#pragma unroll
-          for (int j = 0; j < 32; ++j) acc ^= w[j];
-          if (acc == 0x12345678u) asm volatile("st.shared.b32 [%0], %1;" ::"r"(sbuf), "r"(acc) : "memory");
-        }
         __syncwarp();
-        if (lane == 0 && !(epi.ablate & 4)) {
+        if (lane == 0) {
           tma_store_2d(&tmC, sbuf, ncol, m0 + q * 32);
           bulk_commit();
         }
@@ -371,7 +324,7 @@ template <int BN, int STAGES, bool RTMA = false>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(G2_THREADS, 1)
 gemm_nt3_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const __grid_constant__ CUtensorMap tmC,
                 const __grid_constant__ CUtensorMap tmBt, const __grid_constant__ CUtensorMap tmR, EpiArgs2 epi, int M, int N, int K,
-                int m_tiles, int n_tiles, int tail_start, int tail_split, int n_split) {
+                int m_tiles, int n_tiles, int tail_start, int n_split) {
   using L = G3Smem<BN, STAGES, RTMA>;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
@@ -381,33 +334,17 @@ gemm_nt3_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
   const uint32_t rank = cluster_ctarank();
   const int pair = blockIdx.x >> 1, n_pairs = gridDim.x >> 1;
   const int num_k = K / G2_BK;
-  // Work units: units < tail_start are whole 256 x BN tiles (unit = tile).  The tiles left over after the last full
-  // round of the pairs (tail_start .. ) are each split tail_split ways along K so that the last round is short: a split
-  // unit covers k-blocks [kb0, kb1) of its tile and ADDS its partial product to the fp32 output with vector reductions
-  // (the host zero-fills those tiles first; split 0 also adds bias / residual).  tail_split == 1: no splitting.
-  // n_split > 1 (needs tail_split == 1): the leftover tiles are instead split n_split ways along N — a unit is a
-  // 256 x (BN / n_split) sub-tile with its own, narrower MMA shape and B box (tmBt); nothing is reduced across units, so
-  // any epilogue works.  The short last round costs ~BN/n_split columns of epilogue and a cheaper MMA stream.
-  const int total = tail_start + (m_tiles * n_tiles - tail_start) * tail_split * n_split;
-  auto nsub_of = [&](int u, int& tile, int& n_off, int& width) {  // N-split view of unit u
+  // Work units: units < tail_start are whole 256 x BN tiles (unit = tile).  n_split > 1: the tiles left over after the
+  // last full round of the pairs (tail_start .. ) are each split n_split ways along N — a unit is a 256 x (BN / n_split)
+  // sub-tile with its own, narrower MMA shape and B box (tmBt); nothing is reduced across units, so any epilogue works.
+  // The short last round costs ~BN/n_split columns of epilogue and a cheaper MMA stream.
+  const int total = tail_start + (m_tiles * n_tiles - tail_start) * n_split;
+  auto unit_of = [&](int u, int& tile, int& n_off, int& width) {
     if (u < tail_start || n_split == 1) { tile = u; n_off = 0; width = BN; return; }
     const int j = u - tail_start;
     tile = tail_start + j / n_split;
     width = BN / n_split;
     n_off = (j % n_split) * width;
-  };
-  auto unit_of = [&](int u, int& tile, int& kb0, int& kb1, int& part) {
-    if (u < tail_start || tail_split == 1) {
-      int n_off, width;
-      nsub_of(u, tile, n_off, width);
-      kb0 = 0; kb1 = num_k; part = 0;
-      return;
-    }
-    const int j = u - tail_start, sp = j % tail_split;
-    tile = tail_start + j / tail_split;
-    kb0 = sp * num_k / tail_split;
-    kb1 = (sp + 1) * num_k / tail_split;
-    part = 1 + (sp == 0 ? 0 : 1);  // 1 = first split (carries bias / residual), 2 = the others
   };
   pdl_trigger();
 
@@ -434,18 +371,14 @@ gemm_nt3_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
       const uint32_t full0 = mapa_u32(bar_full, 0);  // the leader's full barriers
       int it = 0;
       for (int u = pair; u < total; u += n_pairs) {
-        int tile, kb0, kb1, part;
-        unit_of(u, tile, kb0, kb1, part);
-        int n_off, width;
-        if (n_split > 1) nsub_of(u, tile, n_off, width);
-        else { n_off = 0; width = BN; }
+        int tile, n_off, width;
+        unit_of(u, tile, n_off, width);
         const bool narrow = width != BN;
         const int m0 = (tile % m_tiles) * 256 + (int)rank * G2_BM, n0 = (tile / m_tiles) * BN + n_off + (int)rank * (width / 2);
         const uint32_t tx = 2u * (uint32_t)(L::A_BYTES + (width / 2) * G2_BK * 2);
-        for (int kb = kb0; kb < kb1; ++kb, ++it) {
+        for (int kb = 0; kb < num_k; ++kb, ++it) {
           const int s = it % STAGES;
           mbar_wait(bar_empty + s * 8, ((it / STAGES) & 1) ^ 1);
-          if (epi.ablate & 2) { if (rank == 0) mbar_arrive(bar_full + s * 8); continue; }
           if (rank == 0) mbar_expect_tx(bar_full + s * 8, tx);
           const uint32_t sa = base + s * L::STAGE_BYTES, sb = sa + L::A_BYTES;
           tma_load_2d_pair(sa, &tmA, full0 + s * 8, kb * G2_BK, m0);
@@ -457,24 +390,21 @@ gemm_nt3_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
     if (rank == 0) {  // MMA issuer of the pair: all 32 lanes walk the schedule, one elected lane issues
       int it = 0, i = 0;
       for (int u = pair; u < total; u += n_pairs, ++i) {
-        int tile, kb0, kb1, part;
-        unit_of(u, tile, kb0, kb1, part);
-        int n_off, width;
-        if (n_split > 1) nsub_of(u, tile, n_off, width);
-        else { n_off = 0; width = BN; }
+        int tile, n_off, width;
+        unit_of(u, tile, n_off, width);
         const uint32_t idesc = make_idesc_bf16(256, width, 0, 0);
         const int ab = i & 1;
         mbar_wait(acc_empty + ab * 8, ((i >> 1) & 1) ^ 1);  // the epilogues of both CTAs have drained this accumulator
         tc_fence_after();
         const uint32_t acc = tmem_base + ab * BN;
-        for (int kb = kb0; kb < kb1; ++kb, ++it) {
+        for (int kb = 0; kb < num_k; ++kb, ++it) {
           const int s = it % STAGES;
           mbar_wait(bar_full + s * 8, (it / STAGES) & 1);
           tc_fence_after();
           const uint32_t sa = base + s * L::STAGE_BYTES, sb = sa + L::A_BYTES;
           const uint64_t da = make_smem_desc(sa, 16, 1024, SWZ_128B);
           const uint64_t db = make_smem_desc(sb, 16, 1024, SWZ_128B);
-          const uint32_t first = kb != kb0 ? 1u : 0u;
+          const uint32_t first = kb != 0 ? 1u : 0u;
           if (elect_one()) {
 #pragma unroll
             for (int k = 0; k < G2_BK / 16; ++k) tc_mma_bf16_pair(acc, da + (uint32_t)(k * 2), db + (uint32_t)(k * 2), idesc, k == 0 ? first : 1u);
@@ -490,7 +420,6 @@ gemm_nt3_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
     const int q = warp & 3;            // TMEM lane quarter this warp may access
     const int ch = (warp - 2) >> 2;    // column half handled by this warp
     epi.drop = resolve_drop(epi.drop);
-    constexpr int HALF = BN / 2;
     const uint32_t acc_empty0 = mapa_u32(acc_empty, 0);
     int i = 0, nbox = 0;
     // RTMA: residual boxes of this warp.  chunks_of() mirrors exactly the conditions under which the chunk loop below
@@ -499,16 +428,14 @@ gemm_nt3_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
     int nres = 0;
     bool r_inflight = false;
     auto chunks_of = [&](int uu, int& cm0, int& cn0, int& clo, int& chi) -> bool {
-      int t2, a0, a1, p2, off2, w2;
-      unit_of(uu, t2, a0, a1, p2);
-      if (n_split > 1) nsub_of(uu, t2, off2, w2);
-      else { off2 = 0; w2 = BN; }
+      int t2, off2, w2;
+      unit_of(uu, t2, off2, w2);
       cm0 = (t2 % m_tiles) * 256 + (int)rank * G2_BM;
       cn0 = (t2 / m_tiles) * BN + off2;
       const int hu = w2 / 2;
       clo = hu >= 32 ? ch * hu : 0;
       chi = hu >= 32 ? clo + hu : (ch == 0 ? w2 : 0);
-      return p2 == 0 && cm0 + q * 32 < M && !(epi.ablate & 1) && clo < chi;
+      return cm0 + q * 32 < M && clo < chi;
     };
     auto issue_res = [&](int ncol, int row0) {
       if (lane == 0) {
@@ -523,38 +450,13 @@ gemm_nt3_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
       if (chunks_of(pair, cm0, cn0, clo, chi)) issue_res(cn0 + clo, cm0 + q * 32);
     }
     for (int u = pair; u < total; u += n_pairs, ++i) {
-      int tile, kb0, kb1, part;
-      unit_of(u, tile, kb0, kb1, part);
-      int n_off, width;
-      if (n_split > 1) nsub_of(u, tile, n_off, width);
-      else { n_off = 0; width = BN; }
+      int tile, n_off, width;
+      unit_of(u, tile, n_off, width);
       const int ab = i & 1;
       const int m0 = (tile % m_tiles) * 256 + (int)rank * G2_BM, n0 = (tile / m_tiles) * BN + n_off;
       mbar_wait(acc_full + ab * 8, (i >> 1) & 1);
       tc_fence_after();
-      if (part != 0) {  // split-K unit: fp32 partial sums are reduced straight into C (zero-filled by the host)
-        const int row = m0 + q * 32 + lane;
-        const uint32_t tacc = tmem_base + ab * BN + ((uint32_t)(q * 32) << 16) + ch * HALF;
-        EpiArgs2 e2 = epi;
-        if (part == 2) e2.flags &= ~(DSF_EPI_BIAS | DSF_EPI_RESIDUAL);
-        if (m0 + q * 32 < M) {
-#pragma unroll 1
-          for (int c = 0; c < HALF; c += 32) {
-            uint32_t r[32];
-            tmem_ld32(tacc + c, r);
-            tmem_wait_ld();
-            float v[32];
-            const int ncol = n0 + ch * HALF + c;
-            epi_math32(e2, row, ncol, r, v, row < M);
-            if (row < M) {
-              float* cp = reinterpret_cast<float*>(epi.C) + (size_t)row * epi.ldc + ncol;
-#pragma unroll
-              for (int j = 0; j < 32; j += 4) red_add_v4(cp + j, v[j], v[j + 1], v[j + 2], v[j + 3]);
-            }
-          }
-        }
-      } else
-      if (m0 + q * 32 < M && !(epi.ablate & 1)) {
+      if (m0 + q * 32 < M) {
         const int row = m0 + q * 32 + lane;
         const uint32_t tacc = tmem_base + ab * BN + ((uint32_t)(q * 32) << 16);
         const uint32_t stg = base + L::STAGING_OFF + (warp - 2) * 8192;
@@ -812,13 +714,6 @@ static int launch_tn2(const CUtensorMap& tmA, const CUtensorMap& tmB, float* C, 
   return check_launch("gemm_tn2");
 }
 
-// Split the leftover tiles of the pair kernel along N (256 x 128 or 256 x 64 units, see the kernel): no partial
-// sums, works with every epilogue.  DSF_GEMM_TAIL_NSPLIT=0 disables it.
-static const bool g_nt_tail_nsplit = getenv("DSF_GEMM_TAIL_NSPLIT") ? atoi(getenv("DSF_GEMM_TAIL_NSPLIT")) != 0 : true;
-
-// fp32 output + residual: prefetch the residual tile by TMA (see the kernel).  DSF_GEMM_RES_TMA=0 disables it.
-static const bool g_nt_res_tma = getenv("DSF_GEMM_RES_TMA") ? atoi(getenv("DSF_GEMM_RES_TMA")) != 0 : true;
-
 template <int BN, int STAGES, bool RTMA = false>
 static int launch_nt3(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmC, const EpiArgs2& epi, int M, int N, int K,
                       cudaStream_t st, const void* Bptr = nullptr, int ldb = 0) {
@@ -838,11 +733,12 @@ static int launch_nt3(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUte
   const int tiles = m_tiles * n_tiles;
   const int pairs = std::min(tiles, num_sms() / 2);
   int tail_start = tiles;
-  const int tail_split = 1;  // (splitting leftover tiles along K was measured slower and is no longer offered by the host side)
   const int rem = tiles % pairs;
+  // Split the leftover tiles along N (256 x 128 or 256 x 64 units, see the kernel): no partial sums, works with every
+  // epilogue.  (Splitting them along K, with fp32 reductions into a zero-filled C, was measured slower and removed.)
   int n_split = 1;
   CUtensorMap tmBt = tmB;
-  if (g_nt_tail_nsplit && tail_split == 1 && BN == 256 && Bptr != nullptr && rem > 0 && tiles > pairs) {
+  if (BN == 256 && Bptr != nullptr && rem > 0 && tiles > pairs) {
     for (int ns = 4; ns >= 2; ns >>= 1) {
       if (rem * ns <= pairs) { n_split = ns; break; }
     }
@@ -852,7 +748,7 @@ static int launch_nt3(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUte
     }
   }
   launch_pdl(gemm_nt3_kernel<BN, STAGES, RTMA>, dim3(2 * pairs), dim3(G2_THREADS), L::DYN, st, tmA, tmB, tmC, tmBt, tmR, epi, M, N, K, m_tiles,
-             n_tiles, tail_start, tail_split, n_split);
+             n_tiles, tail_start, n_split);
   return check_launch("gemm_nt3");
 }
 
@@ -876,13 +772,6 @@ static int pick_bn_nt(int M, int N) {
 
 int gemm_nt_run(const void* A, int lda, const void* B, int ldb, void* C, int ldc, int c_dtype, const float* bias, const float* residual, int M,
                 int N, int K, int flags, const dsf_dropout* drop, const void* relu_src, bool pairs, cudaStream_t st) {
-  // kernel-timing diagnostics only (DESIGN.md "What bounds the tensor-core kernels"): any non-zero value makes the
-  // GEMM results WRONG on purpose (skipped loads / epilogue), hence the loud warning
-  static const int ablate = [] {
-    const int v = getenv("DSF_GEMM_ABLATE") ? atoi(getenv("DSF_GEMM_ABLATE")) : 0;
-    if (v) fprintf(stderr, "dsfuse: DSF_GEMM_ABLATE=%d is set: tensor-core GEMM results are INVALID (timing diagnostics only)\n", v);
-    return v;
-  }();
   CUtensorMap tmA, tmB;
   if (pairs && N % 128 == 0 && M > 128) {
     // CTA-pair kernel: 256 x BN tiles, each CTA loads BN/2 rows of B.  BN = 256 whenever N allows: one tcgen05.mma costs
@@ -894,12 +783,12 @@ int gemm_nt_run(const void* A, int lda, const void* B, int ldb, void* C, int ldc
     if (int e = make_tmap_bf16(&tmB, B, N, K, ldb, BN3 / 2)) return e;
     CUtensorMap tmC3;
     if (int e = make_tmap_2d(&tmC3, C, c_dtype, M, N, ldc, c_dtype == DSF_F32 ? 32 : 64, 32)) return e;
-    EpiArgs2 epi3{C, ldc, c_dtype, bias, residual, flags, N, reinterpret_cast<const __nv_bfloat16*>(relu_src), ablate, make_drop(drop)};
-    if (BN3 == 256 && g_nt_res_tma && c_dtype == DSF_F32 && (flags & DSF_EPI_RESIDUAL) && residual != nullptr && !ablate)
-      return launch_nt3<256, 4, true>(tmA, tmB, tmC3, epi3, M, N, K, st, B, ldb);
+    EpiArgs2 epi3{C, ldc, c_dtype, bias, residual, flags, N, reinterpret_cast<const __nv_bfloat16*>(relu_src), make_drop(drop)};
+    // fp32 output + residual: the residual tile is prefetched by TMA (RTMA, see the kernel)
+    const bool res_tma = c_dtype == DSF_F32 && (flags & DSF_EPI_RESIDUAL) && residual != nullptr;
+    if (BN3 == 256 && res_tma) return launch_nt3<256, 4, true>(tmA, tmB, tmC3, epi3, M, N, K, st, B, ldb);
     if (BN3 == 256) return launch_nt3<256, 5>(tmA, tmB, tmC3, epi3, M, N, K, st, B, ldb);
-    if (g_nt_res_tma && c_dtype == DSF_F32 && (flags & DSF_EPI_RESIDUAL) && residual != nullptr && !ablate)
-      return launch_nt3<128, 5, true>(tmA, tmB, tmC3, epi3, M, N, K, st);
+    if (res_tma) return launch_nt3<128, 5, true>(tmA, tmB, tmC3, epi3, M, N, K, st);
     return launch_nt3<128, 6>(tmA, tmB, tmC3, epi3, M, N, K, st);
   }
   const int BN = pick_bn_nt(M, N);
@@ -907,7 +796,7 @@ int gemm_nt_run(const void* A, int lda, const void* B, int ldb, void* C, int ldc
   if (int e = make_tmap_bf16(&tmB, B, N, K, ldb, BN)) return e;
   CUtensorMap tmC;  // store boxes: 32 rows x 128 bytes
   if (int e = make_tmap_2d(&tmC, C, c_dtype, M, N, ldc, c_dtype == DSF_F32 ? 32 : 64, 32)) return e;
-  EpiArgs2 epi{C, ldc, c_dtype, bias, residual, flags, N, reinterpret_cast<const __nv_bfloat16*>(relu_src), ablate, make_drop(drop)};
+  EpiArgs2 epi{C, ldc, c_dtype, bias, residual, flags, N, reinterpret_cast<const __nv_bfloat16*>(relu_src), make_drop(drop)};
   if (BN == 256) return launch_nt2<256, 3>(tmA, tmB, tmC, epi, M, N, K, st);
   if (BN == 128) return launch_nt2<128, 4>(tmA, tmB, tmC, epi, M, N, K, st);
   return launch_nt2<64, 5>(tmA, tmB, tmC, epi, M, N, K, st);

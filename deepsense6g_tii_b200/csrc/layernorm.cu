@@ -420,16 +420,6 @@ layernorm_bwd2_kernel(const TY* __restrict__ dy, const float* __restrict__ x, co
   }
 }
 
-// 1 = register-resident rows (v1), 2 = cp.async row rings (v2, default where the shape allows)
-static int ln_impl() {
-  static const int v = getenv("DSF_LN_IMPL") ? atoi(getenv("DSF_LN_IMPL")) : 2;
-  return v;
-}
-static int ln_fwd_impl() {  // the forward can be switched on its own (DSF_LN_FWD_IMPL)
-  static const int v = getenv("DSF_LN_FWD_IMPL") ? atoi(getenv("DSF_LN_FWD_IMPL")) : ln_impl();
-  return v;
-}
-
 template <typename K>
 static bool ln2_configure(K kernel, int smem) {
   return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) == cudaSuccess;
@@ -472,7 +462,7 @@ template <typename TY>
 int launch_ln_fwd(const float* x, const float* gamma, const float* beta, void* y, float* mean, float* rstd, int M, int C,
                   float eps, cudaStream_t st) {
   TY* yy = reinterpret_cast<TY*>(y);
-  if (ln_fwd_impl() == 2 && C % 128 == 0) {
+  if (C % 128 == 0) {  // cp.async row rings (v2) where C / 128 is 1, 2, 4 or 8; register-resident rows (v1) otherwise
     switch (C / 128) {
       case 1: return launch_ln_fwd2<TY, 1>(x, gamma, beta, yy, mean, rstd, M, eps, st);
       case 2: return launch_ln_fwd2<TY, 2>(x, gamma, beta, yy, mean, rstd, M, eps, st);
@@ -496,11 +486,10 @@ int launch_ln_bwd(const void* dy, const float* x, const float* gamma, const floa
                   const float* dx_add, float* dx, float* dgamma, float* dbeta, void* dx_bf16, float* dx_colsum, DropArgs drop, int M, int C,
                   cudaStream_t st) {
   // few, fat CTAs: every CTA ends with 2-3 x C atomics
-  static const int mult = getenv("DSF_LN_BWD_MULT") ? std::max(1, atoi(getenv("DSF_LN_BWD_MULT"))) : 4;
-  const int blocks = std::min(cdiv(M, LN_WARPS * 2), num_sms() * mult);
+  const int blocks = std::min(cdiv(M, LN_WARPS * 2), num_sms() * 4);
   const TY* d = reinterpret_cast<const TY*>(dy);
   __nv_bfloat16* xb = reinterpret_cast<__nv_bfloat16*>(dx_bf16);
-  if (ln_impl() == 2 && C % 128 == 0) {
+  if (C % 128 == 0) {
     switch (C / 128) {
       case 1: return launch_ln_bwd2<TY, 1, EXTRA>(d, x, gamma, mean, rstd, dx_add, dx, dgamma, dbeta, xb, dx_colsum, drop, M, st);
       case 2: return launch_ln_bwd2<TY, 2, EXTRA>(d, x, gamma, mean, rstd, dx_add, dx, dgamma, dbeta, xb, dx_colsum, drop, M, st);

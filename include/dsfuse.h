@@ -201,9 +201,6 @@ int dsf_attn_bwd(const void* qkv, const void* y, const void* dy, const float* ls
 int dsf_attn_bwd_parts(const void* qkv, const void* y, const void* dy, const float* lse, float* delta,
                        void* dqkv, int32_t B, int32_t T, int32_t C, int32_t nh, const dsf_dropout* drop,
                        const uint32_t* drop_bits, int32_t parts, void* stream);
-/* Selects the forward CTA shape (process-wide, atomic; tests and A/B timing): 0 = default (128-row CTAs, two per SM),
- * 1 = force 128-row CTAs, 2 = force 256-row CTAs (one per SM, two softmax warpgroups sharing each K/V tile). */
-int dsf_attn_set_impl(int32_t impl);
 
 /* K7 forward.  Replaces slice/view/permute/contiguous (model2_seq.py:275-286) + F.interpolate
  * (bilinear, align_corners=False; :521-523, 539-541, 558-560) + residual add (:524-526 ...).

@@ -1,7 +1,8 @@
-"""In-kernel timeline of the forward attention kernel (diagnostics build):
+"""In-kernel timeline of the forward and dK/dV attention kernels (diagnostics build):
     make -C deepsense6g_tii_b200/csrc trace && DSF_LIB=deepsense6g_tii_b200/libdsfuse_trace.so python scripts/attn_trace.py
-Prints, per K/V iteration of CTA (0,0,0), how long the MMA warp waited for the P tiles and how the softmax warps split
-their time between waiting for S, loading it, the rescale check, waiting for the P buffer and the exp/store phase."""
+Prints, per K/V iteration of the forward's CTA (0,0,0), how long the MMA warp waited for V and for the P tile and how the
+softmax warpgroup split its time between waiting for S, loading it, the rescale check and the exp/store phase; then the
+same for the dK/dV kernel.  Rows of the stamp buffer: 0 / 1 = one warp of math warpgroup 0 / 1, 2 = the MMA warp."""
 import ctypes
 import os
 import sys
@@ -27,17 +28,16 @@ t = torch.tensor(list(buf), dtype=torch.int64).view(3, 64, 6)
 n_kv = (T + 63) // 64
 t0 = int(t[2, 0, 0])
 print("head size %d, T=%d: per-iteration cycles of CTA (0,0,0)" % (C // nh, T))
-print("iter | MMA warp: wait V, wait P(wg0), issue, wait P(wg1) | softmax wg0: wait S, load+max, rescale chk, wait P buf, exp+store | wg1 same | iter total")
+print("iter | MMA warp: wait V, wait P | softmax: wait S, load+max, rescale chk, exp+store | iter total")
 for j in range(n_kv):
     m = t[2, j]
     nxt = int(t[2, j + 1, 0]) if j + 1 < n_kv else None
-    row = "%4d | %6d %6d %6d %6d |" % (j, int(m[1] - m[0]), int(m[2] - m[1]), int(m[3] - m[2]), int(m[4] - m[3]))
-    for w in (0, 1):
-        a = t[w, j]
-        row += " %6d %6d %6d %6d %6d |" % (int(a[1] - a[0]), int(a[2] - a[1]), int(a[3] - a[2]), int(a[4] - a[3]), int(a[5] - a[4]))
+    row = "%4d | %6d %6d |" % (j, int(m[1] - m[0]), int(m[2] - m[1]))
+    a = t[0, j]
+    row += " %6d %6d %6d %6d |" % (int(a[1] - a[0]), int(a[2] - a[1]), int(a[3] - a[2]), int(a[5] - a[3]))
     row += " %s" % ("%6d" % (nxt - int(m[0])) if nxt else "")
     print(row)
-print("whole loop: %d cycles" % (int(t[2, n_kv - 1, 4]) - t0))
+print("whole loop: %d cycles" % (int(t[0, n_kv - 1, 5]) - t0))
 
 # ---- dK/dV backward kernel (CTA (0,0,0) = keys 0..127 of head 0, batch 0): per 64-query iteration
 dy = torch.randn(B * T, C, device=dev).to(torch.bfloat16)

@@ -1,7 +1,7 @@
 """Attention kernels timed one by one (GPU): forward, dK/dV (part 2), dQ (part 4), delta (part 1) at the four stage shapes and
 the 16x16-anchor shape.  CUDA events around back-to-back launches of one kernel; the working set of a shape (<= 75 MB) is
 L2-resident, as it is inside the step (qkv / dy were just written by the preceding kernels).
-Usage: [DSF_ATTN_BWD_PAIRS=1|2] python scripts/bench_attn_parts.py [tag] [fwd]     (fwd: forward kernel only)"""
+Usage: python scripts/bench_attn_parts.py [tag] [fwd]     (tag: label printed with the results; fwd: forward kernel only)"""
 import os
 import sys
 
@@ -12,7 +12,7 @@ from deepsense6g_tii_b200 import _capi as K  # noqa: E402
 
 dev = torch.device("cuda")
 K.check_device()
-tag = sys.argv[1] if len(sys.argv) > 1 else "pairs=%s" % os.environ.get("DSF_ATTN_BWD_PAIRS", "default")
+tag = sys.argv[1] if len(sys.argv) > 1 else "default"
 fwd_only = len(sys.argv) > 2 and sys.argv[2] == "fwd"
 
 

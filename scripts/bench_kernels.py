@@ -36,13 +36,10 @@ if "attn" in what or "attn512" in what or "attnq" in what:
         delta = torch.empty(B, nh, T, device=dev)
         dqkv = torch.empty_like(qkv)
         fl = 4.0 * T * T * C * B
-        for impl in (0, 2):  # forward with 128-row CTAs (two per SM, default) / 256-row CTAs
-            K.attn_set_impl(impl)
-            tf = timeit(lambda: K.attn_fwd(qkv, y, lse, B, T, C, nh))
-            tb = timeit(lambda: K.attn_bwd(qkv, y, dy, lse, delta, dqkv, B, T, C, nh))
-            print("attn v%d B=%d T=%d C=%d hs=%d: fwd %.3f ms (%.0f TF/s)  bwd %.3f ms (%.0f TF/s, 2x fwd flops)"
-                  % (impl, B, T, C, C // nh, tf, fl / tf / 1e9, tb, 2 * fl / tb / 1e9))
-        K.attn_set_impl(0)
+        tf = timeit(lambda: K.attn_fwd(qkv, y, lse, B, T, C, nh))
+        tb = timeit(lambda: K.attn_bwd(qkv, y, dy, lse, delta, dqkv, B, T, C, nh))
+        print("attn B=%d T=%d C=%d hs=%d: fwd %.3f ms (%.0f TF/s)  bwd %.3f ms (%.0f TF/s, 2x fwd flops)"
+              % (B, T, C, C // nh, tf, fl / tf / 1e9, tb, 2 * fl / tb / 1e9))
 
 if "gemm" in what:
     M = 11544
@@ -117,8 +114,7 @@ if "ln" in what:
         it[0] += 1
         K.layernorm_bwd(s["dy"], s["x"], g, mean, rstd, s["add"], s["dx"], dg, db, dx_bf16=s["dxb"], dx_colsum=cs)
     t = timeit(run, iters=40, warm=8)
-    print("layernorm_bwd (step form, HBM-resident) mult=%s: %.4f ms (%.0f GB/s of 18 B/elem)"
-          % (os.environ.get("DSF_LN_BWD_MULT", "default"), t, M * C * 18 / t / 1e6))
+    print("layernorm_bwd (step form, HBM-resident): %.4f ms (%.0f GB/s of 18 B/elem)" % (t, M * C * 18 / t / 1e6))
     yb = torch.empty(M, C, device=dev, dtype=torch.bfloat16)
 
     def runf():

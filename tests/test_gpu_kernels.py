@@ -346,16 +346,7 @@ def _attn_ref(qkv, B, T, C, nh):
 @pytest.mark.parametrize("B,T,C,nh", [(1, 128, 64, 4), (2, 64, 128, 4), (2, 130, 256, 4), (1, 962, 512, 4), (2, 962, 64, 4),
                                       (1, 962, 128, 4), (1, 962, 256, 4), (1, 300, 128, 1), (1, 3842, 64, 4),
                                       (3, 257, 512, 4), (2, 1, 64, 4), (1, 513, 64, 1)])
-@pytest.mark.parametrize("impl", [0, 2], ids=["fwd_128row_ctas", "fwd_256row_ctas"])
-def test_attention_fwd_bwd(K, cuda_dev, B, T, C, nh, impl):
-    K.attn_set_impl(impl)
-    try:
-        _attention_case(K, cuda_dev, B, T, C, nh)
-    finally:
-        K.attn_set_impl(0)
-
-
-def _attention_case(K, cuda_dev, B, T, C, nh):
+def test_attention_fwd_bwd(K, cuda_dev, B, T, C, nh):
     g = _gen(8)
     qkv = torch.randn(B * T, 3 * C, generator=g).to(cuda_dev).to(torch.bfloat16)
     y = torch.empty(B * T, C, device=cuda_dev, dtype=torch.bfloat16)
@@ -377,27 +368,22 @@ def _attention_case(K, cuda_dev, B, T, C, nh):
 
 
 @pytest.mark.parametrize("B,T,C,nh", [(2, 962, 512, 4), (2, 962, 64, 4), (1, 1000, 128, 4), (1, 3842, 256, 4)])
-@pytest.mark.parametrize("impl", [0, 2], ids=["fwd_128row_ctas", "fwd_256row_ctas"])
-def test_attention_fwd_when_the_running_maximum_keeps_moving(K, cuda_dev, B, T, C, nh, impl):
+def test_attention_fwd_when_the_running_maximum_keeps_moving(K, cuda_dev, B, T, C, nh):
     """Keys grow along the sequence, so later key tiles raise a row's maximum by far more than the lazy-rescale threshold (2^8):
     the forward kernel's speculative tiles (exponentials taken against the running maximum first) have to be repeated and the
     output accumulator rescaled.  Same softmax, model2_seq.py:94-106."""
-    K.attn_set_impl(impl)
-    try:
-        g = _gen(21)
-        qkv = torch.randn(B, T, 3 * C, generator=g)
-        ramp = 0.25 + 5.0 * torch.arange(T, dtype=torch.float32).view(1, T, 1) / T
-        qkv[:, :, C:2 * C] *= ramp          # logits of key t scale with ramp[t]: standard deviation 0.25 .. 5.25
-        qkv = qkv.reshape(B * T, 3 * C).to(cuda_dev).to(torch.bfloat16)
-        y = torch.empty(B * T, C, device=cuda_dev, dtype=torch.bfloat16)
-        lse = torch.empty(B, nh, T, device=cuda_dev)
-        K.attn_fwd(qkv, y, lse, B, T, C, nh)
-        torch.cuda.synchronize()
-        ref, lse_ref = _attn_ref(qkv.float(), B, T, C, nh)
-        assert_close(lse, lse_ref, 1e-4, 1e-4, "lse")
-        assert_close(y.float(), ref, 1e-2, 1e-4, "attn fwd")
-    finally:
-        K.attn_set_impl(0)
+    g = _gen(21)
+    qkv = torch.randn(B, T, 3 * C, generator=g)
+    ramp = 0.25 + 5.0 * torch.arange(T, dtype=torch.float32).view(1, T, 1) / T
+    qkv[:, :, C:2 * C] *= ramp          # logits of key t scale with ramp[t]: standard deviation 0.25 .. 5.25
+    qkv = qkv.reshape(B * T, 3 * C).to(cuda_dev).to(torch.bfloat16)
+    y = torch.empty(B * T, C, device=cuda_dev, dtype=torch.bfloat16)
+    lse = torch.empty(B, nh, T, device=cuda_dev)
+    K.attn_fwd(qkv, y, lse, B, T, C, nh)
+    torch.cuda.synchronize()
+    ref, lse_ref = _attn_ref(qkv.float(), B, T, C, nh)
+    assert_close(lse, lse_ref, 1e-4, 1e-4, "lse")
+    assert_close(y.float(), ref, 1e-2, 1e-4, "attn fwd")
 
 
 def test_error_paths(K, cuda_dev):
@@ -509,16 +495,7 @@ def _unpack_bits(bits, B, nh, T, dev):
 
 
 @pytest.mark.parametrize("B,T,C,nh", [(1, 128, 64, 4), (2, 130, 256, 4), (1, 962, 512, 4), (2, 962, 64, 4), (1, 962, 128, 4), (1, 513, 64, 1)])
-@pytest.mark.parametrize("impl", [0, 2], ids=["fwd_128row_ctas", "fwd_256row_ctas"])
-def test_attention_dropout_fwd_bwd(K, cuda_dev, B, T, C, nh, impl):
-    K.attn_set_impl(impl)
-    try:
-        _attention_dropout_case(K, cuda_dev, B, T, C, nh)
-    finally:
-        K.attn_set_impl(0)
-
-
-def _attention_dropout_case(K, cuda_dev, B, T, C, nh):
+def test_attention_dropout_fwd_bwd(K, cuda_dev, B, T, C, nh):
     """attn_drop (:104): softmax -> dropout -> @v.  The kernel's keep-bitmap is fed to a plain torch evaluation."""
     from deepsense6g_tii_b200.functional import attn_drop_scale
     g = _gen(18)
